@@ -2,6 +2,7 @@
 """Benchmark of the trie-mass hot path (BASELINE.json metric: trie weight_sum/max distributions/sec at 128k vocab).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|async1024|smc4096|cfg5]
+                    [--dump-outputs DIR]
 
 Default workload (cfg2 = BASELINE.json configs[1], the one the metric is quoted on): one "step" = batch_weight_sum +
 batch_weight_max over one batch of 64 synthetic Dirichlet rows on the 128,256-token synthetic byte vocabulary; a
@@ -9,8 +10,8 @@ batch_weight_max over one batch of 64 synthetic Dirichlet rows on the 128,256-to
 its own rows (weak scaling, no collective on the data path); `value` is the whole-job rate, timed on the device, max
 over ranks.
 
-  value          device-resident: inputs in HBM, CUDA events around the K steps (one CUDA graph of K steps rotating over
-                 buffer sets larger than L2), repeated until at least --min-ms of device time has passed
+  value          device-resident: inputs in HBM, CUDA events around exactly the K steps (one CUDA graph of K steps
+                 rotating over buffer sets larger than L2, replayed once untimed and, queued right behind it, once timed)
   e2e            the same step through the public, reference-shaped API: pinned HOST rows in, numpy arrays out
                  (ParallelTokenCharacterTrie.batch_weight_sum_max), H2D and D2H inside the timed region
   roofline       dominant kernel (mass_kernel): algorithmic bytes (4V + 8N per distribution) / its CUDA-event time
@@ -28,6 +29,11 @@ Other workloads (BASELINE.json configs[0], [2..4]; one JSON line each, same cont
   smc4096        fused masked logsumexp + multinomial, 4,096 particles x 128,256 tokens, particles sharded over ranks
   cfg5           batch_weight_sum + batch_weight_max at 151,665 tokens, 8,192 rows over 8 GPUs (1,024 per GPU),
                  plus (--allgather) the NCCL all-gather of the full [rows, N] node-mass slab
+
+--dump-outputs DIR (cfg2, cfg5): after the timed steps, rank 0 writes what the last timed step computed, the [B, N]
+weight_sum and weight_max results, as DIR/weight_sum.npy and DIR/weight_max.npy (float32) with DIR/node_ids.npy
+(float64) naming their columns: every node when the two fit in 64 MB, otherwise a fixed seeded sample of the nodes.
+The inputs depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -59,7 +65,6 @@ def parse_args():
     ap.add_argument("--alpha", type=float, default=1.0)
     ap.add_argument("--sets", type=int, default=4, help="rotating buffer sets (cfg2: each 33 MB in + 176 MB out)")
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = min(steps, 10)")
-    ap.add_argument("--min-ms", type=float, default=50.0, help="the K timed steps are repeated until this much device time has passed")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip the torch library-kernel baseline on the GPU")
@@ -67,7 +72,12 @@ def parse_args():
     ap.add_argument("--allgather", action="store_true",
                     help="N > 1 only: also time the optional NCCL all-gather of the node masses (BASELINE config 5's exchange); "
                          "reported separately, never part of the timed step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy (cfg2, cfg5)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("cfg2", "cfg5")):
+        ap.error("--dump-outputs covers the trie-mass workloads (cfg2, cfg5) of --impl ours")
     if not args.vocab:
         args.vocab = {"cfg5": 151665, "cfg0": 50257}.get(args.workload, 128256)
     if not args.batch:
@@ -291,30 +301,24 @@ class Job:
         if self.world > 1:
             self.dist.destroy_process_group()
 
-    def timed_repeats(self, enqueue, min_ms, clocks=None):
-        """Device time of one `enqueue()` (ms, max over ranks): repeated until min_ms have passed, barrier + sync on both sides."""
+    def timed(self, enqueue, clocks=None):
+        """Device time of one `enqueue()` (ms, max over ranks); barrier + sync on both sides.  It is queued right behind an
+        untimed `enqueue()` (a CUDA graph's first replay uploads it), so the device starts the timed work as soon as the
+        start event completes instead of waiting for the host to launch it."""
         torch = self.torch
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        enqueue()
-        torch.cuda.synchronize()
-        ev0.record()
-        enqueue()
-        ev1.record()
-        torch.cuda.synchronize()
-        reps = max(1, int(np.ceil(min_ms / max(ev0.elapsed_time(ev1), 1e-3))))
-        reps = int(self.max_over_ranks(float(reps)))
         self.barrier()
         if clocks is not None:
             clocks.loaded = True
+        enqueue()
         ev0.record()
-        for _ in range(reps):
-            enqueue()
+        enqueue()
         ev1.record()
         torch.cuda.synchronize()
         if clocks is not None:
             clocks.loaded = False
         self.barrier()
-        return self.max_over_ranks(ev0.elapsed_time(ev1)) / reps, reps
+        return self.max_over_ranks(ev0.elapsed_time(ev1))
 
 
 # ---- secondary measurement: the SMC row op (BASELINE.json configs[3], per-GPU share) ---------------------------------
@@ -450,6 +454,26 @@ def reference_gpu_metrics(trie, ws_dev, host_rows, ours_value, ours_e2e):
     }
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_node_slabs(out_dir, slabs):
+    """Writes [B, N] float32 device slabs (name -> tensor) as out_dir/<name>.npy and the node columns they hold as
+    out_dir/node_ids.npy (float64): all N columns when everything fits DUMP_BYTES, otherwise a sorted sample drawn with
+    a fixed seed, so that runs with the same B and N write the same elements."""
+    import torch
+
+    B, N = next(iter(slabs.values())).shape
+    per_col = 4 * B * len(slabs) + 8
+    S = min(N, max(1, (DUMP_BYTES - 4096) // per_col))  # 4096: room for the .npy headers
+    cols = np.arange(N) if S == N else np.sort(np.random.default_rng(0).choice(N, size=S, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    idx = torch.from_numpy(cols).to(next(iter(slabs.values())).device)
+    for name, slab in slabs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), slab[:, idx].cpu().numpy().astype(np.float32, copy=False))
+    np.save(os.path.join(out_dir, "node_ids.npy"), cols.astype(np.float64))
+
+
 # ---- default workload: BASELINE.json configs[1] (and cfg5's per-GPU shape) --------------------------------------------
 def run_mass(args, job):
     torch = job.torch
@@ -507,8 +531,11 @@ def run_mass(args, job):
 
     clocks = ClockSampler(job.local_rank)
     clocks.start()
-    ms_total, reps = job.timed_repeats(run_steps, args.min_ms, clocks)
+    ms_total = job.timed(run_steps, clocks)
     value = world * B * K / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:  # before the per-kernel timings below overwrite the buffers
+        last = (K - 1) % nsets
+        dump_node_slabs(args.dump_outputs, {"weight_sum": sum_sets[last], "weight_max": max_sets[last]})
 
     # per-kernel timing for the roofline (one op, one phase at a time), same buffers ----------------------------------
     def time_phase(phases, ops):
@@ -621,9 +648,9 @@ def run_mass(args, job):
             "parallelism": f"rows sharded, {world} independent GPU(s), no collective",
             "l2_policy": f"rotating {nsets} buffer set(s) of {set_bytes / 1e6:.0f} MB ({nsets * set_bytes / 1e6:.0f} MB total) "
                          f"vs L2 {l2_bytes / 1e6:.0f} MB",
-            "launch": (f"one CUDA graph of the {K} steps, replayed {reps}x ({ms_total * reps:.1f} ms timed)" if graph is not None
-                       else f"direct launches, {reps} repetitions ({ms_total * reps:.1f} ms timed)"),
-            "timed_repeats": reps, "tile_leaves": info["tile_leaves"], "n_span": info["n_span"],
+            "launch": (f"one CUDA graph of the {K} steps, one timed replay ({ms_total:.1f} ms)" if graph is not None
+                       else f"direct launches of the {K} steps ({ms_total:.1f} ms timed)"),
+            "tile_leaves": info["tile_leaves"], "n_span": info["n_span"],
         },
         "e2e": {
             "value": world * B * E / e2e_s, "unit": UNIT, "h2d_bytes_per_step": B * V * 4,
@@ -637,7 +664,7 @@ def run_mass(args, job):
             "api": "ParallelTokenCharacterTrie.batch_weight_sum_max_at(pinned host tensor, node_ids) -> numpy [B, K] x 2",
             "note": "not the headline: same kernels, results read through gt_gather_nodes instead of copying the [B, N] slabs",
         },
-        "gpu_launches": launches_per_step * K * reps,
+        "gpu_launches": launches_per_step * K,
         "roofline": {
             "bound": "hbm", "kernel": "mass_kernel<float,4> (the tile kernel: both reductions of the step in one launch)", "achieved": achieved,
             "peak": peak, "unit": "GB/s", "frac": achieved / peak, "traffic": traffic, "peak_source": peak_src,
@@ -708,8 +735,8 @@ def run_smc(args, job):
         with torch.cuda.graph(g):
             for i in range(K):
                 smc.masked_logsumexp_sample(sets[i % nsets], mask, seed=i, offset=lo)
-        ms, reps = job.timed_repeats(g.replay, args.min_ms, clocks)
-        res[name] = {"ms_per_step": ms / K, "particles_per_s": total * K / (ms / 1e3), "timed_repeats": reps,
+        ms = job.timed(g.replay, clocks)
+        res[name] = {"ms_per_step": ms / K, "particles_per_s": total * K / (ms / 1e3),
                      "per_gpu_GBps": rows * (4 * V + (4 * ((V + 31) // 32) if name == "per_row_bit_mask" else 0) + 8) / (ms / K / 1e3) / 1e9}
     # end to end: pinned host log-probs in, logZ + tokens out on the host
     host = sets[0].cpu().pin_memory()
@@ -751,7 +778,7 @@ def run_smc(args, job):
                    "l2_policy": f"rotating {nsets} logit sets of {rows * V * 4 / 1e6:.0f} MB", "launch": f"one CUDA graph of the {K} steps"},
         "e2e": {"value": total * E / e2e_s, "unit": "particles/s", "h2d_bytes_per_step": rows * V * 4, "d2h_bytes_per_step": rows * 8, "steps": E,
                 "api": "smc.masked_logsumexp_sample(pinned host rows -> device) -> logZ, tokens on the host"},
-        "gpu_launches": K * head["timed_repeats"],
+        "gpu_launches": K,
         "roofline": {"bound": "hbm", "kernel": "lse_sample_kernel<float>", "achieved": head["per_gpu_GBps"], "peak": peak, "unit": "GB/s",
                      "frac": head["per_gpu_GBps"] / peak, "traffic": None, "peak_source": peak_src},
         "variants": res, "reference_gpu": ref, "clocks": clocks.summary(),

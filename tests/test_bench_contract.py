@@ -1,9 +1,13 @@
 """bench.py's reference arm runs without a GPU: it must print ONE JSON line with the contract's keys, must not load the
-product package, and must use every host thread whatever OMP_NUM_THREADS says (torchrun sets it to 1)."""
+product package, and must use every host thread whatever OMP_NUM_THREADS says (torchrun sets it to 1).  On the GPU,
+--dump-outputs must write what the last timed step computed."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -37,3 +41,29 @@ def test_reference_arm_other_ranks_and_workloads():
     assert out.returncode == 0 and out.stdout.strip() == ""  # ranks other than 0 exit without work
     d = run_bench("--impl", "reference", "--workload", "smc4096")
     assert d["impl"] == "reference" and "unavailable" in d
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_the_last_timed_step(tmp_path):
+    """With one timed step the last step is step 0, on the first buffer set: bench.py's rows dirichlet_rows(B, V, alpha=1,
+    seed=1).  At this size every node fits the dump, so the files hold the whole [B, N] results."""
+    import oracle
+    from genlm_backend_b200 import TokenCharacterTrie
+    from genlm_backend_b200.synthetic import synth_vocab, dirichlet_rows
+    from helpers import rel_err
+
+    V, B = 3000, 16
+    d = run_bench("--vocab", str(V), "--batch", str(B), "--steps", "1", "--warmup", "1", "--e2e-steps", "1", "--no-sampler",
+                  "--no-cpu-baseline", "--no-reference-gpu", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == 1 and d["value"] > 0
+    trie = TokenCharacterTrie(synth_vocab(V))  # the host layout only
+    N = len(trie)
+    ids, s, m = (np.load(tmp_path / f"{n}.npy") for n in ("node_ids", "weight_sum", "weight_max"))
+    assert ids.dtype == np.float64 and np.array_equal(ids, np.arange(N))
+    assert s.dtype == m.dtype == np.float32 and s.shape == m.shape == (B, N)
+    lay = trie._layout
+    o = oracle.OracleLayout(trie.idx_to_leaf, lay["child_ptr"], lay["child_idx"])
+    ws = dirichlet_rows(B, V, alpha=1.0, seed=1)
+    r, z = rel_err(s, o.weight_sum(ws))
+    assert r <= 2e-6 and z == 0.0
+    assert np.array_equal(m, o.weight_max(ws).astype(np.float32))
