@@ -17,6 +17,7 @@ GT_FLAG_LOG_INPUT = 1
 GT_FLAG_DFS_ORDER = 2
 GT_FLAG_PHASE_PERMUTE, GT_FLAG_PHASE_TILE, GT_FLAG_PHASE_SPAN = 0x100, 0x200, 0x400
 GT_GATHER_LOG = 1
+GT_CHILD_NORMALIZE, GT_CHILD_LOG = 0x10, 0x20
 GT_MASK_NONE, GT_MASK_ADD_F32, GT_MASK_BOOL_U8, GT_MASK_BITS_U32 = 0, 1, 2, 3
 
 
@@ -55,6 +56,12 @@ SIGNATURES = {
                                 c_void_p, c_int64, c_void_p]),
     "gt_download_rows": (c_int, [c_void_p, c_size_t, c_void_p, c_size_t, c_size_t, c_int64, c_void_p]),
     "gt_subtree_token_mask": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
+    "gt_max_children": (c_int64, [c_void_p]),
+    "gt_child_workspace_bytes": (c_size_t, [c_void_p, c_int64]),
+    "gt_child_masses": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
+    "gt_child_sample": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_uint, c_uint64, c_uint64, c_void_p,
+                                c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "gt_lse_sample": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_float,
                               c_uint64, c_uint64, c_void_p, c_void_p, c_void_p]),
 }

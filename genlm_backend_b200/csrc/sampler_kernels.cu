@@ -18,6 +18,7 @@
 #include <type_traits>
 
 #include "trie_internal.h"
+#include "philox.cuh"
 
 namespace gt {
 
@@ -44,18 +45,6 @@ struct SampleArgs {
     float inv_temp; uint64_t seed, offset;
     float* logZ; int32_t* tok;
 };
-
-__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0,
-                                              uint32_t k1, uint32_t out[4]) {
-#pragma unroll
-    for (int i = 0; i < 10; ++i) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    out[0] = c0; out[1] = c1; out[2] = c2; out[3] = c3;
-}
 
 template <typename T> __device__ __forceinline__ float elem_to_float(T x);
 template <> __device__ __forceinline__ float elem_to_float<float>(float x) { return x; }
@@ -445,10 +434,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) lse_sample_kernel(SampleArgs A)
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
             // 53-bit uniform in [0,1): Philox4x32-10, counter = offset + row, key = seed
-            const uint64_t ctr = A.offset + (uint64_t)b;
-            uint32_t r[4];
-            philox4x32_10((uint32_t)ctr, (uint32_t)(ctr >> 32), 0u, 0u, (uint32_t)A.seed, (uint32_t)(A.seed >> 32), r);
-            const double u = (double)(((uint64_t)(r[0] >> 5) << 26) | (uint64_t)(r[1] >> 6)) * (1.0 / 9007199254740992.0);
+            const double u = philox_uniform53(A.seed, A.offset + (uint64_t)b);
             const bool ok = (M > -INFINITY) && (tot > 0.0) && (tot < (double)INFINITY);  // false for NaN
             int pick = -1; double before = 0.0;
             if (ok) warp_find(s_mass, NT, u * tot, pick, before);

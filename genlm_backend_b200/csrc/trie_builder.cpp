@@ -140,6 +140,7 @@ static int build_layout(const int32_t* symbols, const int64_t* offsets, int64_t 
         int32_t deg = 0;
         for (int32_t c = first_child[u]; c >= 0; c = next_sib[c]) ++deg;
         L.child_ptr[(size_t)n + 1] = deg;
+        if (deg > L.max_children) L.max_children = deg;
     }
     for (int64_t n = 0; n < N; ++n) L.child_ptr[(size_t)n + 1] += L.child_ptr[(size_t)n];
     for (int64_t u = 0; u < N; ++u) {
@@ -187,6 +188,7 @@ int64_t gt_num_nodes(const gt_trie* t) { return t ? t->layout.N : -1; }
 int64_t gt_root(const gt_trie* t) { return t ? t->layout.N - 1 : -1; }
 int64_t gt_num_reach(const gt_trie* t) { return t ? t->layout.nnz : -1; }
 int64_t gt_max_depth(const gt_trie* t) { return t ? t->layout.max_depth : -1; }
+int64_t gt_max_children(const gt_trie* t) { return t ? t->layout.max_children : -1; }
 
 int gt_export_layout(const gt_trie* t, int32_t* leaf_node, int32_t* parent, int32_t* edge_label,
                      int32_t* child_ptr, int32_t* child_idx, int32_t* perm, int32_t* lo, int32_t* hi) {

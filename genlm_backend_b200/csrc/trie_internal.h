@@ -29,6 +29,7 @@ struct NvtxRange {
 // Host layout in the reference's node-id space (post-order, root = N-1).
 struct Layout {
     int64_t V = 0, N = 0, nnz = 0, max_depth = 0;
+    int64_t max_children = 0;         // D: largest child count of any node
     std::vector<int32_t> leaf_node;   // [V]
     std::vector<int32_t> parent;      // [N]
     std::vector<int32_t> edge_label;  // [N]

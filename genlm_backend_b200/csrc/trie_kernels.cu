@@ -23,6 +23,7 @@
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
 
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -34,6 +35,7 @@
 #include <utility>
 
 #include "trie_internal.h"
+#include "philox.cuh"
 
 namespace gt {
 
@@ -48,6 +50,8 @@ struct PlanView {
     int32_t n_span, n_pieces; const int32_t* span_node; const int32_t* span_pp;
     const int32_t* leaf_rank;  // [V] DFS rank of each item's leaf (inverse of Layout::perm)
     const int32_t* node_lo; const int32_t* node_hi;  // [N] DFS leaf range of every node
+    const int32_t* perm;       // [V] DFS rank -> item position (Layout::perm)
+    const int32_t* child_ptr; const int32_t* child_idx;  // children CSR (ascending ids = jump[] order)
     int32_t debug_stop;  // profiling aid (GT_DEBUG_STOP): 0 = normal; 3 = no emit stores; 9 = emit only
     long long* trace;    // profiling aid (GT_TRACE=1): per (CTA, item) SM-clock stamps of the pipeline events, else null
 };
@@ -788,6 +792,7 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
     std::vector<int32_t> leaf_rank((size_t)L.V);
     for (int64_t r = 0; r < L.V; ++r) leaf_rank[(size_t)L.perm[(size_t)r]] = (int32_t)r;
     const size_t o_leaf_rank = ADDV(leaf_rank), o_node_lo = ADDV(L.lo), o_node_hi = ADDV(L.hi);
+    const size_t o_perm = ADDV(L.perm), o_child_ptr = ADDV(L.child_ptr), o_child_idx = ADDV(L.child_idx);
 #undef ADDV
     total += 256;
 
@@ -839,6 +844,8 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
     v.span_node = (const int32_t*)(base + o_span_node); v.span_pp = (const int32_t*)(base + o_span_pp);
     v.leaf_rank = (const int32_t*)(base + o_leaf_rank);
     v.node_lo = (const int32_t*)(base + o_node_lo); v.node_hi = (const int32_t*)(base + o_node_hi);
+    v.perm = (const int32_t*)(base + o_perm);
+    v.child_ptr = (const int32_t*)(base + o_child_ptr); v.child_idx = (const int32_t*)(base + o_child_idx);
     { const char* e = getenv("GT_DEBUG_STOP"); v.debug_stop = e && *e ? atoi(e) : 0; }
     v.trace = nullptr;
     if (const char* e = getenv("GT_TRACE")) {
@@ -1099,6 +1106,380 @@ __global__ void __launch_bounds__(kMaskThreads) subtree_mask_kernel(PlanView P, 
     }
 }
 
+// ---- child masses of one node per row (gt_child_masses / gt_child_sample) ------------------------------------------
+//
+// The children of a node n tile its DFS leaf range [lo(n), hi(n)) with consecutive ranges (post-order numbering, DESIGN
+// section 2), so the job is a segmented reduction over one contiguous range of DFS ranks per row, with at most D segments.
+// The range is cut into *blocks* of kChildBlock ranks aligned to lo(n), and a block is one warp's work: a batch of root
+// rows (251 blocks each at 128k tokens) spreads over every SM, while a deep node's row is a single block.
+//   child_scan_kernel    one CTA: blocks per row and their exclusive scan (the chunk's work list)
+//   child_block_kernel   persistent warps take blocks u = warp, warp + warps, ...; block k of row b writes the fp64 partial
+//                        sum (and the max) of each child segment j it overlaps to slot j + k of the row.  Children are
+//                        consecutive, so k_first(j + 1) >= k_last(j) and (j, k) -> j + k is injective: no atomics
+//   child_finish_kernel  one warp per row: adds each child's slots in k order and writes ids / sums / maxes (normalised,
+//                        logs), or draws the next symbol
+// Every sum is a fixed function of (node, child): lane l of a block adds the block's ranks 4l + 128q + i (q < 4, i < 4)
+// in that order, the warp combines its lanes by a fixed butterfly, and the finish kernel adds a child's blocks in order.
+// The batch, the row's position in it, the chunking, the input order and the grid size change nothing.
+constexpr int kChildBlock = 512;  // DFS ranks per block: 16 per lane, as four quads of 4 consecutive ranks
+constexpr int kChildQuads = kChildBlock / 128;
+constexpr int64_t kMaxChildRows = 1024;  // rows per chunk (the chunk's work list is staged in shared memory)
+constexpr int kChildThreads = 256;
+
+struct ChildArgs {
+    const void* ws; int in_type; int log_input; int dfs_order; int64_t ld_ws;
+    const int32_t* nodes; int n_rows;   // the chunk's rows
+    int32_t* blk_off;                   // [n_rows + 1] exclusive scan of the blocks per row
+    double* part_sum; float* part_max;  // [n_rows][slots]
+    int64_t slots; int need_max;
+    // finish, masses
+    int32_t* child_ids; float* out_sum; float* out_max; int64_t ld_out; int D; int normalize, log_out;
+    // finish, draw (child_out != null)
+    int32_t* child_out; float* logp_out; float* logZ_out; uint64_t seed, ctr0;  // ctr0 = offset + first row of the chunk
+};
+
+// Children CSR range and DFS leaf range of node n; false for an id outside [0, N) and for a leaf.
+__device__ __forceinline__ bool child_node(const PlanView& P, int n, int& cp0, int& deg, int& lo, int& hi) {
+    if (n < 0 || n >= P.N) return false;
+    cp0 = __ldg(P.child_ptr + n);
+    deg = __ldg(P.child_ptr + n + 1) - cp0;
+    if (deg <= 0) return false;
+    lo = __ldg(P.node_lo + n); hi = __ldg(P.node_hi + n);
+    return true;
+}
+
+__global__ void __launch_bounds__(1024) child_scan_kernel(PlanView P, ChildArgs A) {
+    __shared__ int s_warp[32];
+    pdl_wait();  // the node ids may come from the previous kernel; the work list may still be read by the last chunk
+    pdl_trigger();
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    int carry = 0;
+    for (int base = 0; base < A.n_rows; base += 1024) {
+        const int i = base + tid;
+        int x = 0, cp0, deg, lo, hi;
+        if (i < A.n_rows && child_node(P, __ldg(A.nodes + i), cp0, deg, lo, hi)) x = (hi - lo + kChildBlock - 1) / kChildBlock;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, x, o);
+            if (lane >= o) x += y;
+        }
+        if (lane == 31) s_warp[warp] = x;
+        __syncthreads();
+        if (warp == 0) {
+            int w = s_warp[lane];
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int y = __shfl_up_sync(0xffffffffu, w, o);
+                if (lane >= o) w += y;
+            }
+            s_warp[lane] = w;
+        }
+        __syncthreads();
+        if (i < A.n_rows) A.blk_off[i + 1] = carry + x + (warp ? s_warp[warp - 1] : 0);
+        carry += s_warp[31];
+        __syncthreads();  // s_warp is rewritten by the next 1,024 rows
+    }
+    if (tid == 0) A.blk_off[0] = 0;
+}
+
+template <typename IN_T> __device__ __forceinline__ void load_quad(const IN_T* p, IN_T (&x)[4]) {
+    if constexpr (sizeof(IN_T) == 4) { const float4 t = __ldg(reinterpret_cast<const float4*>(p)); memcpy(x, &t, 16); }
+    else if constexpr (sizeof(IN_T) == 2) { const uint2 t = __ldg(reinterpret_cast<const uint2*>(p)); memcpy(x, &t, 8); }
+    else {
+        const double2 a = __ldg(reinterpret_cast<const double2*>(p)), c = __ldg(reinterpret_cast<const double2*>(p) + 1);
+        memcpy(x, &a, 16); memcpy(x + 2, &c, 16);
+    }
+}
+
+// Block k of row b (one warp).
+template <typename IN_T>
+__device__ __forceinline__ void child_block(const PlanView& P, const ChildArgs& A, int b, int k, int lane) {
+    int cp0 = 0, deg = 0, lo = 0, hi = 0;
+    child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi);  // true: the row has blocks
+    const int w0 = lo + k * kChildBlock, w1 = min(hi, w0 + kChildBlock);
+    const IN_T* row = static_cast<const IN_T*>(A.ws) + (size_t)b * A.ld_ws;
+    const bool log_input = A.log_input != 0;
+    // the weights of this lane's ranks w0 + 4 lane + 128 q + i (0 outside the block; never added)
+    float f[kChildQuads][4];
+    if (A.dfs_order) {  // contiguous: one vector load per quad where the row allows it
+        const bool vec = (reinterpret_cast<uintptr_t>(row + w0) & (sizeof(IN_T) == 2 ? 7 : 15)) == 0;
+#pragma unroll
+        for (int q = 0; q < kChildQuads; ++q) {
+            const int r0 = w0 + 4 * lane + 128 * q;
+            if (vec && r0 + 4 <= w1) {
+                IN_T x[4];
+                load_quad<IN_T>(row + r0, x);
+#pragma unroll
+                for (int i = 0; i < 4; ++i) f[q][i] = convert_in<float, IN_T>(x[i], log_input);
+            } else {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) f[q][i] = r0 + i < w1 ? convert_in<float, IN_T>(__ldg(row + r0 + i), log_input) : 0.f;
+            }
+        }
+    } else {  // vocabulary order: ws[b, perm[r]], perm read coalesced (L2-resident metadata)
+        const bool vec = (w0 & 3) == 0;
+        int pi[kChildQuads][4];
+#pragma unroll
+        for (int q = 0; q < kChildQuads; ++q) {
+            const int r0 = w0 + 4 * lane + 128 * q;
+            if (vec && r0 + 4 <= w1) {
+                const int4 t = __ldg(reinterpret_cast<const int4*>(P.perm + r0));
+                pi[q][0] = t.x; pi[q][1] = t.y; pi[q][2] = t.z; pi[q][3] = t.w;
+            } else {
+#pragma unroll
+                for (int i = 0; i < 4; ++i) pi[q][i] = r0 + i < w1 ? __ldg(P.perm + r0 + i) : -1;
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < kChildQuads; ++q)
+#pragma unroll
+            for (int i = 0; i < 4; ++i) f[q][i] = pi[q][i] >= 0 ? convert_in<float, IN_T>(__ldg(row + pi[q][i]), log_input) : 0.f;
+    }
+
+    // first child whose range ends past w0: narrow [a, z] about 31-fold per round (hi(c_z) > w0 holds throughout).  The
+    // probes a, a + s, ..., min(a + 31 s, z) reach z (31 s >= z - a), so some lane always passes
+    const int32_t* ch = P.child_idx + cp0;
+    int a = 0, z = deg - 1;
+    while (z - a >= 32) {
+        const int s = (z - a + 30) / 31;
+        const int j = min(a + lane * s, z);
+        const int l = __ffs(__ballot_sync(0xffffffffu, __ldg(P.node_hi + __ldg(ch + j)) > w0)) - 1;
+        const int na = l == 0 ? a : a + (l - 1) * s + 1;
+        z = min(z, a + l * s);
+        a = na;
+    }
+    const bool first = a + lane <= z && __ldg(P.node_hi + __ldg(ch + a + lane)) > w0;
+    const int jf = a + __ffs(__ballot_sync(0xffffffffu, first)) - 1;
+
+    double* psum = A.part_sum + (size_t)b * A.slots + k;
+    float* pmax = A.part_max + (size_t)b * A.slots + k;
+    for (int j0 = jf; j0 < deg; j0 += 32) {
+        int clo = INT_MAX, chi = INT_MAX;  // the ranges of the next 32 children, one per lane
+        if (j0 + lane < deg) {
+            const int c = __ldg(ch + j0 + lane);
+            clo = __ldg(P.node_lo + c); chi = __ldg(P.node_hi + c);
+        }
+        const int cnt = min(32, deg - j0);
+        for (int t = 0; t < cnt; ++t) {
+            const int sa = max(__shfl_sync(0xffffffffu, clo, t), w0), sb = min(__shfl_sync(0xffffffffu, chi, t), w1);
+            if (sa >= w1) return;  // warp-uniform: this child and the later ones start past the block
+            double s = 0.0;
+            float m = -INFINITY;
+#pragma unroll
+            for (int q = 0; q < kChildQuads; ++q)
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int r = w0 + 4 * lane + 128 * q + i;
+                    if (r >= sa && r < sb) { s += (double)f[q][i]; m = fmaxf(m, f[q][i]); }
+                }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                s += __shfl_xor_sync(0xffffffffu, s, o);
+                m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+            }
+            if (lane == 0) {
+                psum[j0 + t] = s;
+                if (A.need_max) pmax[j0 + t] = m;
+            }
+        }
+    }
+}
+
+// Three CTAs per SM: 70 registers without spills (the default budget for these parameters was 64, which spilled).
+__global__ void __launch_bounds__(kChildThreads, 3) child_block_kernel(PlanView P, ChildArgs A) {
+    __shared__ int s_off[kMaxChildRows + 1];
+    pdl_wait();  // rows, node ids and the work list come from earlier kernels; the slots may still be read by the last chunk
+    pdl_trigger();
+    for (int i = threadIdx.x; i <= A.n_rows; i += kChildThreads) s_off[i] = A.blk_off[i];
+    __syncthreads();
+    const int total = s_off[A.n_rows];
+    const int lane = threadIdx.x & 31;
+    const int warps = (int)gridDim.x * (kChildThreads / 32);
+    for (int u = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5); u < total; u += warps) {
+        int lo = 0, hi = A.n_rows - 1;  // the row of block u: the last b with s_off[b] <= u
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (s_off[mid] <= u) lo = mid; else hi = mid - 1;
+        }
+        GT_IN_TYPE_SWITCH(A.in_type, (child_block<IN_T>(P, A, lo, u - s_off[lo], lane)));
+    }
+}
+
+// One warp per row.  Lane l owns the contiguous children [j_lo, j_hi) of the row's node; their sums are added in order
+// and an inclusive scan over the lanes gives the running sums and the node's mass (fixed order: normalisation and draw
+// see the same total).
+__global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P, ChildArgs A) {
+    pdl_wait();  // the slots come from child_block_kernel
+    pdl_trigger();
+    const int lane = threadIdx.x & 31;
+    const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
+    if (b >= A.n_rows) return;
+    int cp0 = 0, deg = 0, lo = 0, hi = 0;
+    if (!child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi)) deg = 0;
+    const int32_t* ch = P.child_idx + cp0;
+    const double* psum = A.part_sum + (size_t)b * A.slots;
+    const float* pmax = A.part_max + (size_t)b * A.slots;
+    auto blocks = [&](int c, int& k0, int& k1) {  // the blocks child c overlaps
+        k0 = (__ldg(P.node_lo + c) - lo) / kChildBlock;
+        k1 = (__ldg(P.node_hi + c) - 1 - lo) / kChildBlock;
+    };
+    auto child_sum = [&](int j) {
+        int k0, k1;
+        blocks(__ldg(ch + j), k0, k1);
+        double s = 0.0;
+        for (int k = k0; k <= k1; ++k) s += psum[j + k];
+        return s;
+    };
+    const int per = (deg + 31) / 32;
+    const int j_lo = min(deg, lane * per), j_hi = min(deg, j_lo + per);
+    double local = 0.0;
+    for (int j = j_lo; j < j_hi; ++j) local += child_sum(j);
+    double incl = local;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const double y = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += y;
+    }
+    const double total = __shfl_sync(0xffffffffu, incl, 31);
+
+    if (!A.child_out) {
+        int32_t* ids = A.child_ids + (size_t)b * A.ld_out;
+        float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
+        float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
+        for (int j = j_lo; j < j_hi; ++j) {
+            const int c = __ldg(ch + j);
+            ids[j] = c;
+            if (os) {
+                double s = child_sum(j);
+                if (A.normalize) s /= total;
+                os[j] = (float)(A.log_out ? log(s) : s);
+            }
+            if (om) {
+                int k0, k1;
+                blocks(c, k0, k1);
+                float m = -INFINITY;
+                for (int k = k0; k <= k1; ++k) m = fmaxf(m, pmax[j + k]);
+                om[j] = A.log_out ? (float)log((double)m) : m;
+            }
+        }
+        const float pad = A.log_out ? -INFINITY : 0.f;
+        for (int j = deg + lane; j < A.D; j += 32) {
+            ids[j] = -1;
+            if (os) os[j] = pad;
+            if (om) om[j] = pad;
+        }
+        return;
+    }
+
+    // draw: the first child whose running sum exceeds u * total
+    const bool ok = total > 0.0 && total < (double)INFINITY;  // false for NaN
+    int pick = -1;
+    double mass = 0.0;
+    if (ok) {
+        const double target = philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total;
+        const unsigned hit = __ballot_sync(0xffffffffu, incl > target && local > 0.0);
+        if (hit) {
+            const int src = __ffs(hit) - 1;
+            if (lane == src) {
+                double run = incl - local;
+                for (int j = j_lo; j < j_hi; ++j) {
+                    const double s = child_sum(j);
+                    if (s > 0.0) { pick = j; mass = s; if (run + s > target) break; }
+                    run += s;
+                }
+            }
+            pick = __shfl_sync(0xffffffffu, pick, src);
+            mass = __shfl_sync(0xffffffffu, mass, src);
+        } else {  // rounding pushed the target past the running sums: the last child with mass
+            int last = -1;
+            if (local > 0.0)
+                for (int j = j_hi - 1; j >= j_lo; --j)
+                    if (child_sum(j) > 0.0) { last = j; break; }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+            pick = last;
+            mass = child_sum(pick);  // last >= 0: total > 0
+        }
+    }
+    if (lane == 0) {
+        A.child_out[b] = ok ? __ldg(ch + pick) : -1;
+        A.logZ_out[b] = (float)log(total);  // -inf for no mass, NaN for a NaN weight
+        A.logp_out[b] = ok ? (float)(log(mass) - log(total)) : (total == 0.0 ? -INFINITY : NAN);
+    }
+}
+
+
+// Scratch of the child-mass calls for a chunk of `rows` rows:
+//   blk_off [rows + 1] int32 | part_sum [rows][slots] fp64 | part_max [rows][slots] fp32
+// slots = D + ceil(V / kChildBlock): block k of a row writes child j's partials to slot j + k, j < D, k < ceil(V / kChildBlock).
+struct ChildScratch {
+    int32_t* blk_off; double* part_sum; float* part_max;
+    int64_t rows;  // capacity (0: not even one row)
+    static size_t pad(size_t b) { return (b + 255) & ~size_t(255); }
+    static int64_t slots(const Layout& L) { return L.max_children + (L.V + kChildBlock - 1) / kChildBlock; }
+    static size_t total(int64_t rows, int64_t slots) {
+        return pad((size_t)(rows + 1) * 4) + pad((size_t)rows * slots * 8) + pad((size_t)rows * slots * 4);
+    }
+    ChildScratch(void* base, size_t bytes, int64_t slots) {
+        int64_t lo = 0, hi = kMaxChildRows;
+        while (lo < hi) {  // total() is monotone in the row count
+            const int64_t mid = (lo + hi + 1) / 2;
+            if (total(mid, slots) <= bytes) lo = mid; else hi = mid - 1;
+        }
+        rows = lo;
+        char* p = static_cast<char*>(base);
+        blk_off = reinterpret_cast<int32_t*>(p);
+        p += pad((size_t)(rows + 1) * 4);
+        part_sum = reinterpret_cast<double*>(p);
+        p += pad((size_t)rows * slots * 8);
+        part_max = reinterpret_cast<float*>(p);
+    }
+};
+
+// Shared by gt_child_masses and gt_child_sample: arguments are checked by the callers (before any CUDA call); this
+// selects the device plan and launches scan -> blocks -> finish per chunk of rows, chained with programmatic dependent
+// launch on the caller's stream.  A.nodes / A.ws / outputs point at row 0; chunk c advances them.
+static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t out_ld_rows, uint64_t offset, void* workspace,
+                        size_t workspace_bytes, cudaStream_t st, const char* what) {
+    const int64_t slots = ChildScratch::slots(t->layout);
+    const ChildScratch sc(workspace, workspace_bytes, slots);
+    if (sc.rows < 1) {
+        set_error("%s: workspace too small: %zu bytes given, one row needs %zu", what, workspace_bytes, ChildScratch::total(1, slots));
+        return GT_ERR_STATE;
+    }
+    int device = -1;
+    GT_CUDA(cudaGetDevice(&device));
+    auto it = t->dev.find(device);
+    if (it == t->dev.end()) { set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    const PlanView& v = it->second->view;
+    const size_t in_size = A.in_type == GT_F64 ? 8 : A.in_type == GT_F32 ? 4 : 2;
+    const int64_t max_blocks = (t->layout.V + kChildBlock - 1) / kChildBlock;
+    const int resident = sm_count() * resident_ctas(reinterpret_cast<const void*>(child_block_kernel), kChildThreads, 0);
+    A.blk_off = sc.blk_off; A.part_sum = sc.part_sum; A.part_max = sc.part_max; A.slots = slots;
+    const char* ws0 = static_cast<const char*>(A.ws);
+    const int32_t* nodes0 = A.nodes;
+    ChildArgs C = A;
+    NvtxRange nv("gt:child");
+    for (int64_t r0 = 0; r0 < n_rows; r0 += sc.rows) {
+        const int rows = (int)std::min<int64_t>(sc.rows, n_rows - r0);
+        C.n_rows = rows;
+        C.ws = ws0 + (size_t)r0 * A.ld_ws * in_size;
+        C.nodes = nodes0 + r0;
+        const size_t o = (size_t)r0 * out_ld_rows;
+        if (A.child_ids) C.child_ids = A.child_ids + o;
+        if (A.out_sum) C.out_sum = A.out_sum + o;
+        if (A.out_max) C.out_max = A.out_max + o;
+        if (A.child_out) { C.child_out = A.child_out + r0; C.logp_out = A.logp_out + r0; C.logZ_out = A.logZ_out + r0; }
+        C.ctr0 = offset + (uint64_t)r0;
+        const int64_t blocks_ub = (int64_t)rows * max_blocks;  // every row at the root
+        const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(resident, (blocks_ub + kChildThreads / 32 - 1) / (kChildThreads / 32)));
+        GT_CUDA(launch_pdl(child_scan_kernel, dim3(1), dim3(1024), 0, st, v, C));
+        GT_CUDA(launch_pdl(child_block_kernel, dim3(grid), dim3(kChildThreads), 0, st, v, C));
+        GT_CUDA(launch_pdl(child_finish_kernel, dim3((unsigned)((rows + kChildThreads / 32 - 1) / (kChildThreads / 32))),
+                           dim3(kChildThreads), 0, st, v, C));
+    }
+    return GT_OK;
+}
 }  // namespace gt
 
 extern "C" {
@@ -1254,6 +1635,64 @@ int gt_subtree_token_mask(const gt_trie* t, const int32_t* nodes, int64_t n_rows
     gt::subtree_mask_kernel<<<grid, gt::kMaskThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, nodes, (int)n_rows, mask_bits, mask_ld);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
+}
+
+size_t gt_child_workspace_bytes(const gt_trie* t, int64_t max_rows) {
+    if (!t || max_rows <= 0) return 0;
+    return gt::ChildScratch::total(std::min<int64_t>(max_rows, gt::kMaxChildRows), gt::ChildScratch::slots(t->layout)) + 256;
+}
+
+static bool child_in_type_ok(int in_type) { return in_type == GT_F32 || in_type == GT_F64 || in_type == GT_F16 || in_type == GT_BF16; }
+
+int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                    int32_t* child_ids, float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                    void* workspace, size_t workspace_bytes, gt_stream stream) {
+    if (!t) { gt::set_error("gt_child_masses: null trie"); return GT_ERR_ARG; }
+    const unsigned known = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
+    if (n_rows < 0 || !(ops & (GT_OP_SUM | GT_OP_MAX)) || (ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX)) || (flags & ~known) ||
+        !child_in_type_ok(in_type)) {
+        gt::set_error("gt_child_masses: bad n_rows / ops / flags / input type"); return GT_ERR_ARG;
+    }
+    const int64_t D = t->layout.max_children;
+    if (ld_ws < t->layout.V || ld_out < D) {
+        gt::set_error("gt_child_masses: row stride smaller than row length (ld_ws=%lld V=%lld ld_out=%lld D=%lld)",
+                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_out, (long long)D);
+        return GT_ERR_ARG;
+    }
+    if (n_rows == 0 || D == 0) return GT_OK;
+    if ((t->layout.V > 0 && !ws) || !nodes || !child_ids || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
+        gt::set_error("gt_child_masses: null data pointer"); return GT_ERR_ARG;
+    }
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_child_masses: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
+    gt::ChildArgs A{};
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
+    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
+    A.nodes = nodes; A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
+    A.child_ids = child_ids; A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr;
+    A.ld_out = ld_out; A.D = (int)D;
+    A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), "gt_child_masses");
+}
+
+int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                    unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out,
+                    void* workspace, size_t workspace_bytes, gt_stream stream) {
+    if (!t) { gt::set_error("gt_child_sample: null trie"); return GT_ERR_ARG; }
+    if (n_rows < 0 || (flags & ~(unsigned)(GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER)) || !child_in_type_ok(in_type)) {
+        gt::set_error("gt_child_sample: bad n_rows / flags / input type"); return GT_ERR_ARG;
+    }
+    if (ld_ws < t->layout.V) { gt::set_error("gt_child_sample: row stride %lld smaller than V = %lld", (long long)ld_ws, (long long)t->layout.V); return GT_ERR_ARG; }
+    if (n_rows == 0) return GT_OK;
+    if ((t->layout.V > 0 && !ws) || !nodes || !child_out || !logp_out || !logZ_out) {
+        gt::set_error("gt_child_sample: null data pointer"); return GT_ERR_ARG;
+    }
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_child_sample: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
+    gt::ChildArgs A{};
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
+    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
+    A.nodes = nodes; A.need_max = 0;
+    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), "gt_child_sample");
 }
 
 }  // extern "C"

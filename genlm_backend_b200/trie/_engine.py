@@ -51,7 +51,9 @@ class TrieEngine:
         self.nnz = int(lib.gt_num_reach(handle))
         self._uploaded = set()
         self._workspaces = {}
+        self._child_workspaces = {}
         self._ld32 = None
+        self.max_children = int(lib.gt_max_children(handle))  # D: columns of the child read-outs
 
     def __del__(self):
         h = getattr(self, "_handle", None)
@@ -109,14 +111,23 @@ class TrieEngine:
         (device, stream): calls on one stream are ordered, so they may share it; calls on different streams (or
         threads using different streams) never do."""
         need = int(lib.gt_workspace_bytes(self._handle, min(max(rows, 1), _WORKSPACE_ROWS)))
+        return self._scratch(self._workspaces, need, index, stream)
+
+    def _child_workspace(self, index, stream, rows):
+        """Scratch of ``gt_child_masses`` / ``gt_child_sample``, cached per (device, stream) like ``_workspace``."""
+        need = int(lib.gt_child_workspace_bytes(self._handle, min(max(rows, 1), _WORKSPACE_ROWS)))
+        return self._scratch(self._child_workspaces, need, index, stream)
+
+    @staticmethod
+    def _scratch(cache, need, index, stream):
         key = (index, int(stream or 0))
-        buf = self._workspaces.get(key)
+        buf = cache.get(key)
         if buf is None or buf.numel() < need:
-            if buf is None and len(self._workspaces) >= _MAX_WORKSPACES:
-                self._workspaces.pop(next(iter(self._workspaces)))  # the caching allocator keeps the block stream-ordered
+            if buf is None and len(cache) >= _MAX_WORKSPACES:
+                cache.pop(next(iter(cache)))  # the caching allocator keeps the block stream-ordered
             # allocated on `stream` (the caller made it current), so a later reuse of the block is ordered after our kernels
             buf = torch.empty(max(need, 4096), dtype=torch.uint8, device=torch.device("cuda", index))
-            self._workspaces[key] = buf
+            cache[key] = buf
         return buf
 
     def row_stride(self, dtype=torch.float32):
@@ -288,3 +299,73 @@ class TrieEngine:
                     "gt_subtree_token_mask",
                 )
         return bits
+
+    # ---- child masses of one node per row, straight from the rows -----------------------------------------------
+    def _child_inputs(self, ws, nodes):
+        """Checks shared by the child read-outs (those of ``reduce``, plus one node id per row)."""
+        require_cuda()
+        if not (isinstance(ws, torch.Tensor) and ws.is_cuda and ws.dim() == 2):
+            raise ValueError("expected a 2-D CUDA tensor of rows")
+        if ws.shape[1] != self.V:
+            raise AssertionError([ws.shape[1], self.V])
+        if ws.dtype not in _IN_TYPES:
+            ws = ws.to(torch.float32)
+        B = ws.shape[0]
+        if (ws.shape[1] > 1 and ws.stride(1) != 1) or (B > 1 and ws.stride(0) < self.V):
+            ws = ws.contiguous()
+        nodes = torch.as_tensor(nodes)
+        if nodes.dim() != 1 or nodes.shape[0] != B:
+            raise ValueError(f"nodes must be 1-D with one node id per row ({B}), got shape {tuple(nodes.shape)}")
+        nodes = nodes.to(device=ws.device, dtype=torch.int32).contiguous()
+        self.ensure_device(ws.device.index)
+        return ws, nodes, B, (ws.stride(0) if B > 1 else max(self.V, 1))
+
+    def child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """``gt_child_masses`` on the current stream of the input's device.  Returns ``(child_ids int32[B, D],
+        sums float32[B, D] | None, maxes float32[B, D] | None)``; nothing is synchronised."""
+        ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
+        opmask = 0
+        for op in ops:
+            opmask |= OPS[op]
+        D, dev = self.max_children, ws.device
+        ids = torch.empty((B, D), dtype=torch.int32, device=dev)
+        sums = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
+        maxes = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
+        flags = ((_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
+                 | (_lib.GT_CHILD_NORMALIZE if normalize else 0) | (_lib.GT_CHILD_LOG if log else 0))
+        if B and D:
+            with torch.cuda.device(dev.index):
+                stream = torch.cuda.current_stream(dev.index).cuda_stream
+                work = self._child_workspace(dev.index, stream, B)
+                check(
+                    lib.gt_child_masses(
+                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), ids.data_ptr(),
+                        sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None,
+                        D, opmask, flags, work.data_ptr(), work.numel(), stream,
+                    ),
+                    "gt_child_masses",
+                )
+        return ids, sums, maxes
+
+    def child_sample(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False):
+        """``gt_child_sample`` on the current stream of the input's device: ``(child int32[B], logp float32[B],
+        logZ float32[B])``; nothing is synchronised."""
+        ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
+        dev = ws.device
+        child = torch.empty(B, dtype=torch.int32, device=dev)
+        logp = torch.empty(B, dtype=torch.float32, device=dev)
+        logZ = torch.empty(B, dtype=torch.float32, device=dev)
+        flags = (_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
+        if B:
+            with torch.cuda.device(dev.index):
+                stream = torch.cuda.current_stream(dev.index).cuda_stream
+                work = self._child_workspace(dev.index, stream, B)
+                check(
+                    lib.gt_child_sample(
+                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), flags,
+                        int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(), logp.data_ptr(),
+                        logZ.data_ptr(), work.data_ptr(), work.numel(), stream,
+                    ),
+                    "gt_child_sample",
+                )
+        return child, logp, logZ

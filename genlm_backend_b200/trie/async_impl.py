@@ -10,7 +10,8 @@ requests while a batch's kernels and copies are in flight -- the next drain pick
 One batch is in flight at a time (the GPU pipeline inside a batch already overlaps H2D, kernels and D2H).  Every future of
 a ``weight_sum`` / ``weight_max`` request resolves to its own float32 numpy row backed by a page-locked block of at most
 32 rows.  ``weight_sum_at`` / ``weight_max_at`` are the sparse read-out for SMC callers that need a few nodes per request:
-the ``[B, N]`` slab never leaves the GPU.
+the ``[B, N]`` slab never leaves the GPU.  ``child_masses`` is the read-out of a character-level sampler: the masses of
+one node's children per request, computed from the leaves under that node only.
 """
 import asyncio
 import logging
@@ -78,6 +79,13 @@ class AsyncTokenCharacterTrie:
         future = await self._queue_request((ws, ids, None), op)
         return await future
 
+    async def child_masses(self, ws, node, normalize=False, log=False):
+        """Masses of the children of ``node`` under the weights ``ws`` -> ``(child_ids int32[deg], masses float32[deg])``,
+        in ``jump[node]`` order (``ParallelTokenCharacterTrie.batch_child_masses``: only the leaves under the node are
+        read).  Concurrent requests with the same ``normalize`` / ``log`` share one batched call."""
+        future = await self._queue_request((ws, int(node)), ("child", bool(normalize), bool(log)))
+        return await future
+
     def start(self):
         """Start the background task (binds a fresh queue to the running loop)."""
         if not self._task or self._task.done():
@@ -105,6 +113,14 @@ class AsyncTokenCharacterTrie:
             return self.trie.batch_weight_sum_at(rows, ids, normalizer=norm, log=log)
         return self.trie.batch_weight_max_at(rows, ids, log=log)
 
+    def _do_child(self, op, requests):
+        _, normalize, log = op
+        rows = self.trie._preprocess_ws([r[0] for r in requests])
+        nodes = np.asarray([r[1] for r in requests], dtype=np.int32)
+        ids, masses, _ = self.trie.batch_child_masses(rows, nodes, normalize=normalize, log=log)
+        degs = (ids >= 0).sum(axis=1)  # padding columns come last
+        return [(ids[b, :d], masses[b, :d]) for b, d in enumerate(degs.tolist())]
+
     def _run_group(self, op, requests):
         """One batched call (worker thread)."""
         if op == "sum":
@@ -116,6 +132,9 @@ class AsyncTokenCharacterTrie:
         if isinstance(op, tuple) and op[0] in ("sum_at", "max_at") and hasattr(self.trie, "batch_weight_sum_at"):
             logger.debug(f"processing {len(requests)} {op[0]} requests")
             return self._do_at(op, requests)
+        if isinstance(op, tuple) and op[0] == "child" and hasattr(self.trie, "batch_child_masses"):
+            logger.debug(f"processing {len(requests)} child-mass requests")
+            return self._do_child(op, requests)
         raise ValueError(f"Unknown operation: {op}")
 
     async def _background_loop(self):

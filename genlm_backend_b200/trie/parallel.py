@@ -208,6 +208,75 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         an ``int32[B, ceil(V/32)]`` device tensor in the bit-mask layout of ``smc.masked_logsumexp_sample``."""
         return self._engine.subtree_token_mask(nodes, device=device)
 
+    # ---- child masses of one node per row (the next-symbol distribution of a character-level sampler) ------------
+    @property
+    def max_children(self):
+        """``D``: the largest child count of any node, the width of the child read-outs."""
+        return self._engine.max_children
+
+    @property
+    def edge_labels(self):
+        """``int32[N]``: label of the edge into each node: a symbol ``>= 0``; ``-1 - i`` for the leaf of item ``i``
+        ("token ``i`` ends here"); ``INT32_MIN`` for the root."""
+        return self._layout["edge_label"]
+
+    def _child_rows(self, ws):
+        if isinstance(ws, torch.Tensor) and ws.dim() == 2 and ws.dtype in (torch.float16, torch.bfloat16, torch.float32, torch.float64):
+            assert ws.shape[1] == len(self.decode), [ws.shape[1], len(self.decode)]
+        else:
+            ws = self._as_batch(ws)
+        if not ws.is_cuda:
+            ws = ws.to(torch.device("cuda", self._device_list()[0]), non_blocking=True)
+        return ws
+
+    def batch_child_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """Masses of the children of one node per row, computed from the rows alone (the ``[B, N]`` slab is never
+        formed; only the leaves under ``nodes[b]`` are read).
+
+        Returns ``(child_ids int32[B, D], sums float32[B, D] | None, maxes float32[B, D] | None)`` on the input's device,
+        on its current stream, without a sync.  Column ``j`` is child ``jump[nodes[b]][j]``; columns past the node's
+        degree are padding (id ``-1``, mass 0 -- ``-inf`` with ``log``); an invalid id or a leaf gives a padding row.
+        Sums are accumulated in fp64 and rounded once; ``normalize`` divides them by the node's mass (the conditional
+        next-symbol distribution); ``log`` returns logs of both.  Maxes equal ``batch_weight_max_tensor(ws)`` at the ids.
+        ``dfs_order`` as for ``batch_weight_tensor``."""
+        return self._engine.child_masses(self._child_rows(ws), nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
+                                         normalize=normalize, log=log)
+
+    def batch_child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """``batch_child_masses_tensor`` as numpy arrays."""
+        out = self.batch_child_masses_tensor(ws, nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
+                                             normalize=normalize, log=log)
+        return tuple(None if t is None else t.cpu().numpy() for t in out)
+
+    def _edge_labels_on(self, device):
+        cache = self.__dict__.setdefault("_edge_label_dev", {})
+        lab = cache.get(device.index)
+        if lab is None:
+            lab = cache[device.index] = torch.from_numpy(self.edge_labels).to(device)
+        return lab
+
+    def sample_next_symbol(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False, check_valid=False):
+        """One draw of the next symbol per row from the children of ``nodes[b]``, in proportion to their masses.
+
+        Returns ``(child, label, logp, logZ)`` device tensors: the chosen child (int32), its ``edge_labels`` entry (a
+        symbol, or ``-1 - i`` when the draw ends token ``i``), ``log mass(child) - log mass(node)`` and ``log mass(node)``.
+        Row ``b`` uses the Philox counter ``offset + b`` under key ``seed`` (as ``smc.masked_logsumexp_sample``).  A row
+        without mass (also a leaf or an invalid id) gives ``child = -1``, ``label = INT32_MIN`` and ``logZ = -inf``; a NaN
+        weight under the node gives ``logZ = NaN``.  ``check_valid``: synchronise and raise ``RuntimeError`` like
+        ``torch.multinomial`` when a row has no mass or a NaN."""
+        ws = self._child_rows(ws)
+        child, logp, logZ = self._engine.child_sample(ws, nodes, seed=seed, offset=offset, log_input=log_input,
+                                                      dfs_order=dfs_order)
+        lab = self._edge_labels_on(child.device)
+        label = torch.where(child >= 0, lab[child.clamp(min=0).long()], torch.full_like(child, np.iinfo(np.int32).min))
+        if check_valid and child.numel():
+            bad = child < 0
+            if bool(bad.any()):
+                if bool(torch.isnan(logZ[bad]).any()):
+                    raise RuntimeError("probability tensor contains either `inf`, `nan` or element < 0")
+                raise RuntimeError("invalid multinomial distribution (sum of probabilities <= 0)")
+        return child, label, logp, logZ
+
     # ---- reference API: numpy results on the host --------------------------------------------------------------
     def _pipe_streams(self, index):
         if index not in self._streams:

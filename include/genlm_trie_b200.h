@@ -19,6 +19,10 @@
  *                               (masked logsumexp + multinomial of the SMC particle step)
  *   gt_gather_nodes             genlm/backend/trie/parallel.py:103,145 (the .cpu().numpy() of the whole slab)
  *   gt_subtree_token_mask       genlm/backend/trie/parallel.py:33-64 (a column of the reachability matrix)
+ *   gt_child_masses             genlm/backend/trie/parallel.py:92-103 (batch_weight_sum) followed by indexing
+ *                               children(node) of the result on the host: the next-symbol masses of a
+ *                               character-level sampler, without the [B, N] slab
+ *   gt_child_sample             the same, plus one categorical draw of the next symbol per row
  *
  * Conventions
  *   - every function returns 0 on success, non-zero on failure; gt_last_error() returns a
@@ -207,6 +211,46 @@ int gt_download_rows(void* dst_host, size_t dst_pitch, const void* src_dev, size
  * nodes / mask_bits: device; mask_ld >= ceil(V/32) words per row, every word of the first ceil(V/32) is written. */
 int gt_subtree_token_mask(const gt_trie* t, const int32_t* nodes, int64_t n_rows, uint32_t* mask_bits,
                           int64_t mask_ld, gt_stream stream);
+
+/* ---- child masses of one node per row, straight from the rows ------------------------------ */
+
+/* D: the largest child count of any node (host only, no GPU needed); -1 for a null trie. */
+int64_t gt_max_children(const gt_trie* t);
+
+/* Caller-owned scratch of gt_child_masses / gt_child_sample for batches of up to max_rows rows (capped at 1,024: larger
+ * batches, or a smaller workspace, are processed in chunks; any size that holds one row works).  Host only.  One call at
+ * a time may use a workspace; the pointer must be 256-byte aligned. */
+size_t gt_child_workspace_bytes(const gt_trie* t, int64_t max_rows);
+
+#define GT_CHILD_NORMALIZE 0x10u /* divide each child's sum by the node's mass (the fp64 sum over its children) */
+#define GT_CHILD_LOG 0x20u       /* return log-masses (sum and max) */
+
+/* For each row b and the node n = nodes[b] (device int32), with the children c_0 < c_1 < ... of n in jump[n] order:
+ *   child_ids[b, j] = c_j
+ *   out_sum[b, j]   = sum of the row's weights over the leaves under c_j
+ *   out_max[b, j]   = max of the row's weights over the same leaves
+ * for j < deg(n); columns deg(n) <= j < D (D = gt_max_children) are padding: child id -1 and the value of no mass,
+ * 0 (-inf with GT_CHILD_LOG).  A node id < 0 or >= N, or a leaf, gives an all-padding row.
+ *   ws, in_type, ld_ws, GT_FLAG_LOG_INPUT, GT_FLAG_DFS_ORDER   as for gt_weight_reduce
+ *   child_ids / out_sum / out_max   device, row stride ld_out >= D elements; out_sum / out_max may be NULL when the
+ *                                   op is not in `ops` (GT_OP_SUM | GT_OP_MAX)
+ *   flags    GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG
+ * Numerics: each weight is converted exactly as gt_weight_reduce converts it (so out_max is bit-equal to its fp32 max
+ * slab at child_ids); sums are accumulated in fp64 in an order that depends only on (node, child) -- not on the batch,
+ * the row order, the workspace or the input order -- and rounded once.  Only the leaves under nodes[b] are read. */
+int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                    int32_t* child_ids, float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                    void* workspace, size_t workspace_bytes, gt_stream stream);
+
+/* One draw of the next symbol per row: u = 53-bit Philox4x32-10 uniform (counter offset + b, key seed, as
+ * gt_lse_sample), m_j = the fp64 child sums of gt_child_masses, total = sum_j m_j; the chosen child is the first j whose
+ * running sum exceeds u * total (a child without mass is never chosen).
+ *   child_out[b] = c_j,  logp_out[b] = log m_j - log total,  logZ_out[b] = log total (the node's mass)
+ * A row without mass (also a leaf or an invalid node id) gives child -1 and logp = logZ = -inf; a NaN weight under the
+ * node gives child -1 and logp = logZ = NaN.  flags: GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER. */
+int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                    unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out,
+                    void* workspace, size_t workspace_bytes, gt_stream stream);
 
 #ifdef __cplusplus
 }
