@@ -62,6 +62,11 @@ SIGNATURES = {
                                 c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
     "gt_child_sample": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_uint, c_uint64, c_uint64, c_void_p,
                                 c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gt_num_symbols": (c_int64, [c_void_p]),
+    "gt_symbol_masses": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                 c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
+    "gt_symbol_sample": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_uint, c_uint64,
+                                 c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "gt_lse_sample": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_float,
                               c_uint64, c_uint64, c_void_p, c_void_p, c_void_p]),
 }

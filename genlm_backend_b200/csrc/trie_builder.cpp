@@ -75,13 +75,14 @@ static int build_layout(const int32_t* symbols, const int64_t* offsets, int64_t 
 
     EdgeTable table((size_t)total);
     std::vector<int32_t> leaf_old((size_t)V);
-    int64_t max_depth = 0;
+    int64_t max_depth = 0, num_symbols = 256;
     for (int64_t i = 0; i < V; ++i) {
         if (offsets[i + 1] < offsets[i]) { set_error("offsets must be non-decreasing"); return GT_ERR_ARG; }
         int32_t cur = 0;
         for (int64_t k = offsets[i]; k < offsets[i + 1]; ++k) {
             const int32_t sym = symbols[k];
             if (sym < 0) { set_error("negative symbol at item %lld", (long long)i); return GT_ERR_ARG; }
+            if ((int64_t)sym + 1 > num_symbols) num_symbols = (int64_t)sym + 1;
             const uint64_t key = ((uint64_t)(uint32_t)cur << 32) | (uint32_t)sym;
             const size_t slot = table.find(key);
             if (table.keys[slot] == EdgeTable::EMPTY) {
@@ -121,7 +122,7 @@ static int build_layout(const int32_t* symbols, const int64_t* offsets, int64_t 
         }
     }
 
-    L.V = V; L.N = N; L.max_depth = max_depth;
+    L.V = V; L.N = N; L.max_depth = max_depth; L.num_symbols = num_symbols;
     L.leaf_node.resize((size_t)V);
     L.parent.assign((size_t)N, -1);
     L.edge_label.resize((size_t)N);
@@ -189,6 +190,7 @@ int64_t gt_root(const gt_trie* t) { return t ? t->layout.N - 1 : -1; }
 int64_t gt_num_reach(const gt_trie* t) { return t ? t->layout.nnz : -1; }
 int64_t gt_max_depth(const gt_trie* t) { return t ? t->layout.max_depth : -1; }
 int64_t gt_max_children(const gt_trie* t) { return t ? t->layout.max_children : -1; }
+int64_t gt_num_symbols(const gt_trie* t) { return t ? t->layout.num_symbols : -1; }
 
 int gt_export_layout(const gt_trie* t, int32_t* leaf_node, int32_t* parent, int32_t* edge_label,
                      int32_t* child_ptr, int32_t* child_idx, int32_t* perm, int32_t* lo, int32_t* hi) {

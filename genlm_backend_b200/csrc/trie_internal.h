@@ -30,6 +30,7 @@ struct NvtxRange {
 struct Layout {
     int64_t V = 0, N = 0, nnz = 0, max_depth = 0;
     int64_t max_children = 0;         // D: largest child count of any node
+    int64_t num_symbols = 256;        // S = max(256, 1 + largest symbol); column S of the symbol read-outs is end of token
     std::vector<int32_t> leaf_node;   // [V]
     std::vector<int32_t> parent;      // [N]
     std::vector<int32_t> edge_label;  // [N]

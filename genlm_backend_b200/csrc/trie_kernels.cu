@@ -52,6 +52,8 @@ struct PlanView {
     const int32_t* node_lo; const int32_t* node_hi;  // [N] DFS leaf range of every node
     const int32_t* perm;       // [V] DFS rank -> item position (Layout::perm)
     const int32_t* child_ptr; const int32_t* child_idx;  // children CSR (ascending ids = jump[] order)
+    const int32_t* child_sym;  // [N - 1] beside child_idx: the child's edge symbol, S for a leaf child
+    int32_t S;                 // Layout::num_symbols
     int32_t debug_stop;  // profiling aid (GT_DEBUG_STOP): 0 = normal; 3 = no emit stores; 9 = emit only
     long long* trace;    // profiling aid (GT_TRACE=1): per (CTA, item) SM-clock stamps of the pipeline events, else null
 };
@@ -793,6 +795,12 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
     for (int64_t r = 0; r < L.V; ++r) leaf_rank[(size_t)L.perm[(size_t)r]] = (int32_t)r;
     const size_t o_leaf_rank = ADDV(leaf_rank), o_node_lo = ADDV(L.lo), o_node_hi = ADDV(L.hi);
     const size_t o_perm = ADDV(L.perm), o_child_ptr = ADDV(L.child_ptr), o_child_idx = ADDV(L.child_idx);
+    std::vector<int32_t> child_sym(L.child_idx.size());
+    for (size_t e = 0; e < child_sym.size(); ++e) {
+        const int32_t lab = L.edge_label[(size_t)L.child_idx[e]];
+        child_sym[e] = lab >= 0 ? lab : (int32_t)L.num_symbols;  // leaf child: -1 - item
+    }
+    const size_t o_child_sym = ADDV(child_sym);
 #undef ADDV
     total += 256;
 
@@ -846,6 +854,7 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
     v.node_lo = (const int32_t*)(base + o_node_lo); v.node_hi = (const int32_t*)(base + o_node_hi);
     v.perm = (const int32_t*)(base + o_perm);
     v.child_ptr = (const int32_t*)(base + o_child_ptr); v.child_idx = (const int32_t*)(base + o_child_idx);
+    v.child_sym = (const int32_t*)(base + o_child_sym); v.S = (int32_t)L.num_symbols;
     { const char* e = getenv("GT_DEBUG_STOP"); v.debug_stop = e && *e ? atoi(e) : 0; }
     v.trace = nullptr;
     if (const char* e = getenv("GT_TRACE")) {
@@ -1136,6 +1145,8 @@ struct ChildArgs {
     int32_t* child_ids; float* out_sum; float* out_max; int64_t ld_out; int D; int normalize, log_out;
     // finish, draw (child_out != null)
     int32_t* child_out; float* logp_out; float* logZ_out; uint64_t seed, ctr0;  // ctr0 = offset + first row of the chunk
+    // symbol_finish_kernel: draw under per-row symbol log-weights (row stride ld_w, 0 = shared)
+    const float* sym_logw; int64_t ld_w; int32_t* symbol_out; float* logM_out;
 };
 
 // Children CSR range and DFS leaf range of node n; false for an id outside [0, N) and for a leaf.
@@ -1305,6 +1316,65 @@ __global__ void __launch_bounds__(kChildThreads, 3) child_block_kernel(PlanView 
     }
 }
 
+// The slots of row b seen from a finish kernel: child j's sum (its blocks' fp64 partials added in k order) and max.
+struct ChildSlots {
+    const PlanView& P; const int32_t* ch; const double* psum; const float* pmax; int lo;
+    __device__ __forceinline__ void blocks(int c, int& k0, int& k1) const {  // the blocks child c overlaps
+        k0 = (__ldg(P.node_lo + c) - lo) / kChildBlock;
+        k1 = (__ldg(P.node_hi + c) - 1 - lo) / kChildBlock;
+    }
+    __device__ __forceinline__ double sum(int j) const {
+        int k0, k1;
+        blocks(__ldg(ch + j), k0, k1);
+        double s = 0.0;
+        for (int k = k0; k <= k1; ++k) s += psum[j + k];
+        return s;
+    }
+    __device__ __forceinline__ float max(int j) const {
+        int k0, k1;
+        blocks(__ldg(ch + j), k0, k1);
+        float m = -INFINITY;
+        for (int k = k0; k <= k1; ++k) m = fmaxf(m, pmax[j + k]);
+        return m;
+    }
+};
+
+// The draw of a finish kernel: the first child whose running sum of terms q(j) exceeds target (= u * total, total > 0
+// and finite), else -- rounding pushed the target past the running sums -- the last child with q(j) > 0.  Lane l owns
+// the children [j_lo, j_hi); local is the sum of their terms, incl its inclusive scan over the lanes.  Returns the
+// child's position j and its term in `term`.
+template <typename Q>
+__device__ __forceinline__ int pick_child(const Q& q, int j_lo, int j_hi, double local, double incl, double target, int lane,
+                                          double& term) {
+    int pick = -1;
+    double mass = 0.0;
+    const unsigned hit = __ballot_sync(0xffffffffu, incl > target && local > 0.0);
+    if (hit) {
+        const int src = __ffs(hit) - 1;
+        if (lane == src) {
+            double run = incl - local;
+            for (int j = j_lo; j < j_hi; ++j) {
+                const double s = q(j);
+                if (s > 0.0) { pick = j; mass = s; if (run + s > target) break; }
+                run += s;
+            }
+        }
+        pick = __shfl_sync(0xffffffffu, pick, src);
+        mass = __shfl_sync(0xffffffffu, mass, src);
+    } else {
+        int last = -1;
+        if (local > 0.0)
+            for (int j = j_hi - 1; j >= j_lo; --j)
+                if (q(j) > 0.0) { last = j; break; }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+        pick = last;
+        mass = q(pick);  // last >= 0: total > 0
+    }
+    term = mass;
+    return pick;
+}
+
 // One warp per row.  Lane l owns the contiguous children [j_lo, j_hi) of the row's node; their sums are added in order
 // and an inclusive scan over the lanes gives the running sums and the node's mass (fixed order: normalisation and draw
 // see the same total).
@@ -1317,23 +1387,11 @@ __global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P,
     int cp0 = 0, deg = 0, lo = 0, hi = 0;
     if (!child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi)) deg = 0;
     const int32_t* ch = P.child_idx + cp0;
-    const double* psum = A.part_sum + (size_t)b * A.slots;
-    const float* pmax = A.part_max + (size_t)b * A.slots;
-    auto blocks = [&](int c, int& k0, int& k1) {  // the blocks child c overlaps
-        k0 = (__ldg(P.node_lo + c) - lo) / kChildBlock;
-        k1 = (__ldg(P.node_hi + c) - 1 - lo) / kChildBlock;
-    };
-    auto child_sum = [&](int j) {
-        int k0, k1;
-        blocks(__ldg(ch + j), k0, k1);
-        double s = 0.0;
-        for (int k = k0; k <= k1; ++k) s += psum[j + k];
-        return s;
-    };
+    const ChildSlots cs{P, ch, A.part_sum + (size_t)b * A.slots, A.part_max + (size_t)b * A.slots, lo};
     const int per = (deg + 31) / 32;
     const int j_lo = min(deg, lane * per), j_hi = min(deg, j_lo + per);
     double local = 0.0;
-    for (int j = j_lo; j < j_hi; ++j) local += child_sum(j);
+    for (int j = j_lo; j < j_hi; ++j) local += cs.sum(j);
     double incl = local;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -1350,15 +1408,12 @@ __global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P,
             const int c = __ldg(ch + j);
             ids[j] = c;
             if (os) {
-                double s = child_sum(j);
+                double s = cs.sum(j);
                 if (A.normalize) s /= total;
                 os[j] = (float)(A.log_out ? log(s) : s);
             }
             if (om) {
-                int k0, k1;
-                blocks(c, k0, k1);
-                float m = -INFINITY;
-                for (int k = k0; k <= k1; ++k) m = fmaxf(m, pmax[j + k]);
+                const float m = cs.max(j);
                 om[j] = A.log_out ? (float)log((double)m) : m;
             }
         }
@@ -1375,32 +1430,9 @@ __global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P,
     const bool ok = total > 0.0 && total < (double)INFINITY;  // false for NaN
     int pick = -1;
     double mass = 0.0;
-    if (ok) {
-        const double target = philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total;
-        const unsigned hit = __ballot_sync(0xffffffffu, incl > target && local > 0.0);
-        if (hit) {
-            const int src = __ffs(hit) - 1;
-            if (lane == src) {
-                double run = incl - local;
-                for (int j = j_lo; j < j_hi; ++j) {
-                    const double s = child_sum(j);
-                    if (s > 0.0) { pick = j; mass = s; if (run + s > target) break; }
-                    run += s;
-                }
-            }
-            pick = __shfl_sync(0xffffffffu, pick, src);
-            mass = __shfl_sync(0xffffffffu, mass, src);
-        } else {  // rounding pushed the target past the running sums: the last child with mass
-            int last = -1;
-            if (local > 0.0)
-                for (int j = j_hi - 1; j >= j_lo; --j)
-                    if (child_sum(j) > 0.0) { last = j; break; }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
-            pick = last;
-            mass = child_sum(pick);  // last >= 0: total > 0
-        }
-    }
+    if (ok)
+        pick = pick_child([&](int j) { return cs.sum(j); }, j_lo, j_hi, local, incl,
+                          philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total, lane, mass);
     if (lane == 0) {
         A.child_out[b] = ok ? __ldg(ch + pick) : -1;
         A.logZ_out[b] = (float)log(total);  // -inf for no mass, NaN for a NaN weight
@@ -1408,6 +1440,105 @@ __global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P,
     }
 }
 
+
+// ---- the same, indexed by symbol (gt_symbol_masses / gt_symbol_sample) --------------------------------------------
+// Same slots, same lane split and scan as child_finish_kernel, so every per-child sum, the node's mass and the draw of
+// gt_child_sample are reproduced bit for bit; child j goes to column child_sym[j] (S for a leaf child).  Masses: the
+// row is first filled with padding, then each non-leaf child writes its own column (a node has one child per symbol),
+// and column S gets the leaf children's sums added in child order.  Draw: q_j = m_j * exp(logw[sym_j]) in fp64,
+// scanned like the m_j.
+__global__ void __launch_bounds__(kChildThreads) symbol_finish_kernel(PlanView P, ChildArgs A) {
+    pdl_wait();  // the slots come from child_block_kernel
+    pdl_trigger();
+    const int lane = threadIdx.x & 31;
+    const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
+    if (b >= A.n_rows) return;
+    int cp0 = 0, deg = 0, lo = 0, hi = 0;
+    if (!child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi)) deg = 0;
+    const int32_t* ch = P.child_idx + cp0;
+    const int32_t* sy = P.child_sym + cp0;
+    const int S = P.S;
+    const ChildSlots cs{P, ch, A.part_sum + (size_t)b * A.slots, A.part_max + (size_t)b * A.slots, lo};
+    const int per = (deg + 31) / 32;
+    const int j_lo = min(deg, lane * per), j_hi = min(deg, j_lo + per);
+    auto scan = [&](double local) {  // inclusive, over the lanes (the order of child_finish_kernel)
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const double y = __shfl_up_sync(0xffffffffu, local, o);
+            if (lane >= o) local += y;
+        }
+        return local;
+    };
+    double local_m = 0.0;
+    for (int j = j_lo; j < j_hi; ++j) local_m += cs.sum(j);
+    const double incl_m = scan(local_m);
+    const double total_m = __shfl_sync(0xffffffffu, incl_m, 31);
+
+    if (!A.child_out) {
+        float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
+        float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
+        const float pad = A.log_out ? -INFINITY : 0.f;
+        for (int s = lane; s <= S; s += 32) {
+            if (os) os[s] = pad;
+            if (om) om[s] = pad;
+        }
+        __syncwarp();  // the children's columns overwrite the padding
+        auto put = [&](int col, double sum, float mx) {
+            if (os) {
+                if (A.normalize) sum /= total_m;
+                os[col] = (float)(A.log_out ? log(sum) : sum);
+            }
+            if (om) om[col] = A.log_out ? (float)log((double)mx) : mx;
+        };
+        bool has_end = false;
+        for (int j = j_lo; j < j_hi; ++j) {
+            const int sym = __ldg(sy + j);
+            if (sym == S) { has_end = true; continue; }
+            put(sym, os ? cs.sum(j) : 0.0, om ? cs.max(j) : 0.f);
+        }
+        // end of token: the leaf children, lane by lane in child order (usually one lane, one child)
+        const unsigned ends = __ballot_sync(0xffffffffu, has_end);
+        double es = 0.0;
+        float em = -INFINITY;
+        for (unsigned e = ends; e; e &= e - 1) {
+            const int src = __ffs(e) - 1;
+            if (lane == src)
+                for (int j = j_lo; j < j_hi; ++j)
+                    if (__ldg(sy + j) == S) {
+                        if (os) es += cs.sum(j);
+                        if (om) em = fmaxf(em, cs.max(j));
+                    }
+            es = __shfl_sync(0xffffffffu, es, src);
+            em = __shfl_sync(0xffffffffu, em, src);
+        }
+        if (ends && lane == 0) put(S, es, em);
+        return;
+    }
+
+    // draw under the row's symbol log-weights
+    const float* lw = A.sym_logw + (size_t)b * A.ld_w;
+    auto weighted = [&](int j) {  // q_j: no mass stays 0 whatever the weight; a NaN weight poisons the row
+        const float w = __ldg(lw + __ldg(sy + j));
+        if (isnan(w)) return (double)NAN;
+        const double m = cs.sum(j);
+        return m == 0.0 ? 0.0 : m * exp((double)w);
+    };
+    double local = 0.0;
+    for (int j = j_lo; j < j_hi; ++j) local += weighted(j);
+    const double incl = scan(local);
+    const double total = __shfl_sync(0xffffffffu, incl, 31);
+    const bool ok = total > 0.0 && total < (double)INFINITY;  // false for NaN
+    int pick = -1;
+    double mass = 0.0;
+    if (ok) pick = pick_child(weighted, j_lo, j_hi, local, incl, philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total, lane, mass);
+    if (lane == 0) {
+        A.child_out[b] = ok ? __ldg(ch + pick) : -1;
+        A.symbol_out[b] = ok ? __ldg(sy + pick) : -1;
+        A.logZ_out[b] = (float)log(total);  // -inf for no mass, NaN for a NaN weight, +inf for an infinite total
+        A.logp_out[b] = ok ? (float)(log(mass) - log(total)) : (total == 0.0 ? -INFINITY : NAN);
+        if (A.logM_out) A.logM_out[b] = (float)log(total_m);
+    }
+}
 
 // Scratch of the child-mass calls for a chunk of `rows` rows:
 //   blk_off [rows + 1] int32 | part_sum [rows][slots] fp64 | part_max [rows][slots] fp32
@@ -1436,11 +1567,13 @@ struct ChildScratch {
     }
 };
 
-// Shared by gt_child_masses and gt_child_sample: arguments are checked by the callers (before any CUDA call); this
-// selects the device plan and launches scan -> blocks -> finish per chunk of rows, chained with programmatic dependent
-// launch on the caller's stream.  A.nodes / A.ws / outputs point at row 0; chunk c advances them.
+// Shared by gt_child_masses, gt_child_sample, gt_symbol_masses and gt_symbol_sample: arguments are checked by the
+// callers (before any CUDA call); this selects the device plan and launches scan -> blocks -> finish per chunk of rows,
+// chained with programmatic dependent launch on the caller's stream.  A.nodes / A.ws / outputs point at row 0; chunk c
+// advances them.  `finish` is child_finish_kernel or symbol_finish_kernel.
 static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t out_ld_rows, uint64_t offset, void* workspace,
-                        size_t workspace_bytes, cudaStream_t st, const char* what) {
+                        size_t workspace_bytes, cudaStream_t st, const char* what,
+                        void (*finish)(PlanView, ChildArgs) = child_finish_kernel) {
     const int64_t slots = ChildScratch::slots(t->layout);
     const ChildScratch sc(workspace, workspace_bytes, slots);
     if (sc.rows < 1) {
@@ -1470,12 +1603,15 @@ static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t o
         if (A.out_sum) C.out_sum = A.out_sum + o;
         if (A.out_max) C.out_max = A.out_max + o;
         if (A.child_out) { C.child_out = A.child_out + r0; C.logp_out = A.logp_out + r0; C.logZ_out = A.logZ_out + r0; }
+        if (A.symbol_out) C.symbol_out = A.symbol_out + r0;
+        if (A.logM_out) C.logM_out = A.logM_out + r0;
+        if (A.sym_logw) C.sym_logw = A.sym_logw + (size_t)r0 * A.ld_w;
         C.ctr0 = offset + (uint64_t)r0;
         const int64_t blocks_ub = (int64_t)rows * max_blocks;  // every row at the root
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(resident, (blocks_ub + kChildThreads / 32 - 1) / (kChildThreads / 32)));
         GT_CUDA(launch_pdl(child_scan_kernel, dim3(1), dim3(1024), 0, st, v, C));
         GT_CUDA(launch_pdl(child_block_kernel, dim3(grid), dim3(kChildThreads), 0, st, v, C));
-        GT_CUDA(launch_pdl(child_finish_kernel, dim3((unsigned)((rows + kChildThreads / 32 - 1) / (kChildThreads / 32))),
+        GT_CUDA(launch_pdl(finish, dim3((unsigned)((rows + kChildThreads / 32 - 1) / (kChildThreads / 32))),
                            dim3(kChildThreads), 0, st, v, C));
     }
     return GT_OK;
@@ -1693,6 +1829,66 @@ int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_row
     A.nodes = nodes; A.need_max = 0;
     A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
     return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), "gt_child_sample");
+}
+
+int gt_symbol_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                     float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                     void* workspace, size_t workspace_bytes, gt_stream stream) {
+    if (!t) { gt::set_error("gt_symbol_masses: null trie"); return GT_ERR_ARG; }
+    const unsigned known = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
+    if (n_rows < 0 || !(ops & (GT_OP_SUM | GT_OP_MAX)) || (ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX)) || (flags & ~known) ||
+        !child_in_type_ok(in_type)) {
+        gt::set_error("gt_symbol_masses: bad n_rows / ops / flags / input type"); return GT_ERR_ARG;
+    }
+    const int64_t S = t->layout.num_symbols;
+    if (ld_ws < t->layout.V || ld_out < S + 1) {
+        gt::set_error("gt_symbol_masses: row stride smaller than row length (ld_ws=%lld V=%lld ld_out=%lld S+1=%lld)",
+                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_out, (long long)(S + 1));
+        return GT_ERR_ARG;
+    }
+    if (n_rows == 0) return GT_OK;
+    if ((t->layout.V > 0 && !ws) || !nodes || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
+        gt::set_error("gt_symbol_masses: null data pointer"); return GT_ERR_ARG;
+    }
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_symbol_masses: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
+    gt::ChildArgs A{};
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
+    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
+    A.nodes = nodes; A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
+    A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr;
+    A.ld_out = ld_out; A.D = (int)t->layout.max_children;
+    A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream),
+                            "gt_symbol_masses", gt::symbol_finish_kernel);
+}
+
+int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                     const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
+                     int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
+                     void* workspace, size_t workspace_bytes, gt_stream stream) {
+    if (!t) { gt::set_error("gt_symbol_sample: null trie"); return GT_ERR_ARG; }
+    if (n_rows < 0 || (flags & ~(unsigned)(GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER)) || !child_in_type_ok(in_type)) {
+        gt::set_error("gt_symbol_sample: bad n_rows / flags / input type"); return GT_ERR_ARG;
+    }
+    const int64_t S = t->layout.num_symbols;
+    if (ld_ws < t->layout.V || ld_w < 0 || (ld_w > 0 && ld_w < S + 1)) {
+        gt::set_error("gt_symbol_sample: row stride smaller than row length (ld_ws=%lld V=%lld ld_w=%lld S+1=%lld)",
+                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_w, (long long)(S + 1));
+        return GT_ERR_ARG;
+    }
+    if (n_rows == 0) return GT_OK;
+    if ((t->layout.V > 0 && !ws) || !nodes || !sym_logw || !child_out || !symbol_out || !logp_out || !logZ_out) {
+        gt::set_error("gt_symbol_sample: null data pointer"); return GT_ERR_ARG;
+    }
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_symbol_sample: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
+    gt::ChildArgs A{};
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
+    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
+    A.nodes = nodes; A.need_max = 0;
+    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
+    A.sym_logw = sym_logw; A.ld_w = ld_w; A.symbol_out = symbol_out; A.logM_out = logM_out;
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream),
+                            "gt_symbol_sample", gt::symbol_finish_kernel);
 }
 
 }  // extern "C"

@@ -54,6 +54,7 @@ class TrieEngine:
         self._child_workspaces = {}
         self._ld32 = None
         self.max_children = int(lib.gt_max_children(handle))  # D: columns of the child read-outs
+        self.num_symbols = int(lib.gt_num_symbols(handle))  # S: the symbol read-outs have S + 1 columns
 
     def __del__(self):
         h = getattr(self, "_handle", None)
@@ -369,3 +370,64 @@ class TrieEngine:
                     "gt_child_sample",
                 )
         return child, logp, logZ
+
+    # ---- the same, indexed by symbol ---------------------------------------------------------------------------
+    def symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """``gt_symbol_masses`` on the current stream of the input's device.  Returns ``(sums float32[B, S+1] | None,
+        maxes float32[B, S+1] | None)``; nothing is synchronised."""
+        ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
+        opmask = 0
+        for op in ops:
+            opmask |= OPS[op]
+        W, dev = self.num_symbols + 1, ws.device
+        sums = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
+        maxes = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
+        flags = ((_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
+                 | (_lib.GT_CHILD_NORMALIZE if normalize else 0) | (_lib.GT_CHILD_LOG if log else 0))
+        if B:
+            with torch.cuda.device(dev.index):
+                stream = torch.cuda.current_stream(dev.index).cuda_stream
+                work = self._child_workspace(dev.index, stream, B)
+                check(
+                    lib.gt_symbol_masses(
+                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                        sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None,
+                        W, opmask, flags, work.data_ptr(), work.numel(), stream,
+                    ),
+                    "gt_symbol_masses",
+                )
+        return sums, maxes
+
+    def symbol_sample(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False):
+        """``gt_symbol_sample`` on the current stream of the input's device: ``(child int32[B], symbol int32[B],
+        logp float32[B], logZ float32[B], logM float32[B])``; nothing is synchronised.  ``symbol_logw``: ``[S+1]``
+        (shared by all rows) or ``[B, S+1]``, converted to contiguous float32 on the input's device."""
+        ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
+        W, dev = self.num_symbols + 1, ws.device
+        logw = torch.as_tensor(symbol_logw)
+        if not (logw.dim() == 1 and logw.shape[0] == W) and not (logw.dim() == 2 and tuple(logw.shape) == (B, W)):
+            raise ValueError(f"symbol_logw must be [{W}] or [{B}, {W}] (S + 1 = {W} columns), got shape {tuple(logw.shape)}")
+        if not logw.is_floating_point():
+            raise ValueError(f"symbol_logw must hold floating-point log-weights, got {logw.dtype}")
+        logw = logw.to(device=dev, dtype=torch.float32).contiguous()
+        ld_w = 0 if logw.dim() == 1 else W
+        child = torch.empty(B, dtype=torch.int32, device=dev)
+        symbol = torch.empty(B, dtype=torch.int32, device=dev)
+        logp = torch.empty(B, dtype=torch.float32, device=dev)
+        logZ = torch.empty(B, dtype=torch.float32, device=dev)
+        logM = torch.empty(B, dtype=torch.float32, device=dev)
+        flags = (_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
+        if B:
+            with torch.cuda.device(dev.index):
+                stream = torch.cuda.current_stream(dev.index).cuda_stream
+                work = self._child_workspace(dev.index, stream, B)
+                check(
+                    lib.gt_symbol_sample(
+                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), logw.data_ptr(),
+                        ld_w, flags, int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(),
+                        symbol.data_ptr(), logp.data_ptr(), logZ.data_ptr(), logM.data_ptr(), work.data_ptr(),
+                        work.numel(), stream,
+                    ),
+                    "gt_symbol_sample",
+                )
+        return child, symbol, logp, logZ, logM

@@ -11,7 +11,8 @@ One batch is in flight at a time (the GPU pipeline inside a batch already overla
 a ``weight_sum`` / ``weight_max`` request resolves to its own float32 numpy row backed by a page-locked block of at most
 32 rows.  ``weight_sum_at`` / ``weight_max_at`` are the sparse read-out for SMC callers that need a few nodes per request:
 the ``[B, N]`` slab never leaves the GPU.  ``child_masses`` is the read-out of a character-level sampler: the masses of
-one node's children per request, computed from the leaves under that node only.
+one node's children per request, computed from the leaves under that node only; ``symbol_masses`` gives the same
+masses laid out by symbol, aligned with the per-symbol weights of a byte-level potential.
 """
 import asyncio
 import logging
@@ -86,6 +87,13 @@ class AsyncTokenCharacterTrie:
         future = await self._queue_request((ws, int(node)), ("child", bool(normalize), bool(log)))
         return await future
 
+    async def symbol_masses(self, ws, node, normalize=False, log=False, log_input=False):
+        """Masses of the children of ``node`` by symbol -> float32 ``[S+1]`` (``ParallelTokenCharacterTrie.
+        batch_symbol_masses``: column ``S`` is "the token ends here").  Concurrent requests with the same flags share
+        one batched call."""
+        future = await self._queue_request((ws, int(node)), ("symbol", bool(normalize), bool(log), bool(log_input)))
+        return await future
+
     def start(self):
         """Start the background task (binds a fresh queue to the running loop)."""
         if not self._task or self._task.done():
@@ -121,6 +129,13 @@ class AsyncTokenCharacterTrie:
         degs = (ids >= 0).sum(axis=1)  # padding columns come last
         return [(ids[b, :d], masses[b, :d]) for b, d in enumerate(degs.tolist())]
 
+    def _do_symbol(self, op, requests):
+        _, normalize, log, log_input = op
+        rows = self.trie._preprocess_ws([r[0] for r in requests])
+        nodes = np.asarray([r[1] for r in requests], dtype=np.int32)
+        sums, _ = self.trie.batch_symbol_masses(rows, nodes, normalize=normalize, log=log, log_input=log_input)
+        return list(sums)
+
     def _run_group(self, op, requests):
         """One batched call (worker thread)."""
         if op == "sum":
@@ -135,6 +150,9 @@ class AsyncTokenCharacterTrie:
         if isinstance(op, tuple) and op[0] == "child" and hasattr(self.trie, "batch_child_masses"):
             logger.debug(f"processing {len(requests)} child-mass requests")
             return self._do_child(op, requests)
+        if isinstance(op, tuple) and op[0] == "symbol" and hasattr(self.trie, "batch_symbol_masses"):
+            logger.debug(f"processing {len(requests)} symbol-mass requests")
+            return self._do_symbol(op, requests)
         raise ValueError(f"Unknown operation: {op}")
 
     async def _background_loop(self):

@@ -277,6 +277,65 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
                 raise RuntimeError("invalid multinomial distribution (sum of probabilities <= 0)")
         return child, label, logp, logZ
 
+    # ---- the same indexed by symbol, and a draw under per-row symbol weights (a byte-level potential) -------------
+    @property
+    def num_symbols(self):
+        """``S``: symbols ``0 .. S-1`` are the edge labels (bytes first, then other labels); the symbol read-outs have
+        ``S + 1`` columns, the last one (``end_symbol``) being "the token ends here"."""
+        return self._engine.num_symbols
+
+    @property
+    def end_symbol(self):
+        """Column of "the token ends here" (the node's leaf children) in the symbol read-outs: ``S``."""
+        return self._engine.num_symbols
+
+    @property
+    def symbol_labels(self):
+        """The ``S`` edge-label objects by symbol: byte ``s`` for ``s < 256``, then the other labels of the vocabulary
+        in order of first appearance."""
+        return list(self._edge_labels)
+
+    def batch_symbol_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """``batch_child_masses_tensor`` laid out by symbol: ``(sums float32[B, S+1] | None, maxes float32[B, S+1] |
+        None)`` on the input's device, on its current stream, without a sync.
+
+        Column ``s < S`` is the child of ``nodes[b]`` whose edge symbol is ``s`` (0 -- ``-inf`` with ``log`` -- when
+        there is none); column ``S`` adds up (sum) or maxes over all leaf children of the node, i.e. the items whose
+        spelling ends there.  The values of the non-end columns are bit-equal to those of ``batch_child_masses_tensor``
+        under the same flags; an invalid id or a leaf gives a padding row."""
+        return self._engine.symbol_masses(self._child_rows(ws), nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
+                                          normalize=normalize, log=log)
+
+    def batch_symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        """``batch_symbol_masses_tensor`` as numpy arrays."""
+        out = self.batch_symbol_masses_tensor(ws, nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
+                                              normalize=normalize, log=log)
+        return tuple(None if t is None else t.cpu().numpy() for t in out)
+
+    def sample_next_symbol_weighted(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False,
+                                    check_valid=False):
+        """One draw of the next symbol per row in proportion to ``mass(child) * exp(symbol_logw[b, symbol(child)])``.
+
+        ``symbol_logw`` holds log-weights by symbol, ``[S+1]`` (shared by every row) or ``[B, S+1]``; its last column
+        weighs "the token ends here".  Returns ``(child, symbol, logp, logZ, log_mass)`` device tensors: the chosen
+        child (int32; among several items ending at the node, the one drawn), its symbol (``S`` for a leaf child),
+        ``log q(child) - logZ``, ``logZ = log sum_j q_j`` (the particle's weight increment) and the node's
+        log-mass.  Counters and key as in ``sample_next_symbol``; with all log-weights 0 the child, ``logp`` and
+        ``logZ`` are those of ``sample_next_symbol``.  A row without a draw gives child and symbol ``-1`` and
+        ``logZ = -inf`` (no weighted mass), NaN (a NaN weight or log-weight) or ``+inf``.  ``check_valid``:
+        synchronise and raise ``RuntimeError`` like ``torch.multinomial`` for such rows."""
+        ws = self._child_rows(ws)
+        child, symbol, logp, logZ, logM = self._engine.symbol_sample(ws, nodes, symbol_logw, seed=seed, offset=offset,
+                                                                     log_input=log_input, dfs_order=dfs_order)
+        if check_valid and child.numel():
+            bad = child < 0
+            if bool(bad.any()):
+                z = logZ[bad]
+                if bool((torch.isnan(z) | (z == float("inf"))).any()):
+                    raise RuntimeError("probability tensor contains either `inf`, `nan` or element < 0")
+                raise RuntimeError("invalid multinomial distribution (sum of probabilities <= 0)")
+        return child, symbol, logp, logZ, logM
+
     # ---- reference API: numpy results on the host --------------------------------------------------------------
     def _pipe_streams(self, index):
         if index not in self._streams:

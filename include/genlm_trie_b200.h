@@ -23,6 +23,10 @@
  *                               children(node) of the result on the host: the next-symbol masses of a
  *                               character-level sampler, without the [B, N] slab
  *   gt_child_sample             the same, plus one categorical draw of the next symbol per row
+ *   gt_symbol_masses            the child masses laid out by symbol (column S = end of token), aligned with the
+ *                               per-symbol weight vector of a byte-level potential
+ *   gt_symbol_sample            the draw of the next symbol in proportion to mass(child) * weight(symbol), with the
+ *                               weighted normaliser (the particle's weight increment)
  *
  * Conventions
  *   - every function returns 0 on success, non-zero on failure; gt_last_error() returns a
@@ -251,6 +255,41 @@ int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_row
 int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                     unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out,
                     void* workspace, size_t workspace_bytes, gt_stream stream);
+
+/* ---- next-symbol masses indexed by symbol, and a draw under per-row symbol log-weights ---------- */
+
+/* S = max(256, 1 + the largest symbol passed to gt_build); -1 for a null trie.  Host only.  The symbol read-outs are
+ * S + 1 wide: column s < S is the child whose edge symbol is s, column S is "the token ends here" (the leaf children). */
+int64_t gt_num_symbols(const gt_trie* t);
+
+/* For each row b and the node n = nodes[b], with the per-child fp64 sums and fp32 maxes of gt_child_masses:
+ *   out_sum[b, s] / out_max[b, s]   (s < S) the sum / max over the leaves under the child of n with edge symbol s;
+ *                                   0 (-inf with GT_CHILD_LOG) when n has no such child
+ *   out_sum[b, S]                   the fp64 sum of the sums of all leaf children of n, added in child order, rounded once
+ *   out_max[b, S]                   the max over the maxes of the leaf children of n
+ * A node id < 0 or >= N, or a leaf, gives an all-padding row.  ws, in_type, ld_ws, ops, flags (GT_FLAG_LOG_INPUT |
+ * GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG) and the workspace (gt_child_workspace_bytes) are those of
+ * gt_child_masses; out_sum / out_max are device, row stride ld_out >= S + 1.  out_sum[b, sym(c_j)] is bit-equal to
+ * gt_child_masses' out_sum[b, j] under the same flags (column S too when n has one leaf child); maxes likewise. */
+int gt_symbol_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                     float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                     void* workspace, size_t workspace_bytes, gt_stream stream);
+
+/* One draw of the next symbol per row in proportion to q_j = m_j * exp(sym_logw[b, sym(c_j)]) (fp64; q_j = 0 when
+ * m_j = 0, whatever the log-weight), with m_j the child sums of gt_child_masses and sym(c) the edge symbol of child c,
+ * S for a leaf child.  Z = sum_j q_j in the order gt_child_sample adds the m_j; u as in gt_child_sample (counter
+ * offset + b, key seed); the pick is the first child whose running sum exceeds u * Z (else the last with q_j > 0).
+ *   child_out[b] = c_j, symbol_out[b] = sym(c_j), logp_out[b] = log q_j - log Z, logZ_out[b] = log Z,
+ *   logM_out[b] = log sum_j m_j (gt_child_sample's logZ; logM_out may be NULL)
+ * sym_logw: device fp32 log-weights, [rows][S + 1]; ld_w = 0 shares row 0 between all rows, else ld_w >= S + 1.
+ * With every log-weight 0, child / logp / logZ are bit-identical to gt_child_sample.  A row without a draw gives
+ * child = symbol = -1: Z = 0 (also a leaf or an invalid id) gives logp = logZ = -inf; a NaN weight under the node, or
+ * a NaN log-weight at a symbol the node has, gives logp = logZ = NaN; Z = +inf gives logZ = +inf, logp = NaN.
+ * flags: GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER. */
+int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                     const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
+                     int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
+                     void* workspace, size_t workspace_bytes, gt_stream stream);
 
 #ifdef __cplusplus
 }
