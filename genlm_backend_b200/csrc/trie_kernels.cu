@@ -54,6 +54,8 @@ struct PlanView {
     const int32_t* child_ptr; const int32_t* child_idx;  // children CSR (ascending ids = jump[] order)
     const int32_t* child_sym;  // [N - 1] beside child_idx: the child's edge symbol, S for a leaf child
     int32_t S;                 // Layout::num_symbols
+    const int32_t* node_depth;                             // [N] symbols on the path root -> node (a leaf edge adds none)
+    const int32_t* item_sym_ptr; const int32_t* item_sym;  // [V+1] CSR of every item's symbols, in item order
     int32_t debug_stop;  // profiling aid (GT_DEBUG_STOP): 0 = normal; 3 = no emit stores; 9 = emit only
     long long* trace;    // profiling aid (GT_TRACE=1): per (CTA, item) SM-clock stamps of the pipeline events, else null
 };
@@ -801,6 +803,19 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
         child_sym[e] = lab >= 0 ? lab : (int32_t)L.num_symbols;  // leaf child: -1 - item
     }
     const size_t o_child_sym = ADDV(child_sym);
+    // post-order ids: a parent's id is larger than its children's, so one descending pass sees every parent first
+    std::vector<int32_t> node_depth((size_t)L.N, 0);
+    for (int64_t n = L.N - 2; n >= 0; --n)
+        node_depth[(size_t)n] = node_depth[(size_t)L.parent[(size_t)n]] + (L.edge_label[(size_t)n] >= 0 ? 1 : 0);
+    std::vector<int32_t> item_sym_ptr((size_t)L.V + 1, 0);
+    for (int64_t i = 0; i < L.V; ++i) item_sym_ptr[(size_t)i + 1] = item_sym_ptr[(size_t)i] + node_depth[(size_t)L.leaf_node[(size_t)i]];
+    std::vector<int32_t> item_sym((size_t)item_sym_ptr[(size_t)L.V]);
+    for (int64_t i = 0; i < L.V; ++i) {  // the edge labels from the leaf's parent up to the root, stored back to front
+        int32_t at = item_sym_ptr[(size_t)i + 1];
+        for (int32_t n = L.parent[(size_t)L.leaf_node[(size_t)i]]; n >= 0 && at > item_sym_ptr[(size_t)i]; n = L.parent[(size_t)n])
+            item_sym[(size_t)--at] = L.edge_label[(size_t)n];
+    }
+    const size_t o_node_depth = ADDV(node_depth), o_item_sym_ptr = ADDV(item_sym_ptr), o_item_sym = ADDV(item_sym);
 #undef ADDV
     total += 256;
 
@@ -855,6 +870,8 @@ static DevicePlan* upload_plan(const Layout& L, const Plan& P, int device) {
     v.perm = (const int32_t*)(base + o_perm);
     v.child_ptr = (const int32_t*)(base + o_child_ptr); v.child_idx = (const int32_t*)(base + o_child_idx);
     v.child_sym = (const int32_t*)(base + o_child_sym); v.S = (int32_t)L.num_symbols;
+    v.node_depth = (const int32_t*)(base + o_node_depth);
+    v.item_sym_ptr = (const int32_t*)(base + o_item_sym_ptr); v.item_sym = (const int32_t*)(base + o_item_sym);
     { const char* e = getenv("GT_DEBUG_STOP"); v.debug_stop = e && *e ? atoi(e) : 0; }
     v.trace = nullptr;
     if (const char* e = getenv("GT_TRACE")) {
@@ -1113,6 +1130,112 @@ __global__ void __launch_bounds__(kMaskThreads) subtree_mask_kernel(PlanView P, 
         const unsigned word = __ballot_sync(0xffffffffu, r >= 0 && (unsigned)(r - s_lo[q]) < s_len[q]);
         if ((threadIdx.x & 31) == 0 && w < ld_bits) bits[(size_t)(b0 + q) * ld_bits + w] = word;
     }
+}
+
+// ---- token masks under a byte DFA (gt_dfa_token_mask / gt_dfa_advance) ------------------------------------------------
+//
+// Row b stands at node n = nodes[b] (the root without nodes) in DFA state q = states[b].  Item i is allowed iff its leaf
+// lies under n, q is live (in [0, Q)) and delta walked from q over the item's symbols depth(n) .. len(i)-1 never leaves
+// [0, Q).  dfa_mask_kernel: one thread per item, so that a warp's ballot is one mask word (as in subtree_mask_kernel), and
+// kDfaRows rows per CTA.  The loop runs over the item's symbols outside and the rows inside: symbol k is loaded once and
+// steps the state of every row of the group, which gives each thread kDfaRows independent chains of dependent table loads
+// instead of one long chain.  A row outside the subtree, or with a dead start state, starts dead; a thread stops once every
+// row of its group is dead.  The table is read through the read-only path (__ldg): a hot table stays in L1 / L2.
+// Rows per CTA.  Measured on B200 at 64 rows (DESIGN section 5.10): 8 is 9 % faster than 4 for root rows under a 256-state
+// table and 10-29 % slower for depth-1 rows, which have few items each.
+#ifndef GT_DFA_ROWS
+#define GT_DFA_ROWS 8
+#endif
+constexpr int kDfaThreads = 256, kDfaRows = GT_DFA_ROWS;
+
+struct DfaArgs {
+    const int32_t* delta; int32_t Q, ld;  // [Q][ld] next state; Q * ld < 2^31 (checked by the entry points)
+    const int32_t* states; const int32_t* nodes;  // nodes == null: every row at the root
+    int n_rows;
+};
+
+// Start of row b: its state, the DFS leaf range and the depth of its node; false for an invalid node or a dead state.
+__device__ __forceinline__ bool dfa_row(const PlanView& P, const DfaArgs& A, int b, int& q, int& lo, unsigned& len, int& d) {
+    const int n = A.nodes ? __ldg(A.nodes + b) : (int)P.N - 1;
+    q = __ldg(A.states + b);
+    if (n < 0 || n >= P.N || q < 0 || q >= A.Q) return false;
+    lo = __ldg(P.node_lo + n);
+    len = (unsigned)(__ldg(P.node_hi + n) - lo);
+    d = __ldg(P.node_depth + n);
+    return true;
+}
+
+// One transition; every value outside [0, Q) is a reject, so a malformed table never leads to a read outside it.
+__device__ __forceinline__ int dfa_step(const DfaArgs& A, int q, int s) {
+    const int nq = __ldg(A.delta + q * A.ld + s);
+    return (unsigned)nq < (unsigned)A.Q ? nq : -1;
+}
+
+__global__ void __launch_bounds__(kDfaThreads) dfa_mask_kernel(PlanView P, DfaArgs A, uint32_t* __restrict__ bits, int64_t ld_bits,
+                                                               int64_t words) {
+    __shared__ int s_q[kDfaRows], s_lo[kDfaRows], s_d[kDfaRows];
+    __shared__ unsigned s_len[kDfaRows];
+    const int b0 = blockIdx.y * kDfaRows;
+    if (threadIdx.x < kDfaRows) {
+        const int b = b0 + threadIdx.x;
+        int q = -1, lo = 0, d = 0;
+        unsigned len = 0;
+        if (b >= A.n_rows || !dfa_row(P, A, b, q, lo, len, d)) { q = -1; len = 0; }
+        s_q[threadIdx.x] = q; s_lo[threadIdx.x] = lo; s_len[threadIdx.x] = len; s_d[threadIdx.x] = d;
+    }
+    const int64_t i = (int64_t)blockIdx.x * kDfaThreads + threadIdx.x;
+    int r = -1, p0 = 0, L = 0;
+    if (i < P.V) {
+        r = __ldg(P.leaf_rank + i);
+        p0 = __ldg(P.item_sym_ptr + i);
+        L = __ldg(P.item_sym_ptr + i + 1) - p0;
+    }
+    __syncthreads();
+    int st[kDfaRows], dk[kDfaRows];
+    int k0 = INT_MAX;
+#pragma unroll
+    for (int g = 0; g < kDfaRows; ++g) {
+        const bool in = r >= 0 && s_q[g] >= 0 && (unsigned)(r - s_lo[g]) < s_len[g];
+        st[g] = in ? s_q[g] : -1;
+        dk[g] = s_d[g];
+        if (in) k0 = min(k0, dk[g]);
+    }
+    const int32_t* sy = P.item_sym + p0;
+    for (int k = k0; k < L; ++k) {
+        const int s = __ldg(sy + k);
+        bool any = false;
+#pragma unroll
+        for (int g = 0; g < kDfaRows; ++g) {
+            if (st[g] >= 0 && k >= dk[g]) st[g] = dfa_step(A, st[g], s);
+            any |= st[g] >= 0;
+        }
+        if (!any) break;
+    }
+    const int64_t w = i >> 5;
+    const int rows = min(kDfaRows, A.n_rows - b0);
+#pragma unroll
+    for (int g = 0; g < kDfaRows; ++g) {
+        if (g >= rows) break;
+        const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
+        if ((threadIdx.x & 31) == 0 && w < words) bits[(size_t)(b0 + g) * ld_bits + w] = word;
+    }
+}
+
+// One thread per row walks the drawn item's remaining symbols: the state the particle stands in after the token.
+constexpr int kDfaAdvanceThreads = 256;
+__global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanView P, DfaArgs A, const int32_t* __restrict__ tokens,
+                                                                         int32_t* __restrict__ out) {
+    const int b = blockIdx.x * kDfaAdvanceThreads + threadIdx.x;
+    if (b >= A.n_rows) return;
+    const int t = __ldg(tokens + b);
+    int q, lo, d, res = -1;
+    unsigned len;
+    if (t >= 0 && t < P.V && dfa_row(P, A, b, q, lo, len, d) && (unsigned)(__ldg(P.leaf_rank + t) - lo) < len) {
+        const int p1 = __ldg(P.item_sym_ptr + t + 1);
+        for (int p = __ldg(P.item_sym_ptr + t) + d; p < p1 && q >= 0; ++p) q = dfa_step(A, q, __ldg(P.item_sym + p));
+        res = q;
+    }
+    out[b] = res;
 }
 
 // ---- child masses of one node per row (gt_child_masses / gt_child_sample) ------------------------------------------
@@ -1889,6 +2012,66 @@ int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_ro
     A.sym_logw = sym_logw; A.ld_w = ld_w; A.symbol_out = symbol_out; A.logM_out = logM_out;
     return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream),
                             "gt_symbol_sample", gt::symbol_finish_kernel);
+}
+
+// Checks shared by the two DFA entry points (host only, before any CUDA call); fills the kernels' table / row arguments.
+static int dfa_args(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta, const int32_t* states,
+                    const int32_t* nodes, int64_t n_rows, const char* what, gt::DfaArgs& A) {
+    const int64_t S = t->layout.num_symbols;
+    if (n_states < 1 || ld_delta < S || n_rows < 0) {
+        gt::set_error("%s: bad n_states / ld_delta / n_rows (n_states=%lld >= 1, ld_delta=%lld >= S=%lld, n_rows=%lld >= 0)", what,
+                      (long long)n_states, (long long)ld_delta, (long long)S, (long long)n_rows);
+        return GT_ERR_ARG;
+    }
+    if (n_states > (int64_t)INT32_MAX / ld_delta) {  // the kernels index the table with 32-bit offsets
+        gt::set_error("%s: table of %lld x %lld entries reaches 2^31", what, (long long)n_states, (long long)ld_delta);
+        return GT_ERR_LIMIT;
+    }
+    A.delta = delta; A.Q = (int32_t)n_states; A.ld = (int32_t)ld_delta;
+    A.states = states; A.nodes = nodes; A.n_rows = (int)std::min<int64_t>(n_rows, INT32_MAX);
+    return GT_OK;
+}
+
+int gt_dfa_token_mask(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta, const int32_t* states,
+                      const int32_t* nodes, int64_t n_rows, uint32_t* mask_bits, int64_t mask_ld, gt_stream stream) {
+    if (!t) { gt::set_error("gt_dfa_token_mask: null trie"); return GT_ERR_ARG; }
+    if (!delta || !states || !mask_bits) { gt::set_error("gt_dfa_token_mask: null data pointer"); return GT_ERR_ARG; }
+    const int64_t words = (t->layout.V + 31) / 32;
+    if (mask_ld < words) { gt::set_error("gt_dfa_token_mask: mask_ld %lld < %lld words", (long long)mask_ld, (long long)words); return GT_ERR_ARG; }
+    gt::DfaArgs A{};
+    const int rc = dfa_args(t, delta, n_states, ld_delta, states, nodes, n_rows, "gt_dfa_token_mask", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0 || words == 0) return GT_OK;
+    if (n_rows > (int64_t)65535 * gt::kDfaRows) { gt::set_error("gt_dfa_token_mask: too many rows"); return GT_ERR_LIMIT; }
+    int device = -1;
+    GT_CUDA(cudaGetDevice(&device));
+    auto it = t->dev.find(device);
+    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    // the grid covers whole mask words: ceil(V/32) of them, kDfaThreads/32 per CTA
+    dim3 grid((unsigned)((words * 32 + gt::kDfaThreads - 1) / gt::kDfaThreads), (unsigned)((n_rows + gt::kDfaRows - 1) / gt::kDfaRows));
+    gt::NvtxRange nv("gt:dfa_mask");
+    gt::dfa_mask_kernel<<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, A, mask_bits, mask_ld, words);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
+}
+
+int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta, const int32_t* states,
+                   const int32_t* nodes, const int32_t* tokens, int64_t n_rows, int32_t* states_out, gt_stream stream) {
+    if (!t) { gt::set_error("gt_dfa_advance: null trie"); return GT_ERR_ARG; }
+    if (!delta || !states || !tokens || !states_out) { gt::set_error("gt_dfa_advance: null data pointer"); return GT_ERR_ARG; }
+    gt::DfaArgs A{};
+    const int rc = dfa_args(t, delta, n_states, ld_delta, states, nodes, n_rows, "gt_dfa_advance", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0) return GT_OK;
+    if (n_rows > INT32_MAX) { gt::set_error("gt_dfa_advance: too many rows"); return GT_ERR_LIMIT; }
+    int device = -1;
+    GT_CUDA(cudaGetDevice(&device));
+    auto it = t->dev.find(device);
+    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    const unsigned grid = (unsigned)((n_rows + gt::kDfaAdvanceThreads - 1) / gt::kDfaAdvanceThreads);
+    gt::dfa_advance_kernel<<<grid, gt::kDfaAdvanceThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, A, tokens, states_out);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
 }
 
 }  // extern "C"

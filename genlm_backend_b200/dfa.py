@@ -1,0 +1,62 @@
+"""Byte-level DFAs as tables over the trie's symbols, for constrained sampling.
+
+A DFA is an int32 table ``delta[Q, S]`` (``S = ParallelTokenCharacterTrie.num_symbols``: bytes 0..255, then the non-byte
+labels such as EOS): ``delta[q, s]`` is the state after symbol ``s`` from state ``q``, or -1 to reject.  One table drives
+both proposals of a constrained sampler:
+
+- token level: ``trie.dfa_token_mask(delta, states)`` -> ``smc.masked_logsumexp_sample`` -> ``trie.dfa_advance``;
+- byte level: ``symbol_logw(delta, states)`` -> ``trie.sample_next_symbol_weighted``; after a byte draw the next state is
+  ``delta[states, symbol]``, a plain gather (a drawn end of token, symbol ``S``, keeps the state).
+
+Several constraints in one call: stack their tables into one ``delta`` with disjoint state ranges (add each table's
+offset to its non-negative entries) and give each row its own start state.
+"""
+import numpy as np
+import torch
+
+
+def trim(delta, accepting):
+    """Trimmed copy of ``delta`` (host numpy, int32): every transition into a state that cannot reach an accepting
+    state becomes -1, as does every entry outside ``[0, Q)``.  State numbering is kept, so callers' state ids stay
+    valid.  ``accepting``: state ids, or a bool mask of length ``Q``."""
+    delta = np.array(delta, dtype=np.int64)
+    if delta.ndim != 2:
+        raise ValueError(f"delta must be a 2-D [states, symbols] table, got shape {delta.shape}")
+    Q = delta.shape[0]
+    acc = np.asarray(accepting)
+    good = acc.astype(bool).copy() if acc.dtype == bool else np.zeros(Q, dtype=bool)
+    if acc.dtype != bool:
+        good[acc.astype(np.int64)] = True
+    if good.shape != (Q,):
+        raise ValueError(f"accepting must name states of a {Q}-state table")
+    valid = (delta >= 0) & (delta < Q)
+    src, _ = np.nonzero(valid)
+    dst = delta[valid]
+    order = np.argsort(dst, kind="stable")
+    src, dst = src[order], dst[order]
+    first = np.searchsorted(dst, np.arange(Q + 1))  # the sources of transitions into q: src[first[q]:first[q+1]]
+    frontier = np.flatnonzero(good)
+    while frontier.size:  # reverse BFS from the accepting states
+        preds = np.concatenate([src[first[q]:first[q + 1]] for q in frontier.tolist()])
+        preds = np.unique(preds[~good[preds]])
+        good[preds] = True
+        frontier = preds
+    keep = valid & good[np.where(valid, delta, 0)]
+    return np.where(keep, delta, -1).astype(np.int32)
+
+
+def symbol_logw(delta, states, num_symbols=None):
+    """``float32[B, S+1]`` log-weights for ``sample_next_symbol_weighted``: column ``s < S`` is 0 where ``delta[q, s]``
+    is a live state and ``-inf`` elsewhere; column ``S`` ("the token ends here") is 0 iff ``q`` itself is live.  A
+    state outside ``[0, Q)`` gives an all ``-inf`` row.  ``S`` is ``num_symbols`` (default: the table's width).  The
+    result is on the device of ``delta`` when it is a tensor."""
+    delta = torch.as_tensor(delta)
+    states = torch.as_tensor(states, device=delta.device).reshape(-1).long()
+    Q = delta.shape[0]
+    S = delta.shape[1] if num_symbols is None else int(num_symbols)
+    live = (states >= 0) & (states < Q)
+    nxt = delta[states.clamp(0, Q - 1), :S]
+    ok = live[:, None] & (nxt >= 0) & (nxt < Q)
+    zero = torch.zeros((), dtype=torch.float32, device=delta.device)
+    ninf = torch.full((), float("-inf"), dtype=torch.float32, device=delta.device)
+    return torch.cat([torch.where(ok, zero, ninf), torch.where(live, zero, ninf)[:, None]], dim=1)

@@ -301,6 +301,62 @@ class TrieEngine:
                 )
         return bits
 
+    # ---- token masks under a byte DFA, and the DFA advance -------------------------------------------------------
+    def _dfa_inputs(self, delta, states, nodes, tokens=None):
+        """``(delta, states, nodes | None, tokens | None, device)`` as contiguous int32 tensors on one CUDA device: that of
+        ``states`` when it is a CUDA tensor, else that of ``delta``, else the current device."""
+        require_cuda()
+        delta, states = torch.as_tensor(delta), torch.as_tensor(states)
+        device = states.device if states.is_cuda else delta.device if delta.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        if delta.dim() != 2:
+            raise ValueError(f"delta must be a 2-D [states, symbols] table, got shape {tuple(delta.shape)}")
+        delta = delta.to(device=device, dtype=torch.int32).contiguous()
+        states = states.to(device=device, dtype=torch.int32).reshape(-1).contiguous()
+        B = states.shape[0]
+
+        def per_row(x, what):
+            x = torch.as_tensor(x).to(device=device, dtype=torch.int32).reshape(-1).contiguous()
+            if x.shape[0] != B:
+                raise ValueError(f"{what} must hold one entry per row ({B}), got {x.shape[0]}")
+            return x
+
+        nodes = None if nodes is None else per_row(nodes, "nodes")
+        tokens = None if tokens is None else per_row(tokens, "tokens")
+        self.ensure_device(device.index)
+        return delta, states, nodes, tokens, device
+
+    def dfa_token_mask(self, delta, states, nodes=None):
+        """``gt_dfa_token_mask`` on the current stream of the inputs' device: keep-bitmask ``int32[B, ceil(V/32)]`` of the
+        items allowed under the DFA ``delta`` (``[Q, ld >= S]``) from ``states[b]`` at ``nodes[b]`` (the root when None)."""
+        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
+        B, W = states.shape[0], (self.V + 31) // 32
+        bits = torch.empty((B, W), dtype=torch.int32, device=device)
+        if B and W:
+            with torch.cuda.device(device.index):
+                check(
+                    lib.gt_dfa_token_mask(self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(),
+                                          nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W,
+                                          torch.cuda.current_stream(device.index).cuda_stream),
+                    "gt_dfa_token_mask",
+                )
+        return bits
+
+    def dfa_advance(self, delta, states, tokens, nodes=None):
+        """``gt_dfa_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after the remaining
+        symbols of item ``tokens[b]``, or -1."""
+        delta, states, nodes, tokens, device = self._dfa_inputs(delta, states, nodes, tokens)
+        B = states.shape[0]
+        out = torch.empty(B, dtype=torch.int32, device=device)
+        if B:
+            with torch.cuda.device(device.index):
+                check(
+                    lib.gt_dfa_advance(self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(),
+                                       nodes.data_ptr() if nodes is not None else None, tokens.data_ptr(), B, out.data_ptr(),
+                                       torch.cuda.current_stream(device.index).cuda_stream),
+                    "gt_dfa_advance",
+                )
+        return out
+
     # ---- child masses of one node per row, straight from the rows -----------------------------------------------
     def _child_inputs(self, ws, nodes):
         """Checks shared by the child read-outs (those of ``reduce``, plus one node id per row)."""

@@ -208,6 +208,24 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         an ``int32[B, ceil(V/32)]`` device tensor in the bit-mask layout of ``smc.masked_logsumexp_sample``."""
         return self._engine.subtree_token_mask(nodes, device=device)
 
+    # ---- token masks under a byte-level DFA (a constrained token-level SMC step) ------------------------------------
+    def dfa_token_mask(self, delta, states, nodes=None):
+        """Keep-bitmask ``int32[B, ceil(V/32)]`` of the tokens each particle may emit next without leaving its
+        constraint's language, in the bit-mask layout of ``smc.masked_logsumexp_sample``.
+
+        ``delta`` is a DFA over the trie's symbols (``num_symbols``): an int32 ``[Q, ld >= S]`` table, ``delta[q, s]``
+        the next state or -1 to reject (see ``genlm_backend_b200.dfa``: ``trim`` it first).  ``states[b]`` is row
+        ``b``'s state after the symbols of the path to ``nodes[b]`` (every row at the root when ``nodes`` is None); a
+        token is allowed iff it lies under that node and the walk over its remaining symbols never rejects.  An invalid
+        node or state gives an all-zero row.  Runs on the current stream of the inputs' device; no sync."""
+        return self._engine.dfa_token_mask(delta, states, nodes)
+
+    def dfa_advance(self, delta, states, tokens, nodes=None):
+        """``int32[B]``: row ``b``'s DFA state after the remaining symbols of token ``tokens[b]`` (those past
+        ``nodes[b]``'s depth), or -1 for a token that ``dfa_token_mask`` does not allow -- also the sampler's "no draw"
+        (-1).  Keeps ``mask -> masked_logsumexp_sample -> advance`` on the device."""
+        return self._engine.dfa_advance(delta, states, tokens, nodes)
+
     # ---- child masses of one node per row (the next-symbol distribution of a character-level sampler) ------------
     @property
     def max_children(self):

@@ -27,6 +27,9 @@
  *                               per-symbol weight vector of a byte-level potential
  *   gt_symbol_sample            the draw of the next symbol in proportion to mass(child) * weight(symbol), with the
  *                               weighted normaliser (the particle's weight increment)
+ *   gt_dfa_token_mask           the host-side walk of every token's bytes through a constraint's automaton that a
+ *                               constrained token sampler does to build the mask of README.md:82-91's masked draw
+ *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
  *
  * Conventions
  *   - every function returns 0 on success, non-zero on failure; gt_last_error() returns a
@@ -290,6 +293,36 @@ int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_ro
                      const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
                      int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
                      void* workspace, size_t workspace_bytes, gt_stream stream);
+
+/* ---- token masks under a byte-level DFA, and the DFA advance over drawn tokens ------------------------------------ */
+
+/* delta: device int32 [n_states][ld_delta], ld_delta >= S (gt_num_symbols): delta[q * ld_delta + s] is the state after
+ * symbol s from state q; -1 (any value outside [0, n_states)) rejects.  A state is live iff it lies in [0, n_states).  The
+ * table is meant to be trimmed (every state a non-reject transition reaches can still reach an accepting state), so that
+ * "live" means "the prefix can still be completed"; the kernels only follow the table.  depth(n) is the number of symbols
+ * on the path root -> n (a leaf edge consumes none: a leaf's depth is its item's length).  For row b, n = nodes[b] (the
+ * root when nodes == NULL) and q = states[b], the state after the symbols of the path to n; item i is allowed iff its leaf
+ * lies under n (gt_subtree_token_mask), q is live, and delta walked from q over item i's symbols depth(n) .. len(i)-1 never
+ * leaves the live states (an item with no remaining symbols: iff q is live).  A node id < 0 or >= N, or a state outside
+ * [0, n_states), gives an all-zero row.  End of sequence needs no special case: an EOS item spells a non-byte symbol, whose
+ * column decides it (delta[q, eos] = q for accepting q, -1 otherwise).  Several constraints in one call: stack their tables
+ * with disjoint state ranges (offset each table's states) and give each row its own start state.
+ * Argument checks (GT_ERR_ARG, before any device work): null t / delta / states / outputs (tokens for the advance),
+ * n_states < 1, ld_delta < S, n_rows < 0, mask_ld < ceil(V/32); n_states * ld_delta >= 2^31 gives GT_ERR_LIMIT.  No
+ * allocation, no synchronisation, launches on `stream`, graph-capturable. */
+
+/* keep-bitmask (GT_MASK_BITS_U32 layout, item order) of the items allowed under a byte DFA, per row.  Every word of the
+ * first ceil(V/32) words of each row is written (bits >= V of the last word are 0); words beyond them are not touched. */
+int gt_dfa_token_mask(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta,
+                      const int32_t* states, const int32_t* nodes /* NULL = root */, int64_t n_rows,
+                      uint32_t* mask_bits, int64_t mask_ld, gt_stream stream);
+
+/* states_out[b] = state after item tokens[b]'s symbols depth(nodes[b]) .. end, walked from states[b]; -1 for a token < 0 or
+ * >= V (the sampler's "no draw"), a token not under nodes[b], an invalid node, a dead or invalid start state, or any reject
+ * on the way.  states_out[b] >= 0 exactly when gt_dfa_token_mask sets the token's bit for that row. */
+int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta,
+                   const int32_t* states, const int32_t* nodes /* NULL = root */, const int32_t* tokens,
+                   int64_t n_rows, int32_t* states_out, gt_stream stream);
 
 #ifdef __cplusplus
 }
