@@ -1238,7 +1238,8 @@ __global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanVie
     out[b] = res;
 }
 
-// ---- child masses of one node per row (gt_child_masses / gt_child_sample) ------------------------------------------
+// ---- next-symbol read-outs: masses of the children of one node per row, by child or by symbol, and the draw ---------
+// (gt_child_masses / gt_child_sample / gt_symbol_masses / gt_symbol_sample)
 //
 // The children of a node n tile its DFS leaf range [lo(n), hi(n)) with consecutive ranges (post-order numbering, DESIGN
 // section 2), so the job is a segmented reduction over one contiguous range of DFS ranks per row, with at most D segments.
@@ -1248,8 +1249,11 @@ __global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanVie
 //   child_block_kernel   persistent warps take blocks u = warp, warp + warps, ...; block k of row b writes the fp64 partial
 //                        sum (and the max) of each child segment j it overlaps to slot j + k of the row.  Children are
 //                        consecutive, so k_first(j + 1) >= k_last(j) and (j, k) -> j + k is injective: no atomics
-//   child_finish_kernel  one warp per row: adds each child's slots in k order and writes ids / sums / maxes (normalised,
-//                        logs), or draws the next symbol
+//   finish kernels       one warp per row, all starting from finish_row (a child's slots added in k order, the lanes'
+//                        sums scanned in a fixed order); one per job:
+//     child_masses_kernel   ids / sums / maxes by child (normalised, logs)
+//     symbol_masses_kernel  sums / maxes by symbol
+//     child_draw_kernel     the next child, optionally under per-row symbol log-weights
 // Every sum is a fixed function of (node, child): lane l of a block adds the block's ranks 4l + 128q + i (q < 4, i < 4)
 // in that order, the warp combines its lanes by a fixed butterfly, and the finish kernel adds a child's blocks in order.
 // The batch, the row's position in it, the chunking, the input order and the grid size change nothing.
@@ -1264,11 +1268,11 @@ struct ChildArgs {
     int32_t* blk_off;                   // [n_rows + 1] exclusive scan of the blocks per row
     double* part_sum; float* part_max;  // [n_rows][slots]
     int64_t slots; int need_max;
-    // finish, masses
+    // child_masses_kernel (child_ids, D) and symbol_masses_kernel
     int32_t* child_ids; float* out_sum; float* out_max; int64_t ld_out; int D; int normalize, log_out;
-    // finish, draw (child_out != null)
+    // child_draw_kernel
     int32_t* child_out; float* logp_out; float* logZ_out; uint64_t seed, ctr0;  // ctr0 = offset + first row of the chunk
-    // symbol_finish_kernel: draw under per-row symbol log-weights (row stride ld_w, 0 = shared)
+    // ... optional: per-row symbol log-weights (row stride ld_w, 0 = shared), the drawn symbol and the node's log-mass
     const float* sym_logw; int64_t ld_w; int32_t* symbol_out; float* logM_out;
 };
 
@@ -1498,168 +1502,148 @@ __device__ __forceinline__ int pick_child(const Q& q, int j_lo, int j_hi, double
     return pick;
 }
 
-// One warp per row.  Lane l owns the contiguous children [j_lo, j_hi) of the row's node; their sums are added in order
-// and an inclusive scan over the lanes gives the running sums and the node's mass (fixed order: normalisation and draw
-// see the same total).
-__global__ void __launch_bounds__(kChildThreads) child_finish_kernel(PlanView P, ChildArgs A) {
-    pdl_wait();  // the slots come from child_block_kernel
-    pdl_trigger();
-    const int lane = threadIdx.x & 31;
-    const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
-    if (b >= A.n_rows) return;
+__device__ __forceinline__ double warp_inclusive_scan(double x, int lane) {
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const double y = __shfl_up_sync(0xffffffffu, x, o);
+        if (lane >= o) x += y;
+    }
+    return x;
+}
+
+// Where every finish kernel starts (one warp per row b): the row's node (no children for an invalid id or a leaf), its
+// slots, and the children [j_lo, j_hi) lane l owns.  local adds their sums in order and an inclusive scan over the lanes
+// gives the running sums incl and the node's mass total: one fixed order, so normalisation, draw and every finish kernel
+// see the same sums.
+struct FinishRow {
+    ChildSlots cs; const int32_t* sy; int deg, j_lo, j_hi; double local, incl, total;
+};
+__device__ __forceinline__ FinishRow finish_row(const PlanView& P, const ChildArgs& A, int b, int lane) {
     int cp0 = 0, deg = 0, lo = 0, hi = 0;
     if (!child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi)) deg = 0;
-    const int32_t* ch = P.child_idx + cp0;
-    const ChildSlots cs{P, ch, A.part_sum + (size_t)b * A.slots, A.part_max + (size_t)b * A.slots, lo};
+    const ChildSlots cs{P, P.child_idx + cp0, A.part_sum + (size_t)b * A.slots, A.part_max + (size_t)b * A.slots, lo};
     const int per = (deg + 31) / 32;
     const int j_lo = min(deg, lane * per), j_hi = min(deg, j_lo + per);
     double local = 0.0;
     for (int j = j_lo; j < j_hi; ++j) local += cs.sum(j);
-    double incl = local;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const double y = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += y;
-    }
-    const double total = __shfl_sync(0xffffffffu, incl, 31);
-
-    if (!A.child_out) {
-        int32_t* ids = A.child_ids + (size_t)b * A.ld_out;
-        float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
-        float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
-        for (int j = j_lo; j < j_hi; ++j) {
-            const int c = __ldg(ch + j);
-            ids[j] = c;
-            if (os) {
-                double s = cs.sum(j);
-                if (A.normalize) s /= total;
-                os[j] = (float)(A.log_out ? log(s) : s);
-            }
-            if (om) {
-                const float m = cs.max(j);
-                om[j] = A.log_out ? (float)log((double)m) : m;
-            }
-        }
-        const float pad = A.log_out ? -INFINITY : 0.f;
-        for (int j = deg + lane; j < A.D; j += 32) {
-            ids[j] = -1;
-            if (os) os[j] = pad;
-            if (om) om[j] = pad;
-        }
-        return;
-    }
-
-    // draw: the first child whose running sum exceeds u * total
-    const bool ok = total > 0.0 && total < (double)INFINITY;  // false for NaN
-    int pick = -1;
-    double mass = 0.0;
-    if (ok)
-        pick = pick_child([&](int j) { return cs.sum(j); }, j_lo, j_hi, local, incl,
-                          philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total, lane, mass);
-    if (lane == 0) {
-        A.child_out[b] = ok ? __ldg(ch + pick) : -1;
-        A.logZ_out[b] = (float)log(total);  // -inf for no mass, NaN for a NaN weight
-        A.logp_out[b] = ok ? (float)(log(mass) - log(total)) : (total == 0.0 ? -INFINITY : NAN);
-    }
+    const double incl = warp_inclusive_scan(local, lane);
+    return {cs, P.child_sym + cp0, deg, j_lo, j_hi, local, incl, __shfl_sync(0xffffffffu, incl, 31)};
 }
 
+// A child's sum and max as the masses read-outs write them: the sum divided by the node's mass (GT_CHILD_NORMALIZE),
+// both as logs (GT_CHILD_LOG), rounded to fp32 once.
+__device__ __forceinline__ float sum_out(const ChildArgs& A, double s, double total) {
+    if (A.normalize) s /= total;
+    return (float)(A.log_out ? log(s) : s);
+}
+__device__ __forceinline__ float max_out(const ChildArgs& A, float m) { return A.log_out ? (float)log((double)m) : m; }
 
-// ---- the same, indexed by symbol (gt_symbol_masses / gt_symbol_sample) --------------------------------------------
-// Same slots, same lane split and scan as child_finish_kernel, so every per-child sum, the node's mass and the draw of
-// gt_child_sample are reproduced bit for bit; child j goes to column child_sym[j] (S for a leaf child).  Masses: the
-// row is first filled with padding, then each non-leaf child writes its own column (a node has one child per symbol),
-// and column S gets the leaf children's sums added in child order.  Draw: q_j = m_j * exp(logw[sym_j]) in fp64,
-// scanned like the m_j.
-__global__ void __launch_bounds__(kChildThreads) symbol_finish_kernel(PlanView P, ChildArgs A) {
+__global__ void __launch_bounds__(kChildThreads) child_masses_kernel(PlanView P, ChildArgs A) {
     pdl_wait();  // the slots come from child_block_kernel
     pdl_trigger();
     const int lane = threadIdx.x & 31;
     const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
     if (b >= A.n_rows) return;
-    int cp0 = 0, deg = 0, lo = 0, hi = 0;
-    if (!child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi)) deg = 0;
-    const int32_t* ch = P.child_idx + cp0;
-    const int32_t* sy = P.child_sym + cp0;
-    const int S = P.S;
-    const ChildSlots cs{P, ch, A.part_sum + (size_t)b * A.slots, A.part_max + (size_t)b * A.slots, lo};
-    const int per = (deg + 31) / 32;
-    const int j_lo = min(deg, lane * per), j_hi = min(deg, j_lo + per);
-    auto scan = [&](double local) {  // inclusive, over the lanes (the order of child_finish_kernel)
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const double y = __shfl_up_sync(0xffffffffu, local, o);
-            if (lane >= o) local += y;
-        }
-        return local;
-    };
-    double local_m = 0.0;
-    for (int j = j_lo; j < j_hi; ++j) local_m += cs.sum(j);
-    const double incl_m = scan(local_m);
-    const double total_m = __shfl_sync(0xffffffffu, incl_m, 31);
-
-    if (!A.child_out) {
-        float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
-        float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
-        const float pad = A.log_out ? -INFINITY : 0.f;
-        for (int s = lane; s <= S; s += 32) {
-            if (os) os[s] = pad;
-            if (om) om[s] = pad;
-        }
-        __syncwarp();  // the children's columns overwrite the padding
-        auto put = [&](int col, double sum, float mx) {
-            if (os) {
-                if (A.normalize) sum /= total_m;
-                os[col] = (float)(A.log_out ? log(sum) : sum);
-            }
-            if (om) om[col] = A.log_out ? (float)log((double)mx) : mx;
-        };
-        bool has_end = false;
-        for (int j = j_lo; j < j_hi; ++j) {
-            const int sym = __ldg(sy + j);
-            if (sym == S) { has_end = true; continue; }
-            put(sym, os ? cs.sum(j) : 0.0, om ? cs.max(j) : 0.f);
-        }
-        // end of token: the leaf children, lane by lane in child order (usually one lane, one child)
-        const unsigned ends = __ballot_sync(0xffffffffu, has_end);
-        double es = 0.0;
-        float em = -INFINITY;
-        for (unsigned e = ends; e; e &= e - 1) {
-            const int src = __ffs(e) - 1;
-            if (lane == src)
-                for (int j = j_lo; j < j_hi; ++j)
-                    if (__ldg(sy + j) == S) {
-                        if (os) es += cs.sum(j);
-                        if (om) em = fmaxf(em, cs.max(j));
-                    }
-            es = __shfl_sync(0xffffffffu, es, src);
-            em = __shfl_sync(0xffffffffu, em, src);
-        }
-        if (ends && lane == 0) put(S, es, em);
-        return;
+    const FinishRow r = finish_row(P, A, b, lane);
+    int32_t* ids = A.child_ids + (size_t)b * A.ld_out;
+    float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
+    float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
+    for (int j = r.j_lo; j < r.j_hi; ++j) {
+        ids[j] = __ldg(r.cs.ch + j);
+        if (os) os[j] = sum_out(A, r.cs.sum(j), r.total);
+        if (om) om[j] = max_out(A, r.cs.max(j));
     }
+    const float pad = A.log_out ? -INFINITY : 0.f;
+    for (int j = r.deg + lane; j < A.D; j += 32) {
+        ids[j] = -1;
+        if (os) os[j] = pad;
+        if (om) om[j] = pad;
+    }
+}
 
-    // draw under the row's symbol log-weights
-    const float* lw = A.sym_logw + (size_t)b * A.ld_w;
-    auto weighted = [&](int j) {  // q_j: no mass stays 0 whatever the weight; a NaN weight poisons the row
-        const float w = __ldg(lw + __ldg(sy + j));
+// Indexed by symbol: child j goes to column child_sym[j] (S for a leaf child), so every value is bit-equal to that of
+// child_masses_kernel.  The row is first filled with padding, then each non-leaf child writes its own column (a node
+// has one child per symbol), and column S gets the leaf children's sums added in child order.
+__global__ void __launch_bounds__(kChildThreads) symbol_masses_kernel(PlanView P, ChildArgs A) {
+    pdl_wait();  // the slots come from child_block_kernel
+    pdl_trigger();
+    const int lane = threadIdx.x & 31;
+    const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
+    if (b >= A.n_rows) return;
+    const FinishRow r = finish_row(P, A, b, lane);
+    const int S = P.S;
+    float* os = A.out_sum ? A.out_sum + (size_t)b * A.ld_out : nullptr;
+    float* om = A.out_max ? A.out_max + (size_t)b * A.ld_out : nullptr;
+    const float pad = A.log_out ? -INFINITY : 0.f;
+    for (int s = lane; s <= S; s += 32) {
+        if (os) os[s] = pad;
+        if (om) om[s] = pad;
+    }
+    __syncwarp();  // the children's columns overwrite the padding
+    bool has_end = false;
+    for (int j = r.j_lo; j < r.j_hi; ++j) {
+        const int sym = __ldg(r.sy + j);
+        if (sym == S) { has_end = true; continue; }
+        if (os) os[sym] = sum_out(A, r.cs.sum(j), r.total);
+        if (om) om[sym] = max_out(A, r.cs.max(j));
+    }
+    // end of token: the leaf children, lane by lane in child order (usually one lane, one child)
+    const unsigned ends = __ballot_sync(0xffffffffu, has_end);
+    double es = 0.0;
+    float em = -INFINITY;
+    for (unsigned e = ends; e; e &= e - 1) {
+        const int src = __ffs(e) - 1;
+        if (lane == src)
+            for (int j = r.j_lo; j < r.j_hi; ++j)
+                if (__ldg(r.sy + j) == S) {
+                    if (os) es += r.cs.sum(j);
+                    if (om) em = fmaxf(em, r.cs.max(j));
+                }
+        es = __shfl_sync(0xffffffffu, es, src);
+        em = __shfl_sync(0xffffffffu, em, src);
+    }
+    if (ends && lane == 0) {
+        if (os) os[S] = sum_out(A, es, r.total);
+        if (om) om[S] = max_out(A, em);
+    }
+}
+
+// The next-symbol draw: the first child whose running sum of terms q_j exceeds u * Z, Z the sum of all q_j.  Without
+// log-weights q_j is the child's mass m_j and Z the node's mass.  With them (gt_symbol_sample) q_j = m_j * exp(logw[sym_j])
+// in fp64, scanned like the m_j: no mass stays 0 whatever the weight, and a NaN weight poisons the row.  With all
+// log-weights 0 the two give the same bits.  symbol_out and logM_out are optional.
+__global__ void __launch_bounds__(kChildThreads) child_draw_kernel(PlanView P, ChildArgs A) {
+    pdl_wait();  // the slots come from child_block_kernel
+    pdl_trigger();
+    const int lane = threadIdx.x & 31;
+    const int b = (int)blockIdx.x * (kChildThreads / 32) + (int)(threadIdx.x >> 5);
+    if (b >= A.n_rows) return;
+    const FinishRow r = finish_row(P, A, b, lane);
+    const float* lw = A.sym_logw ? A.sym_logw + (size_t)b * A.ld_w : nullptr;
+    auto term = [&](int j) {
+        if (!lw) return r.cs.sum(j);
+        const float w = __ldg(lw + __ldg(r.sy + j));
         if (isnan(w)) return (double)NAN;
-        const double m = cs.sum(j);
+        const double m = r.cs.sum(j);
         return m == 0.0 ? 0.0 : m * exp((double)w);
     };
-    double local = 0.0;
-    for (int j = j_lo; j < j_hi; ++j) local += weighted(j);
-    const double incl = scan(local);
-    const double total = __shfl_sync(0xffffffffu, incl, 31);
+    double local = r.local, incl = r.incl, total = r.total;
+    if (lw) {
+        local = 0.0;
+        for (int j = r.j_lo; j < r.j_hi; ++j) local += term(j);
+        incl = warp_inclusive_scan(local, lane);
+        total = __shfl_sync(0xffffffffu, incl, 31);
+    }
     const bool ok = total > 0.0 && total < (double)INFINITY;  // false for NaN
     int pick = -1;
     double mass = 0.0;
-    if (ok) pick = pick_child(weighted, j_lo, j_hi, local, incl, philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total, lane, mass);
+    if (ok) pick = pick_child(term, r.j_lo, r.j_hi, local, incl, philox_uniform53(A.seed, A.ctr0 + (uint64_t)b) * total, lane, mass);
     if (lane == 0) {
-        A.child_out[b] = ok ? __ldg(ch + pick) : -1;
-        A.symbol_out[b] = ok ? __ldg(sy + pick) : -1;
+        A.child_out[b] = ok ? __ldg(r.cs.ch + pick) : -1;
+        if (A.symbol_out) A.symbol_out[b] = ok ? __ldg(r.sy + pick) : -1;
         A.logZ_out[b] = (float)log(total);  // -inf for no mass, NaN for a NaN weight, +inf for an infinite total
         A.logp_out[b] = ok ? (float)(log(mass) - log(total)) : (total == 0.0 ? -INFINITY : NAN);
-        if (A.logM_out) A.logM_out[b] = (float)log(total_m);
+        if (A.logM_out) A.logM_out[b] = (float)log(r.total);
     }
 }
 
@@ -1690,24 +1674,31 @@ struct ChildScratch {
     }
 };
 
+// The plan metadata resident on the current device, for the launches of one call.
+static int resident_plan(const gt_trie* t, const PlanView*& v) {
+    int device = -1;
+    GT_CUDA(cudaGetDevice(&device));
+    auto it = t->dev.find(device);
+    if (it == t->dev.end()) { set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    v = &it->second->view;
+    return GT_OK;
+}
+
 // Shared by gt_child_masses, gt_child_sample, gt_symbol_masses and gt_symbol_sample: arguments are checked by the
 // callers (before any CUDA call); this selects the device plan and launches scan -> blocks -> finish per chunk of rows,
 // chained with programmatic dependent launch on the caller's stream.  A.nodes / A.ws / outputs point at row 0; chunk c
-// advances them.  `finish` is child_finish_kernel or symbol_finish_kernel.
+// advances them.
 static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t out_ld_rows, uint64_t offset, void* workspace,
-                        size_t workspace_bytes, cudaStream_t st, const char* what,
-                        void (*finish)(PlanView, ChildArgs) = child_finish_kernel) {
+                        size_t workspace_bytes, cudaStream_t st, const char* what, void (*finish)(PlanView, ChildArgs)) {
     const int64_t slots = ChildScratch::slots(t->layout);
     const ChildScratch sc(workspace, workspace_bytes, slots);
     if (sc.rows < 1) {
         set_error("%s: workspace too small: %zu bytes given, one row needs %zu", what, workspace_bytes, ChildScratch::total(1, slots));
         return GT_ERR_STATE;
     }
-    int device = -1;
-    GT_CUDA(cudaGetDevice(&device));
-    auto it = t->dev.find(device);
-    if (it == t->dev.end()) { set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
-    const PlanView& v = it->second->view;
+    const PlanView* pv = nullptr;
+    if (const int rc = resident_plan(t, pv); rc != GT_OK) return rc;
+    const PlanView& v = *pv;
     const size_t in_size = A.in_type == GT_F64 ? 8 : A.in_type == GT_F32 ? 4 : 2;
     const int64_t max_blocks = (t->layout.V + kChildBlock - 1) / kChildBlock;
     const int resident = sm_count() * resident_ctas(reinterpret_cast<const void*>(child_block_kernel), kChildThreads, 0);
@@ -1806,11 +1797,13 @@ size_t gt_workspace_bytes(const gt_trie* t, int64_t max_rows) {
                                          std::min<int64_t>(max_rows, gt::kMaxSpanRows)) + 256;
 }
 
+static bool ops_ok(unsigned ops) { return (ops & (GT_OP_SUM | GT_OP_MAX)) && !(ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX)); }
+
 int gt_weight_reduce(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, void* out_sum,
                      void* out_max, int out_type, int64_t ld_out, unsigned ops, unsigned flags, void* workspace,
                      size_t workspace_bytes, gt_stream stream) {
     if (!t) { gt::set_error("gt_weight_reduce: null trie"); return GT_ERR_ARG; }
-    if (n_rows < 0 || !(ops & (GT_OP_SUM | GT_OP_MAX)) || (ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX))) {
+    if (n_rows < 0 || !ops_ok(ops)) {
         gt::set_error("gt_weight_reduce: bad n_rows / ops"); return GT_ERR_ARG;
     }
     if (n_rows == 0) return GT_OK;
@@ -1826,15 +1819,12 @@ int gt_weight_reduce(const gt_trie* t, const void* ws, int in_type, int64_t n_ro
                       (long long)ld_ws, (long long)t->layout.V, (long long)ld_out, (long long)t->layout.N);
         return GT_ERR_ARG;
     }
-    int device = -1;
-    GT_CUDA(cudaGetDevice(&device));
-    auto it = t->dev.find(device);
-    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
-    const gt::PlanView& v = it->second->view;
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_weight_reduce: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     gt::NvtxRange nv("gt:weight_reduce");
-#define GT_REDUCE(VT, R) gt::reduce_typed<VT, R>(v, ws, in_type, n_rows, ld_ws, out_sum, out_max, ld_out, ops, flags, \
+#define GT_REDUCE(VT, R) gt::reduce_typed<VT, R>(*v, ws, in_type, n_rows, ld_ws, out_sum, out_max, ld_out, ops, flags, \
                                                 workspace, workspace_bytes, st)
     // 16-byte value slots: four fp32 rows or two fp64 rows per work item
     if (out_type == GT_F32) return GT_REDUCE(float, 4);
@@ -1885,13 +1875,11 @@ int gt_subtree_token_mask(const gt_trie* t, const int32_t* nodes, int64_t n_rows
     if (n_rows == 0 || words == 0) return GT_OK;
     if (!nodes || !mask_bits) { gt::set_error("gt_subtree_token_mask: null data pointer"); return GT_ERR_ARG; }
     if (n_rows > (int64_t)65535 * gt::kMaskRows) { gt::set_error("gt_subtree_token_mask: too many rows"); return GT_ERR_LIMIT; }
-    int device = -1;
-    GT_CUDA(cudaGetDevice(&device));
-    auto it = t->dev.find(device);
-    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     // the grid covers whole mask words: ceil(V/32) of them, kMaskThreads/32 per CTA
     dim3 grid((unsigned)((words * 32 + gt::kMaskThreads - 1) / gt::kMaskThreads), (unsigned)((n_rows + gt::kMaskRows - 1) / gt::kMaskRows));
-    gt::subtree_mask_kernel<<<grid, gt::kMaskThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, nodes, (int)n_rows, mask_bits, mask_ld);
+    gt::subtree_mask_kernel<<<grid, gt::kMaskThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, nodes, (int)n_rows, mask_bits, mask_ld);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }
@@ -1903,115 +1891,118 @@ size_t gt_child_workspace_bytes(const gt_trie* t, int64_t max_rows) {
 
 static bool child_in_type_ok(int in_type) { return in_type == GT_F32 || in_type == GT_F64 || in_type == GT_F16 || in_type == GT_BF16; }
 
+// Checks shared by the four next-symbol read-outs.  Each call makes its checks in one order: the scalars and strides
+// (child_check_scalars, then its own), the early return for no rows, the data pointers (its own outputs, then
+// child_check_pointers) and last the workspace, so that a call without rows accepts null pointers.
+// child_check_scalars fills the input half of A.
+static int child_check_scalars(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws,
+                               const int32_t* nodes, unsigned flags, unsigned known, const char* what, gt::ChildArgs& A) {
+    if (!t) { gt::set_error("%s: null trie", what); return GT_ERR_ARG; }
+    if (n_rows < 0 || (flags & ~known) || !child_in_type_ok(in_type)) {
+        gt::set_error("%s: bad n_rows / flags / input type", what); return GT_ERR_ARG;
+    }
+    if (ld_ws < t->layout.V) {
+        gt::set_error("%s: row stride %lld smaller than V = %lld", what, (long long)ld_ws, (long long)t->layout.V); return GT_ERR_ARG;
+    }
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws; A.nodes = nodes;
+    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
+    A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
+    return GT_OK;
+}
+
+static int child_check_pointers(const gt_trie* t, const void* ws, const int32_t* nodes, const void* workspace, const char* what) {
+    if ((t->layout.V > 0 && !ws) || !nodes) { gt::set_error("%s: null data pointer", what); return GT_ERR_ARG; }
+    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) {
+        gt::set_error("%s: workspace must be a 256-byte aligned device pointer", what); return GT_ERR_ARG;
+    }
+    return GT_OK;
+}
+
+static const unsigned kMassesFlags = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
+static const unsigned kSampleFlags = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER;
+
 int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                     int32_t* child_ids, float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
                     void* workspace, size_t workspace_bytes, gt_stream stream) {
-    if (!t) { gt::set_error("gt_child_masses: null trie"); return GT_ERR_ARG; }
-    const unsigned known = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
-    if (n_rows < 0 || !(ops & (GT_OP_SUM | GT_OP_MAX)) || (ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX)) || (flags & ~known) ||
-        !child_in_type_ok(in_type)) {
-        gt::set_error("gt_child_masses: bad n_rows / ops / flags / input type"); return GT_ERR_ARG;
-    }
+    gt::ChildArgs A{};
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kMassesFlags, __func__, A);
+    if (rc != GT_OK) return rc;
     const int64_t D = t->layout.max_children;
-    if (ld_ws < t->layout.V || ld_out < D) {
-        gt::set_error("gt_child_masses: row stride smaller than row length (ld_ws=%lld V=%lld ld_out=%lld D=%lld)",
-                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_out, (long long)D);
+    if (!ops_ok(ops) || ld_out < D) {
+        gt::set_error("%s: bad ops, or output row stride %lld smaller than D = %lld", __func__, (long long)ld_out, (long long)D);
         return GT_ERR_ARG;
     }
     if (n_rows == 0 || D == 0) return GT_OK;
-    if ((t->layout.V > 0 && !ws) || !nodes || !child_ids || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
-        gt::set_error("gt_child_masses: null data pointer"); return GT_ERR_ARG;
+    if (!child_ids || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
+        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
     }
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_child_masses: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
-    gt::ChildArgs A{};
-    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
-    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
-    A.nodes = nodes; A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
+    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
+    A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
     A.child_ids = child_ids; A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr;
     A.ld_out = ld_out; A.D = (int)D;
-    A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
-    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), "gt_child_masses");
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+                            gt::child_masses_kernel);
 }
 
 int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                     unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out,
                     void* workspace, size_t workspace_bytes, gt_stream stream) {
-    if (!t) { gt::set_error("gt_child_sample: null trie"); return GT_ERR_ARG; }
-    if (n_rows < 0 || (flags & ~(unsigned)(GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER)) || !child_in_type_ok(in_type)) {
-        gt::set_error("gt_child_sample: bad n_rows / flags / input type"); return GT_ERR_ARG;
-    }
-    if (ld_ws < t->layout.V) { gt::set_error("gt_child_sample: row stride %lld smaller than V = %lld", (long long)ld_ws, (long long)t->layout.V); return GT_ERR_ARG; }
-    if (n_rows == 0) return GT_OK;
-    if ((t->layout.V > 0 && !ws) || !nodes || !child_out || !logp_out || !logZ_out) {
-        gt::set_error("gt_child_sample: null data pointer"); return GT_ERR_ARG;
-    }
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_child_sample: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
     gt::ChildArgs A{};
-    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
-    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
-    A.nodes = nodes; A.need_max = 0;
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kSampleFlags, __func__, A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0) return GT_OK;
+    if (!child_out || !logp_out || !logZ_out) { gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG; }
+    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
     A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
-    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), "gt_child_sample");
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+                            gt::child_draw_kernel);
 }
 
 int gt_symbol_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                      float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
                      void* workspace, size_t workspace_bytes, gt_stream stream) {
-    if (!t) { gt::set_error("gt_symbol_masses: null trie"); return GT_ERR_ARG; }
-    const unsigned known = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
-    if (n_rows < 0 || !(ops & (GT_OP_SUM | GT_OP_MAX)) || (ops & ~(unsigned)(GT_OP_SUM | GT_OP_MAX)) || (flags & ~known) ||
-        !child_in_type_ok(in_type)) {
-        gt::set_error("gt_symbol_masses: bad n_rows / ops / flags / input type"); return GT_ERR_ARG;
-    }
+    gt::ChildArgs A{};
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kMassesFlags, __func__, A);
+    if (rc != GT_OK) return rc;
     const int64_t S = t->layout.num_symbols;
-    if (ld_ws < t->layout.V || ld_out < S + 1) {
-        gt::set_error("gt_symbol_masses: row stride smaller than row length (ld_ws=%lld V=%lld ld_out=%lld S+1=%lld)",
-                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_out, (long long)(S + 1));
+    if (!ops_ok(ops) || ld_out < S + 1) {
+        gt::set_error("%s: bad ops, or output row stride %lld smaller than S + 1 = %lld", __func__, (long long)ld_out,
+                      (long long)(S + 1));
         return GT_ERR_ARG;
     }
     if (n_rows == 0) return GT_OK;
-    if ((t->layout.V > 0 && !ws) || !nodes || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
-        gt::set_error("gt_symbol_masses: null data pointer"); return GT_ERR_ARG;
+    if (((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
+        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
     }
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_symbol_masses: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
-    gt::ChildArgs A{};
-    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
-    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
-    A.nodes = nodes; A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
-    A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr;
-    A.ld_out = ld_out; A.D = (int)t->layout.max_children;
-    A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
-    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream),
-                            "gt_symbol_masses", gt::symbol_finish_kernel);
+    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
+    A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
+    A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr; A.ld_out = ld_out;
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+                            gt::symbol_masses_kernel);
 }
 
 int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                      const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
                      int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
                      void* workspace, size_t workspace_bytes, gt_stream stream) {
-    if (!t) { gt::set_error("gt_symbol_sample: null trie"); return GT_ERR_ARG; }
-    if (n_rows < 0 || (flags & ~(unsigned)(GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER)) || !child_in_type_ok(in_type)) {
-        gt::set_error("gt_symbol_sample: bad n_rows / flags / input type"); return GT_ERR_ARG;
-    }
+    gt::ChildArgs A{};
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kSampleFlags, __func__, A);
+    if (rc != GT_OK) return rc;
     const int64_t S = t->layout.num_symbols;
-    if (ld_ws < t->layout.V || ld_w < 0 || (ld_w > 0 && ld_w < S + 1)) {
-        gt::set_error("gt_symbol_sample: row stride smaller than row length (ld_ws=%lld V=%lld ld_w=%lld S+1=%lld)",
-                      (long long)ld_ws, (long long)t->layout.V, (long long)ld_w, (long long)(S + 1));
+    if (ld_w < 0 || (ld_w > 0 && ld_w < S + 1)) {
+        gt::set_error("%s: log-weight row stride %lld is neither 0 (shared) nor >= S + 1 = %lld", __func__, (long long)ld_w,
+                      (long long)(S + 1));
         return GT_ERR_ARG;
     }
     if (n_rows == 0) return GT_OK;
-    if ((t->layout.V > 0 && !ws) || !nodes || !sym_logw || !child_out || !symbol_out || !logp_out || !logZ_out) {
-        gt::set_error("gt_symbol_sample: null data pointer"); return GT_ERR_ARG;
+    if (!sym_logw || !child_out || !symbol_out || !logp_out || !logZ_out) {
+        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
     }
-    if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) { gt::set_error("gt_symbol_sample: workspace must be a 256-byte aligned device pointer"); return GT_ERR_ARG; }
-    gt::ChildArgs A{};
-    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws;
-    A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
-    A.nodes = nodes; A.need_max = 0;
+    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
     A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
     A.sym_logw = sym_logw; A.ld_w = ld_w; A.symbol_out = symbol_out; A.logM_out = logM_out;
-    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream),
-                            "gt_symbol_sample", gt::symbol_finish_kernel);
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+                            gt::child_draw_kernel);
 }
 
 // Checks shared by the two DFA entry points (host only, before any CUDA call); fills the kernels' table / row arguments.
@@ -2043,14 +2034,12 @@ int gt_dfa_token_mask(const gt_trie* t, const int32_t* delta, int64_t n_states, 
     if (rc != GT_OK) return rc;
     if (n_rows == 0 || words == 0) return GT_OK;
     if (n_rows > (int64_t)65535 * gt::kDfaRows) { gt::set_error("gt_dfa_token_mask: too many rows"); return GT_ERR_LIMIT; }
-    int device = -1;
-    GT_CUDA(cudaGetDevice(&device));
-    auto it = t->dev.find(device);
-    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     // the grid covers whole mask words: ceil(V/32) of them, kDfaThreads/32 per CTA
     dim3 grid((unsigned)((words * 32 + gt::kDfaThreads - 1) / gt::kDfaThreads), (unsigned)((n_rows + gt::kDfaRows - 1) / gt::kDfaRows));
     gt::NvtxRange nv("gt:dfa_mask");
-    gt::dfa_mask_kernel<<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, A, mask_bits, mask_ld, words);
+    gt::dfa_mask_kernel<<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, mask_bits, mask_ld, words);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }
@@ -2064,12 +2053,10 @@ int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int
     if (rc != GT_OK) return rc;
     if (n_rows == 0) return GT_OK;
     if (n_rows > INT32_MAX) { gt::set_error("gt_dfa_advance: too many rows"); return GT_ERR_LIMIT; }
-    int device = -1;
-    GT_CUDA(cudaGetDevice(&device));
-    auto it = t->dev.find(device);
-    if (it == t->dev.end()) { gt::set_error("trie metadata is not resident on device %d (call gt_upload)", device); return GT_ERR_STATE; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     const unsigned grid = (unsigned)((n_rows + gt::kDfaAdvanceThreads - 1) / gt::kDfaAdvanceThreads);
-    gt::dfa_advance_kernel<<<grid, gt::kDfaAdvanceThreads, 0, static_cast<cudaStream_t>(stream)>>>(it->second->view, A, tokens, states_out);
+    gt::dfa_advance_kernel<<<grid, gt::kDfaAdvanceThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, tokens, states_out);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }

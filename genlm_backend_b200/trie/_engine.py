@@ -29,6 +29,18 @@ _WORKSPACE_ROWS = int(os.environ.get("GT_WORKSPACE_ROWS", "1024"))
 _MAX_WORKSPACES = 16  # per engine: (device, stream) pairs we keep scratch for
 
 
+def _opmask(ops):
+    mask = 0
+    for op in ops:
+        mask |= OPS[op]
+    return mask
+
+
+def _flags(log_input=False, dfs_order=False, normalize=False, log=False):
+    return ((_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
+            | (_lib.GT_CHILD_NORMALIZE if normalize else 0) | (_lib.GT_CHILD_LOG if log else 0))
+
+
 def require_cuda():
     if not torch.cuda.is_available():
         raise RuntimeError(
@@ -119,6 +131,16 @@ class TrieEngine:
         need = int(lib.gt_child_workspace_bytes(self._handle, min(max(rows, 1), _WORKSPACE_ROWS)))
         return self._scratch(self._child_workspaces, need, index, stream)
 
+    def _launch(self, fn, index, *args, workspace=None, rows=0):
+        """``lib.<fn>(*args, [scratch, scratch bytes,] stream)`` on the current stream of device ``index``, checked.
+        ``workspace`` (``_workspace`` or ``_child_workspace``) gives the call its scratch for ``rows`` rows."""
+        with torch.cuda.device(index):
+            stream = torch.cuda.current_stream(index).cuda_stream
+            if workspace is not None:
+                work = workspace(index, stream, rows)
+                args += (work.data_ptr(), work.numel())
+            check(getattr(lib, fn)(*args, stream), fn)
+
     @staticmethod
     def _scratch(cache, need, index, stream):
         key = (index, int(stream or 0))
@@ -157,16 +179,12 @@ class TrieEngine:
             raise AssertionError([ws.shape[1], self.V])
         if ws.dtype not in _IN_TYPES:
             ws = ws.to(torch.float32)
-        if ws.shape[0] > 1 and ws.shape[1] > 1 and ws.stride(1) != 1:
-            ws = ws.contiguous()
-        elif ws.shape[1] > 1 and ws.stride(1) != 1:
+        if ws.shape[1] > 1 and ws.stride(1) != 1:
             ws = ws.contiguous()
         B = ws.shape[0]
         index = ws.device.index
         self.ensure_device(index)
-        opmask = 0
-        for op in ops:
-            opmask |= OPS[op]
+        opmask = _opmask(ops)
 
         def _out(t):
             if t is None:
@@ -183,20 +201,12 @@ class TrieEngine:
         if out_sum is not None and out_max is not None and B > 1 and out_sum.stride(0) != out_max.stride(0):
             raise ValueError("out_sum and out_max must share a row stride")
         ld_ws = ws.stride(0) if B > 1 else max(self.V, 1)
-        with torch.cuda.device(index):
-            stream = torch.cuda.current_stream(index).cuda_stream
-            work = self._workspace(index, stream, B)
-            check(
-                lib.gt_weight_reduce(
-                    self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws,
-                    out_sum.data_ptr() if out_sum is not None else None,
-                    out_max.data_ptr() if out_max is not None else None,
-                    _OUT_TYPES[out_dtype], ld_out, opmask,
-                    (_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0) | int(phases),
-                    work.data_ptr(), work.numel(), stream,
-                ),
-                "gt_weight_reduce",
-            )
+        self._launch(
+            "gt_weight_reduce", index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws,
+            out_sum.data_ptr() if out_sum is not None else None, out_max.data_ptr() if out_max is not None else None,
+            _OUT_TYPES[out_dtype], ld_out, opmask, _flags(log_input, dfs_order) | int(phases),
+            workspace=self._workspace, rows=B,
+        )
         return out_sum, out_max
 
     def reduce_raw(self, ws, opmask, log_input, index, stream_ptr):
@@ -269,15 +279,11 @@ class TrieEngine:
                 raise ValueError("normalizer must be a node id or one node id per row")
         out = torch.empty((B, K), dtype=mass.dtype, device=dev)
         if B and K:
-            with torch.cuda.device(dev.index):
-                check(
-                    lib.gt_gather_nodes(
-                        mass.data_ptr(), _OUT_TYPES[mass.dtype], B, self.N, mass.stride(0) if B > 1 else self.N,
-                        ids.data_ptr(), K, ids_ld, norm.data_ptr() if norm is not None else None,
-                        _lib.GT_GATHER_LOG if log else 0, out.data_ptr(), K, torch.cuda.current_stream(dev.index).cuda_stream,
-                    ),
-                    "gt_gather_nodes",
-                )
+            self._launch(
+                "gt_gather_nodes", dev.index, mass.data_ptr(), _OUT_TYPES[mass.dtype], B, self.N,
+                mass.stride(0) if B > 1 else self.N, ids.data_ptr(), K, ids_ld, norm.data_ptr() if norm is not None else None,
+                _lib.GT_GATHER_LOG if log else 0, out.data_ptr(), K,
+            )
         return out
 
     def subtree_token_mask(self, nodes, device=None):
@@ -293,12 +299,7 @@ class TrieEngine:
         self.ensure_device(device.index)
         bits = torch.empty((B, W), dtype=torch.int32, device=device)
         if B and W:
-            with torch.cuda.device(device.index):
-                check(
-                    lib.gt_subtree_token_mask(self._handle, nodes.data_ptr(), B, bits.data_ptr(), W,
-                                              torch.cuda.current_stream(device.index).cuda_stream),
-                    "gt_subtree_token_mask",
-                )
+            self._launch("gt_subtree_token_mask", device.index, self._handle, nodes.data_ptr(), B, bits.data_ptr(), W)
         return bits
 
     # ---- token masks under a byte DFA, and the DFA advance -------------------------------------------------------
@@ -332,13 +333,8 @@ class TrieEngine:
         B, W = states.shape[0], (self.V + 31) // 32
         bits = torch.empty((B, W), dtype=torch.int32, device=device)
         if B and W:
-            with torch.cuda.device(device.index):
-                check(
-                    lib.gt_dfa_token_mask(self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(),
-                                          nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W,
-                                          torch.cuda.current_stream(device.index).cuda_stream),
-                    "gt_dfa_token_mask",
-                )
+            self._launch("gt_dfa_token_mask", device.index, self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1],
+                         states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W)
         return bits
 
     def dfa_advance(self, delta, states, tokens, nodes=None):
@@ -348,13 +344,9 @@ class TrieEngine:
         B = states.shape[0]
         out = torch.empty(B, dtype=torch.int32, device=device)
         if B:
-            with torch.cuda.device(device.index):
-                check(
-                    lib.gt_dfa_advance(self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(),
-                                       nodes.data_ptr() if nodes is not None else None, tokens.data_ptr(), B, out.data_ptr(),
-                                       torch.cuda.current_stream(device.index).cuda_stream),
-                    "gt_dfa_advance",
-                )
+            self._launch("gt_dfa_advance", device.index, self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1],
+                         states.data_ptr(), nodes.data_ptr() if nodes is not None else None, tokens.data_ptr(), B,
+                         out.data_ptr())
         return out
 
     # ---- child masses of one node per row, straight from the rows -----------------------------------------------
@@ -381,27 +373,18 @@ class TrieEngine:
         """``gt_child_masses`` on the current stream of the input's device.  Returns ``(child_ids int32[B, D],
         sums float32[B, D] | None, maxes float32[B, D] | None)``; nothing is synchronised."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
-        opmask = 0
-        for op in ops:
-            opmask |= OPS[op]
+        opmask = _opmask(ops)
         D, dev = self.max_children, ws.device
         ids = torch.empty((B, D), dtype=torch.int32, device=dev)
         sums = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
         maxes = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
-        flags = ((_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
-                 | (_lib.GT_CHILD_NORMALIZE if normalize else 0) | (_lib.GT_CHILD_LOG if log else 0))
         if B and D:
-            with torch.cuda.device(dev.index):
-                stream = torch.cuda.current_stream(dev.index).cuda_stream
-                work = self._child_workspace(dev.index, stream, B)
-                check(
-                    lib.gt_child_masses(
-                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), ids.data_ptr(),
-                        sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None,
-                        D, opmask, flags, work.data_ptr(), work.numel(), stream,
-                    ),
-                    "gt_child_masses",
-                )
+            self._launch(
+                "gt_child_masses", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                ids.data_ptr(), sums.data_ptr() if sums is not None else None,
+                maxes.data_ptr() if maxes is not None else None, D, opmask, _flags(log_input, dfs_order, normalize, log),
+                workspace=self._child_workspace, rows=B,
+            )
         return ids, sums, maxes
 
     def child_sample(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False):
@@ -412,19 +395,12 @@ class TrieEngine:
         child = torch.empty(B, dtype=torch.int32, device=dev)
         logp = torch.empty(B, dtype=torch.float32, device=dev)
         logZ = torch.empty(B, dtype=torch.float32, device=dev)
-        flags = (_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
         if B:
-            with torch.cuda.device(dev.index):
-                stream = torch.cuda.current_stream(dev.index).cuda_stream
-                work = self._child_workspace(dev.index, stream, B)
-                check(
-                    lib.gt_child_sample(
-                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), flags,
-                        int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(), logp.data_ptr(),
-                        logZ.data_ptr(), work.data_ptr(), work.numel(), stream,
-                    ),
-                    "gt_child_sample",
-                )
+            self._launch(
+                "gt_child_sample", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                _flags(log_input, dfs_order), int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(),
+                logp.data_ptr(), logZ.data_ptr(), workspace=self._child_workspace, rows=B,
+            )
         return child, logp, logZ
 
     # ---- the same, indexed by symbol ---------------------------------------------------------------------------
@@ -432,26 +408,16 @@ class TrieEngine:
         """``gt_symbol_masses`` on the current stream of the input's device.  Returns ``(sums float32[B, S+1] | None,
         maxes float32[B, S+1] | None)``; nothing is synchronised."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
-        opmask = 0
-        for op in ops:
-            opmask |= OPS[op]
+        opmask = _opmask(ops)
         W, dev = self.num_symbols + 1, ws.device
         sums = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
         maxes = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
-        flags = ((_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
-                 | (_lib.GT_CHILD_NORMALIZE if normalize else 0) | (_lib.GT_CHILD_LOG if log else 0))
         if B:
-            with torch.cuda.device(dev.index):
-                stream = torch.cuda.current_stream(dev.index).cuda_stream
-                work = self._child_workspace(dev.index, stream, B)
-                check(
-                    lib.gt_symbol_masses(
-                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
-                        sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None,
-                        W, opmask, flags, work.data_ptr(), work.numel(), stream,
-                    ),
-                    "gt_symbol_masses",
-                )
+            self._launch(
+                "gt_symbol_masses", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None, W, opmask,
+                _flags(log_input, dfs_order, normalize, log), workspace=self._child_workspace, rows=B,
+            )
         return sums, maxes
 
     def symbol_sample(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False):
@@ -472,18 +438,11 @@ class TrieEngine:
         logp = torch.empty(B, dtype=torch.float32, device=dev)
         logZ = torch.empty(B, dtype=torch.float32, device=dev)
         logM = torch.empty(B, dtype=torch.float32, device=dev)
-        flags = (_lib.GT_FLAG_LOG_INPUT if log_input else 0) | (_lib.GT_FLAG_DFS_ORDER if dfs_order else 0)
         if B:
-            with torch.cuda.device(dev.index):
-                stream = torch.cuda.current_stream(dev.index).cuda_stream
-                work = self._child_workspace(dev.index, stream, B)
-                check(
-                    lib.gt_symbol_sample(
-                        self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), logw.data_ptr(),
-                        ld_w, flags, int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(),
-                        symbol.data_ptr(), logp.data_ptr(), logZ.data_ptr(), logM.data_ptr(), work.data_ptr(),
-                        work.numel(), stream,
-                    ),
-                    "gt_symbol_sample",
-                )
+            self._launch(
+                "gt_symbol_sample", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                logw.data_ptr(), ld_w, _flags(log_input, dfs_order), int(seed) & (2**64 - 1), int(offset) & (2**64 - 1),
+                child.data_ptr(), symbol.data_ptr(), logp.data_ptr(), logZ.data_ptr(), logM.data_ptr(),
+                workspace=self._child_workspace, rows=B,
+            )
         return child, symbol, logp, logZ, logM

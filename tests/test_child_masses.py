@@ -13,26 +13,13 @@ import numpy as np
 import pytest
 import torch
 
-import oracle
-from genlm_backend_b200 import AsyncTokenCharacterTrie, ParallelTokenCharacterTrie, Token, TokenCharacterTrie, _lib
+from genlm_backend_b200 import AsyncTokenCharacterTrie, ParallelTokenCharacterTrie, TokenCharacterTrie, _lib
 from genlm_backend_b200.synthetic import dirichlet_rows, synth_vocab
 import child_oracle
-from helpers import EOS, load_golden, tokens, unflat
+from helpers import assert_within_ulp, depth1_node, golden_layout, golden_vocab, trie_layout
 
 F32, SUM, MAX = _lib.GT_F32, _lib.GT_OP_SUM, _lib.GT_OP_MAX
 INT32_MIN = np.iinfo(np.int32).min
-
-
-def golden_vocab(name):
-    if name == "sentinel":
-        return [Token(0, b"ab"), Token(1, b""), Token(2, b"ab"), Token(3, b"a"), EOS(), b"plain"]
-    g = load_golden(name)
-    return tokens(unflat(g["blob"], g["lens"]))
-
-
-def golden_layout(name):
-    g = load_golden(name)
-    return oracle.OracleLayout(g["idx_to_leaf"], g["jump_ptr"], g["jump_idx"]), g
 
 
 # ---- CPU ---------------------------------------------------------------------------------------------------------
@@ -56,7 +43,7 @@ def test_oracle_child_masses_pinned_to_golden(name):
 
 @pytest.mark.parametrize("name", ["toy", "synth128256"])
 def test_max_children_host_only(name):
-    trie = TokenCharacterTrie(golden_vocab("toy") if name == "toy" else synth_vocab(128256))
+    trie = TokenCharacterTrie(golden_vocab(name))
     want = max(len(j) for j in trie.jump)
     assert trie._engine.max_children == want == _lib.lib.gt_max_children(trie._engine._handle)
     assert want == (3 if name == "toy" else 256)
@@ -88,6 +75,12 @@ def test_child_entry_points_reject_bad_arguments_without_a_gpu():
     assert masses(ops=SUM, m=None, flags=_lib.GT_CHILD_NORMALIZE | _lib.GT_CHILD_LOG, work_bytes=16) == 3  # too small
     assert b"workspace too small" in lib.gt_last_error()
     assert masses(n=0) == 0
+    # the order of the checks: scalars and strides, the early return for no rows, data pointers, the workspace
+    nulls = dict(ws=None, nodes=None, ids=None, s=None, m=None, work=None)
+    assert masses(n=0, **nulls) == 0
+    for bad in (dict(ops=0), dict(flags=0x40), dict(in_type=7), dict(ld_ws=V - 1), dict(ld_out=D - 1)):
+        assert masses(n=0, **nulls, **bad) == 1, bad
+    assert masses(ids=None, work=None) == 1 and b"null data pointer" in lib.gt_last_error()
 
     def sample(**kw):
         a = dict(t=h, ws=p, in_type=F32, n=4, ld_ws=V, nodes=p, flags=0, c=p, lp=p, lz=p, work=p, work_bytes=ws_bytes)
@@ -100,21 +93,14 @@ def test_child_entry_points_reject_bad_arguments_without_a_gpu():
         assert sample(**bad) == 1, bad
     assert sample(work_bytes=16) == 3
     assert sample(n=0) == 0
+    nulls = dict(ws=None, nodes=None, c=None, lp=None, lz=None, work=None)
+    assert sample(n=0, **nulls) == 0
+    for bad in (dict(flags=_lib.GT_CHILD_NORMALIZE), dict(in_type=-1), dict(ld_ws=V - 1)):
+        assert sample(n=0, **nulls, **bad) == 1, bad
+    assert sample(lz=None, work=None) == 1 and b"null data pointer" in lib.gt_last_error()
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------------
-def assert_within_ulp(have, want):
-    """fp32 results within one fp32 ulp of fp64 values; exact zeros and infinities kept."""
-    have = np.asarray(have, dtype=np.float64)
-    want = np.asarray(want, dtype=np.float64)
-    fin = np.isfinite(want)
-    assert np.array_equal(have[~fin], want[~fin], equal_nan=True)
-    assert (have[want == 0] == 0).all()
-    ulp = np.spacing(np.abs(want[fin]).astype(np.float32)).astype(np.float64)
-    err = np.abs(have[fin] - want[fin])
-    assert (err <= ulp).all(), float((err / np.maximum(ulp, 1e-300)).max())
-
-
 def slab_max_at(trie, ws, ids, **kw):
     mx = trie._engine.reduce(ws, ("max",), **kw)[1].cpu().numpy()
     return np.where(ids >= 0, np.take_along_axis(mx, np.maximum(ids, 0), axis=1), 0.0).astype(np.float32)
@@ -134,7 +120,7 @@ def check_all(trie, lay, ws_t, nodes, ws32=None):
 def test_every_node_matches_oracle(name):
     dec = golden_vocab(name)
     trie = ParallelTokenCharacterTrie(dec)
-    lay = oracle.OracleLayout(trie.idx_to_leaf, trie._layout["child_ptr"], trie._layout["child_idx"])
+    lay = trie_layout(trie)
     N, V = len(trie), len(dec)
     nodes = np.concatenate([np.arange(N), [-1, N]]).astype(np.int32)
     base = np.concatenate([dirichlet_rows(3, V, alpha=0.1, seed=11), dirichlet_rows(2, V, alpha=1.0, seed=12)])
@@ -146,7 +132,7 @@ def test_every_node_matches_oracle(name):
 def test_full_vocabulary_sampled_nodes_and_input_orders():
     V = 128256
     trie = ParallelTokenCharacterTrie(synth_vocab(V))
-    lay = oracle.OracleLayout(trie.idx_to_leaf, trie._layout["child_ptr"], trie._layout["child_idx"])
+    lay = trie_layout(trie)
     rng = np.random.default_rng(5)
     nodes = np.concatenate([[trie.root, -1, len(trie)], rng.integers(0, len(trie), 509)]).astype(np.int32)
     base = dirichlet_rows(4, V, alpha=0.1, seed=3)
@@ -165,7 +151,7 @@ def test_full_vocabulary_sampled_nodes_and_input_orders():
 def test_input_types_and_flags(dtype, log_input):
     dec = golden_vocab("synth3000")
     trie = ParallelTokenCharacterTrie(dec)
-    lay = oracle.OracleLayout(trie.idx_to_leaf, trie._layout["child_ptr"], trie._layout["child_idx"])
+    lay = trie_layout(trie)
     B = 96
     nodes = np.random.default_rng(1).integers(0, len(trie), B).astype(np.int32)
     nodes[:4] = trie.root
@@ -254,12 +240,6 @@ def test_bit_identical_across_batches_calls_workspaces_and_graphs():
         assert torch.equal(a, b)
 
 
-def _depth1(trie):
-    kids = trie.jump[trie.root]
-    internal = [int(c) for c in kids if len(trie.jump[c])]
-    return max(internal, key=lambda c: len(trie.jump[c]))
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("where", ["root", "depth1"])
 def test_draw_distribution_chi_square(where):
@@ -267,7 +247,7 @@ def test_draw_distribution_chi_square(where):
 
     dec = golden_vocab("synth3000")
     trie = ParallelTokenCharacterTrie(dec)
-    node = trie.root if where == "root" else _depth1(trie)
+    node = trie.root if where == "root" else depth1_node(trie)
     row = torch.tensor(dirichlet_rows(1, len(dec), alpha=1.0, seed=21))
     n = 20000
     ws = row.expand(n, -1).cuda()

@@ -14,31 +14,17 @@ import torch
 
 import oracle
 from genlm_backend_b200 import ParallelTokenCharacterTrie, _lib, dfa, smc
-from genlm_backend_b200.synthetic import dirichlet_rows, logsoftmax_rows, synth_vocab
+from genlm_backend_b200.synthetic import dirichlet_rows, logsoftmax_rows
 import dfa_oracle
-from helpers import EOS, load_golden, tokens, unflat
-
-
-def golden_vocab(name):
-    if name == "sentinel":
-        from genlm_backend_b200 import Token
-
-        return [Token(0, b"ab"), Token(1, b""), Token(2, b"ab"), Token(3, b"a"), EOS(), b"plain"]
-    if name == "synth128256":
-        return synth_vocab(128256)
-    g = load_golden(name)
-    return tokens(unflat(g["blob"], g["lens"]))
+from helpers import golden_layout, golden_vocab, trie_layout
 
 
 def golden_oracle(name):
-    g = load_golden(name)
-    lay = oracle.OracleLayout(g["idx_to_leaf"], g["jump_ptr"], g["jump_idx"])
-    return dfa_oracle.DfaOracle(lay, golden_vocab(name))
+    return dfa_oracle.DfaOracle(golden_layout(name)[0], golden_vocab(name))
 
 
 def trie_oracle(trie):
-    lay = oracle.OracleLayout(trie.idx_to_leaf, trie._layout["child_ptr"], trie._layout["child_idx"])
-    return dfa_oracle.DfaOracle(lay, trie.decode)
+    return dfa_oracle.DfaOracle(trie_layout(trie), trie.decode)
 
 
 def a_then_b(S):

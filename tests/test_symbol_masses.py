@@ -14,33 +14,14 @@ import numpy as np
 import pytest
 import torch
 
-import oracle
 from genlm_backend_b200 import AsyncTokenCharacterTrie, ParallelTokenCharacterTrie, _lib
 from genlm_backend_b200.synthetic import dirichlet_rows, synth_vocab
 import child_oracle
 import symbol_oracle
-from helpers import EOS, load_golden, tokens, unflat
+from helpers import EOS, assert_within_ulp, depth1_node, golden_layout, golden_vocab, trie_layout
 
 F32, SUM, MAX = _lib.GT_F32, _lib.GT_OP_SUM, _lib.GT_OP_MAX
 NORM, LOG = _lib.GT_CHILD_NORMALIZE, _lib.GT_CHILD_LOG
-
-
-def golden_vocab(name):
-    if name == "sentinel":
-        from genlm_backend_b200 import Token
-
-        return [Token(0, b"ab"), Token(1, b""), Token(2, b"ab"), Token(3, b"a"), EOS(), b"plain"]
-    g = load_golden(name)
-    return tokens(unflat(g["blob"], g["lens"]))
-
-
-def golden_layout(name):
-    g = load_golden(name)
-    return oracle.OracleLayout(g["idx_to_leaf"], g["jump_ptr"], g["jump_idx"]), g
-
-
-def trie_layout(trie):
-    return oracle.OracleLayout(trie.idx_to_leaf, trie._layout["child_ptr"], trie._layout["child_idx"])
 
 
 def random_logw(rng, shape, frac_neginf=0.3):
@@ -52,7 +33,7 @@ def random_logw(rng, shape, frac_neginf=0.3):
 # ---- CPU ---------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("name", ["toy", "edge", "sentinel", "synth128256"])
 def test_num_symbols_and_labels_host_only(name):
-    dec = synth_vocab(128256) if name == "synth128256" else golden_vocab(name)
+    dec = golden_vocab(name)
     trie = ParallelTokenCharacterTrie(dec)
     S = int(_lib.lib.gt_num_symbols(trie._engine._handle))
     labels = trie.symbol_labels
@@ -148,6 +129,12 @@ def test_symbol_entry_points_reject_bad_arguments_without_a_gpu():
     assert masses(ops=SUM, m=None, flags=NORM | LOG, work_bytes=16) == 3  # too small
     assert b"workspace too small" in lib.gt_last_error()
     assert masses(n=0) == 0
+    # the order of the checks: scalars and strides, the early return for no rows, data pointers, the workspace
+    nulls = dict(ws=None, nodes=None, s=None, m=None, work=None)
+    assert masses(n=0, **nulls) == 0
+    for bad in (dict(ops=0), dict(flags=0x40), dict(in_type=7), dict(ld_ws=V - 1), dict(ld_out=S)):
+        assert masses(n=0, **nulls, **bad) == 1, bad
+    assert masses(s=None, work=None) == 1 and b"null data pointer" in lib.gt_last_error()
 
     def sample(**kw):
         a = dict(t=h, ws=p, in_type=F32, n=4, ld_ws=V, nodes=p, w=p, ld_w=0, flags=0, c=p, sy=p, lp=p, lz=p, lm=p,
@@ -163,21 +150,14 @@ def test_symbol_entry_points_reject_bad_arguments_without_a_gpu():
         assert sample(**bad) == 1, bad
     assert sample(work_bytes=16) == 3
     assert sample(n=0) == 0 and sample(n=0, lm=None, ld_w=S + 1) == 0
+    nulls = dict(ws=None, nodes=None, w=None, c=None, sy=None, lp=None, lz=None, lm=None, work=None)
+    assert sample(n=0, **nulls) == 0
+    for bad in (dict(flags=NORM), dict(in_type=-1), dict(ld_ws=V - 1), dict(ld_w=S), dict(ld_w=-1)):
+        assert sample(n=0, **nulls, **bad) == 1, bad
+    assert sample(sy=None, work=None) == 1 and b"null data pointer" in lib.gt_last_error()
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------------
-def assert_within_ulp(have, want):
-    """fp32 results within one fp32 ulp of fp64 values; exact zeros and infinities kept."""
-    have = np.asarray(have, dtype=np.float64)
-    want = np.asarray(want, dtype=np.float64)
-    fin = np.isfinite(want)
-    assert np.array_equal(have[~fin], want[~fin], equal_nan=True)
-    assert (have[want == 0] == 0).all()
-    ulp = np.spacing(np.abs(want[fin]).astype(np.float32)).astype(np.float64)
-    err = np.abs(have[fin] - want[fin])
-    assert (err <= ulp).all(), float((err / np.maximum(ulp, 1e-300)).max())
-
-
 def kernel_weights(x, log_input):
     """The weights the kernels reduce: the fp32 conversion of the input, exponentiated for log inputs."""
     x32 = x.float().cpu().numpy()
@@ -239,7 +219,7 @@ def child_columns(trie, ids):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["edge", "synth3000", "synth128256"])
 def test_bit_equal_to_child_masses_and_slab_max(name):
-    dec = synth_vocab(128256) if name == "synth128256" else golden_vocab(name)
+    dec = golden_vocab(name)
     trie = ParallelTokenCharacterTrie(dec)
     N, V, S = len(trie), len(dec), trie.num_symbols
     rng = np.random.default_rng(3)
@@ -277,7 +257,7 @@ def test_bit_equal_to_child_masses_and_slab_max(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["edge", "synth128256"])
 def test_zero_log_weights_reproduce_sample_next_symbol(name):
-    dec = synth_vocab(128256) if name == "synth128256" else golden_vocab(name)
+    dec = golden_vocab(name)
     trie = ParallelTokenCharacterTrie(dec)
     N, V, S = len(trie), len(dec), trie.num_symbols
     B = 1024
@@ -294,12 +274,6 @@ def test_zero_log_weights_reproduce_sample_next_symbol(name):
         cc = c.cpu().numpy()
         want_sym = np.where(cc >= 0, child_columns(trie, cc[None, :])[0], -1)
         assert np.array_equal(sy.cpu().numpy(), want_sym)
-
-
-def _depth1(trie):
-    kids = trie.jump[trie.root]
-    internal = [int(c) for c in kids if len(trie.jump[c])]
-    return max(internal, key=lambda c: len(trie.jump[c]))
 
 
 def _chi_square(counts, p):
@@ -325,7 +299,7 @@ def test_weighted_draw_chi_square(where):
     if where == "shared_end":  # the node spelling b"ab": three leaf children (items 0, 2, 8) and the child b"c"
         node = int(trie._layout["parent"][trie.idx_to_leaf[0, 1]])
     else:
-        node = trie.root if where == "root" else _depth1(trie)
+        node = trie.root if where == "root" else depth1_node(trie)
     row = dirichlet_rows(1, len(dec), alpha=1.0, seed=21)
     logw = random_logw(np.random.default_rng(9), S + 1)
     if where == "shared_end":  # the three items split in proportion to their masses; b"abc" is never drawn
