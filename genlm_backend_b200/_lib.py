@@ -67,6 +67,15 @@ SIGNATURES = {
                                  c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
     "gt_symbol_sample": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_uint, c_uint64,
                                  c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gt_child_masses_masked": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                       c_void_p, c_void_p, c_int64, c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
+    "gt_child_sample_masked": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_uint,
+                                       c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "gt_symbol_masses_masked": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                        c_void_p, c_int64, c_uint, c_uint, c_void_p, c_size_t, c_void_p]),
+    "gt_symbol_sample_masked": (c_int, [c_void_p, c_void_p, c_int, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                        c_int64, c_uint, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                        c_void_p, c_size_t, c_void_p]),
     "gt_dfa_token_mask": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
                                   c_void_p]),
     "gt_dfa_advance": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,

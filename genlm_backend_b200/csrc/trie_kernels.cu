@@ -1239,7 +1239,8 @@ __global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanVie
 }
 
 // ---- next-symbol read-outs: masses of the children of one node per row, by child or by symbol, and the draw ---------
-// (gt_child_masses / gt_child_sample / gt_symbol_masses / gt_symbol_sample)
+// (gt_child_masses / gt_child_sample / gt_symbol_masses / gt_symbol_sample, and their *_masked twins, which restrict
+// the rows to the items a per-row keep-bitmask allows: only the block kernel differs, by a compile-time parameter)
 //
 // The children of a node n tile its DFS leaf range [lo(n), hi(n)) with consecutive ranges (post-order numbering, DESIGN
 // section 2), so the job is a segmented reduction over one contiguous range of DFS ranks per row, with at most D segments.
@@ -1274,6 +1275,8 @@ struct ChildArgs {
     int32_t* child_out; float* logp_out; float* logZ_out; uint64_t seed, ctr0;  // ctr0 = offset + first row of the chunk
     // ... optional: per-row symbol log-weights (row stride ld_w, 0 = shared), the drawn symbol and the node's log-mass
     const float* sym_logw; int64_t ld_w; int32_t* symbol_out; float* logM_out;
+    // the *_masked calls: keep-bitmask in item order (GT_MASK_BITS_U32), row stride mask_ld words (0 = shared)
+    const uint32_t* mask; int64_t mask_ld;
 };
 
 // Children CSR range and DFS leaf range of node n; false for an id outside [0, N) and for a leaf.
@@ -1329,29 +1332,55 @@ template <typename IN_T> __device__ __forceinline__ void load_quad(const IN_T* p
     }
 }
 
-// Block k of row b (one warp).
-template <typename IN_T>
+// Bit i of the keep-bitmask row m (item order, bit i % 32 of word i / 32).
+__device__ __forceinline__ bool mask_keeps(const uint32_t* m, int i) { return (__ldg(m + (i >> 5)) >> (i & 31)) & 1u; }
+
+// Block k of row b (one warp).  MASKED: an item whose bit in the row's keep-bitmask is 0 contributes the weight 0.f
+// (its weight is not loaded where that is cheap), which is the converted weight of a zeroed row (-inf under
+// GT_FLAG_LOG_INPUT): every sum, its order and every max are those of the zeroed row.
+template <typename IN_T, bool MASKED>
 __device__ __forceinline__ void child_block(const PlanView& P, const ChildArgs& A, int b, int k, int lane) {
     int cp0 = 0, deg = 0, lo = 0, hi = 0;
     child_node(P, __ldg(A.nodes + b), cp0, deg, lo, hi);  // true: the row has blocks
     const int w0 = lo + k * kChildBlock, w1 = min(hi, w0 + kChildBlock);
     const IN_T* row = static_cast<const IN_T*>(A.ws) + (size_t)b * A.ld_ws;
     const bool log_input = A.log_input != 0;
+    const uint32_t* mrow = MASKED ? A.mask + (size_t)b * A.mask_ld : nullptr;
     // the weights of this lane's ranks w0 + 4 lane + 128 q + i (0 outside the block; never added)
     float f[kChildQuads][4];
     if (A.dfs_order) {  // contiguous: one vector load per quad where the row allows it
+        unsigned keep = 0xffffu;  // MASKED: bit 4 q + i is the mask bit of rank w0 + 4 lane + 128 q + i
+        if constexpr (MASKED) {  // the rank's item perm[r], then its mask word
+            keep = 0;
+#pragma unroll
+            for (int q = 0; q < kChildQuads; ++q)
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int r = w0 + 4 * lane + 128 * q + i;
+                    if (r < w1 && mask_keeps(mrow, __ldg(P.perm + r))) keep |= 1u << (4 * q + i);
+                }
+        }
         const bool vec = (reinterpret_cast<uintptr_t>(row + w0) & (sizeof(IN_T) == 2 ? 7 : 15)) == 0;
 #pragma unroll
         for (int q = 0; q < kChildQuads; ++q) {
             const int r0 = w0 + 4 * lane + 128 * q;
             if (vec && r0 + 4 <= w1) {
-                IN_T x[4];
-                load_quad<IN_T>(row + r0, x);
+                if (!MASKED || ((keep >> (4 * q)) & 15u)) {
+                    IN_T x[4];
+                    load_quad<IN_T>(row + r0, x);
 #pragma unroll
-                for (int i = 0; i < 4; ++i) f[q][i] = convert_in<float, IN_T>(x[i], log_input);
+                    for (int i = 0; i < 4; ++i) f[q][i] = convert_in<float, IN_T>(x[i], log_input);
+                } else {
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) f[q][i] = 0.f;
+                }
             } else {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) f[q][i] = r0 + i < w1 ? convert_in<float, IN_T>(__ldg(row + r0 + i), log_input) : 0.f;
+            }
+            if constexpr (MASKED) {  // the cleared bits of a quad loaded as a whole, and of a block's edge
+#pragma unroll
+                for (int i = 0; i < 4; ++i) f[q][i] = (keep >> (4 * q + i)) & 1u ? f[q][i] : 0.f;
             }
         }
     } else {  // vocabulary order: ws[b, perm[r]], perm read coalesced (L2-resident metadata)
@@ -1371,7 +1400,9 @@ __device__ __forceinline__ void child_block(const PlanView& P, const ChildArgs& 
 #pragma unroll
         for (int q = 0; q < kChildQuads; ++q)
 #pragma unroll
-            for (int i = 0; i < 4; ++i) f[q][i] = pi[q][i] >= 0 ? convert_in<float, IN_T>(__ldg(row + pi[q][i]), log_input) : 0.f;
+            for (int i = 0; i < 4; ++i)
+                f[q][i] = pi[q][i] >= 0 && (!MASKED || mask_keeps(mrow, pi[q][i]))
+                              ? convert_in<float, IN_T>(__ldg(row + pi[q][i]), log_input) : 0.f;
     }
 
     // first child whose range ends past w0: narrow [a, z] about 31-fold per round (hi(c_z) > w0 holds throughout).  The
@@ -1424,6 +1455,8 @@ __device__ __forceinline__ void child_block(const PlanView& P, const ChildArgs& 
 }
 
 // Three CTAs per SM: 70 registers without spills (the default budget for these parameters was 64, which spilled).
+// MASKED (the *_masked calls) is a separate instantiation, so the unmasked kernel is the code it was without masks.
+template <bool MASKED>
 __global__ void __launch_bounds__(kChildThreads, 3) child_block_kernel(PlanView P, ChildArgs A) {
     __shared__ int s_off[kMaxChildRows + 1];
     pdl_wait();  // rows, node ids and the work list come from earlier kernels; the slots may still be read by the last chunk
@@ -1439,7 +1472,7 @@ __global__ void __launch_bounds__(kChildThreads, 3) child_block_kernel(PlanView 
             const int mid = (lo + hi + 1) >> 1;
             if (s_off[mid] <= u) lo = mid; else hi = mid - 1;
         }
-        GT_IN_TYPE_SWITCH(A.in_type, (child_block<IN_T>(P, A, lo, u - s_off[lo], lane)));
+        GT_IN_TYPE_SWITCH(A.in_type, (child_block<IN_T, MASKED>(P, A, lo, u - s_off[lo], lane)));
     }
 }
 
@@ -1684,10 +1717,10 @@ static int resident_plan(const gt_trie* t, const PlanView*& v) {
     return GT_OK;
 }
 
-// Shared by gt_child_masses, gt_child_sample, gt_symbol_masses and gt_symbol_sample: arguments are checked by the
-// callers (before any CUDA call); this selects the device plan and launches scan -> blocks -> finish per chunk of rows,
-// chained with programmatic dependent launch on the caller's stream.  A.nodes / A.ws / outputs point at row 0; chunk c
-// advances them.
+// Shared by gt_child_masses, gt_child_sample, gt_symbol_masses and gt_symbol_sample and their *_masked twins: arguments
+// are checked by the callers (before any CUDA call); this selects the device plan and launches scan -> blocks -> finish
+// per chunk of rows, chained with programmatic dependent launch on the caller's stream.  A.nodes / A.ws / A.mask /
+// outputs point at row 0; chunk c advances them.  A mask selects the masked instantiation of the block kernel.
 static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t out_ld_rows, uint64_t offset, void* workspace,
                         size_t workspace_bytes, cudaStream_t st, const char* what, void (*finish)(PlanView, ChildArgs)) {
     const int64_t slots = ChildScratch::slots(t->layout);
@@ -1701,7 +1734,8 @@ static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t o
     const PlanView& v = *pv;
     const size_t in_size = A.in_type == GT_F64 ? 8 : A.in_type == GT_F32 ? 4 : 2;
     const int64_t max_blocks = (t->layout.V + kChildBlock - 1) / kChildBlock;
-    const int resident = sm_count() * resident_ctas(reinterpret_cast<const void*>(child_block_kernel), kChildThreads, 0);
+    void (*block)(PlanView, ChildArgs) = A.mask ? child_block_kernel<true> : child_block_kernel<false>;
+    const int resident = sm_count() * resident_ctas(reinterpret_cast<const void*>(block), kChildThreads, 0);
     A.blk_off = sc.blk_off; A.part_sum = sc.part_sum; A.part_max = sc.part_max; A.slots = slots;
     const char* ws0 = static_cast<const char*>(A.ws);
     const int32_t* nodes0 = A.nodes;
@@ -1720,11 +1754,12 @@ static int launch_child(const gt_trie* t, ChildArgs A, int64_t n_rows, int64_t o
         if (A.symbol_out) C.symbol_out = A.symbol_out + r0;
         if (A.logM_out) C.logM_out = A.logM_out + r0;
         if (A.sym_logw) C.sym_logw = A.sym_logw + (size_t)r0 * A.ld_w;
+        if (A.mask) C.mask = A.mask + (size_t)r0 * A.mask_ld;
         C.ctr0 = offset + (uint64_t)r0;
         const int64_t blocks_ub = (int64_t)rows * max_blocks;  // every row at the root
         const unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(resident, (blocks_ub + kChildThreads / 32 - 1) / (kChildThreads / 32)));
         GT_CUDA(launch_pdl(child_scan_kernel, dim3(1), dim3(1024), 0, st, v, C));
-        GT_CUDA(launch_pdl(child_block_kernel, dim3(grid), dim3(kChildThreads), 0, st, v, C));
+        GT_CUDA(launch_pdl(block, dim3(grid), dim3(kChildThreads), 0, st, v, C));
         GT_CUDA(launch_pdl(finish, dim3((unsigned)((rows + kChildThreads / 32 - 1) / (kChildThreads / 32))),
                            dim3(kChildThreads), 0, st, v, C));
     }
@@ -1891,12 +1926,14 @@ size_t gt_child_workspace_bytes(const gt_trie* t, int64_t max_rows) {
 
 static bool child_in_type_ok(int in_type) { return in_type == GT_F32 || in_type == GT_F64 || in_type == GT_F16 || in_type == GT_BF16; }
 
-// Checks shared by the four next-symbol read-outs.  Each call makes its checks in one order: the scalars and strides
+// Checks shared by the next-symbol read-outs.  Each of the four calls and its *_masked twin share one implementation
+// (the unmasked call passes no mask), which makes its checks in one order: the scalars and strides
 // (child_check_scalars, then its own), the early return for no rows, the data pointers (its own outputs, then
 // child_check_pointers) and last the workspace, so that a call without rows accepts null pointers.
 // child_check_scalars fills the input half of A.
 static int child_check_scalars(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws,
-                               const int32_t* nodes, unsigned flags, unsigned known, const char* what, gt::ChildArgs& A) {
+                               const int32_t* nodes, const uint32_t* mask, int64_t mask_ld, unsigned flags, unsigned known,
+                               const char* what, gt::ChildArgs& A) {
     if (!t) { gt::set_error("%s: null trie", what); return GT_ERR_ARG; }
     if (n_rows < 0 || (flags & ~known) || !child_in_type_ok(in_type)) {
         gt::set_error("%s: bad n_rows / flags / input type", what); return GT_ERR_ARG;
@@ -1904,14 +1941,22 @@ static int child_check_scalars(const gt_trie* t, const void* ws, int in_type, in
     if (ld_ws < t->layout.V) {
         gt::set_error("%s: row stride %lld smaller than V = %lld", what, (long long)ld_ws, (long long)t->layout.V); return GT_ERR_ARG;
     }
-    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws; A.nodes = nodes;
+    const int64_t words = (t->layout.V + 31) / 32;
+    if (mask_ld < 0 || (mask_ld > 0 && mask_ld < words)) {
+        gt::set_error("%s: mask row stride %lld is neither 0 (shared) nor >= ceil(V/32) = %lld", what, (long long)mask_ld,
+                      (long long)words);
+        return GT_ERR_ARG;
+    }
+    A.ws = ws; A.in_type = in_type; A.ld_ws = ld_ws; A.nodes = nodes; A.mask = mask; A.mask_ld = mask_ld;
     A.log_input = (flags & GT_FLAG_LOG_INPUT) ? 1 : 0; A.dfs_order = (flags & GT_FLAG_DFS_ORDER) ? 1 : 0;
     A.normalize = (flags & GT_CHILD_NORMALIZE) ? 1 : 0; A.log_out = (flags & GT_CHILD_LOG) ? 1 : 0;
     return GT_OK;
 }
 
-static int child_check_pointers(const gt_trie* t, const void* ws, const int32_t* nodes, const void* workspace, const char* what) {
-    if ((t->layout.V > 0 && !ws) || !nodes) { gt::set_error("%s: null data pointer", what); return GT_ERR_ARG; }
+// masked: the *_masked twin, which needs its mask.
+static int child_check_pointers(const gt_trie* t, const void* ws, const int32_t* nodes, bool masked, const uint32_t* mask,
+                                const void* workspace, const char* what) {
+    if ((t->layout.V > 0 && !ws) || !nodes || (masked && !mask)) { gt::set_error("%s: null data pointer", what); return GT_ERR_ARG; }
     if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 255)) {
         gt::set_error("%s: workspace must be a 256-byte aligned device pointer", what); return GT_ERR_ARG;
     }
@@ -1921,88 +1966,153 @@ static int child_check_pointers(const gt_trie* t, const void* ws, const int32_t*
 static const unsigned kMassesFlags = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER | GT_CHILD_NORMALIZE | GT_CHILD_LOG;
 static const unsigned kSampleFlags = GT_FLAG_LOG_INPUT | GT_FLAG_DFS_ORDER;
 
-int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
-                    int32_t* child_ids, float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
-                    void* workspace, size_t workspace_bytes, gt_stream stream) {
+static int child_masses_impl(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                             bool masked, const uint32_t* mask_bits, int64_t mask_ld, int32_t* child_ids, float* out_sum,
+                             float* out_max, int64_t ld_out, unsigned ops, unsigned flags, void* workspace,
+                             size_t workspace_bytes, gt_stream stream, const char* what) {
     gt::ChildArgs A{};
-    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kMassesFlags, __func__, A);
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, mask_bits, mask_ld, flags, kMassesFlags, what, A);
     if (rc != GT_OK) return rc;
     const int64_t D = t->layout.max_children;
     if (!ops_ok(ops) || ld_out < D) {
-        gt::set_error("%s: bad ops, or output row stride %lld smaller than D = %lld", __func__, (long long)ld_out, (long long)D);
+        gt::set_error("%s: bad ops, or output row stride %lld smaller than D = %lld", what, (long long)ld_out, (long long)D);
         return GT_ERR_ARG;
     }
     if (n_rows == 0 || D == 0) return GT_OK;
     if (!child_ids || ((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
-        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
+        gt::set_error("%s: null data pointer", what); return GT_ERR_ARG;
     }
-    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
+    if ((rc = child_check_pointers(t, ws, nodes, masked, mask_bits, workspace, what)) != GT_OK) return rc;
     A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
     A.child_ids = child_ids; A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr;
     A.ld_out = ld_out; A.D = (int)D;
-    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), what,
                             gt::child_masses_kernel);
+}
+
+int gt_child_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                    int32_t* child_ids, float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                    void* workspace, size_t workspace_bytes, gt_stream stream) {
+    return child_masses_impl(t, ws, in_type, n_rows, ld_ws, nodes, false, nullptr, 0, child_ids, out_sum, out_max, ld_out, ops,
+                             flags, workspace, workspace_bytes, stream, __func__);
+}
+
+int gt_child_masses_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                           const uint32_t* mask_bits, int64_t mask_ld, int32_t* child_ids, float* out_sum, float* out_max,
+                           int64_t ld_out, unsigned ops, unsigned flags, void* workspace, size_t workspace_bytes,
+                           gt_stream stream) {
+    return child_masses_impl(t, ws, in_type, n_rows, ld_ws, nodes, true, mask_bits, mask_ld, child_ids, out_sum, out_max,
+                             ld_out, ops, flags, workspace, workspace_bytes, stream, __func__);
+}
+
+static int child_sample_impl(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                             bool masked, const uint32_t* mask_bits, int64_t mask_ld, unsigned flags, uint64_t seed,
+                             uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out, void* workspace,
+                             size_t workspace_bytes, gt_stream stream, const char* what) {
+    gt::ChildArgs A{};
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, mask_bits, mask_ld, flags, kSampleFlags, what, A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0) return GT_OK;
+    if (!child_out || !logp_out || !logZ_out) { gt::set_error("%s: null data pointer", what); return GT_ERR_ARG; }
+    if ((rc = child_check_pointers(t, ws, nodes, masked, mask_bits, workspace, what)) != GT_OK) return rc;
+    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), what,
+                            gt::child_draw_kernel);
 }
 
 int gt_child_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                     unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, float* logp_out, float* logZ_out,
                     void* workspace, size_t workspace_bytes, gt_stream stream) {
-    gt::ChildArgs A{};
-    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kSampleFlags, __func__, A);
-    if (rc != GT_OK) return rc;
-    if (n_rows == 0) return GT_OK;
-    if (!child_out || !logp_out || !logZ_out) { gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG; }
-    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
-    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
-    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
-                            gt::child_draw_kernel);
+    return child_sample_impl(t, ws, in_type, n_rows, ld_ws, nodes, false, nullptr, 0, flags, seed, offset, child_out, logp_out,
+                             logZ_out, workspace, workspace_bytes, stream, __func__);
 }
 
-int gt_symbol_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
-                     float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
-                     void* workspace, size_t workspace_bytes, gt_stream stream) {
+int gt_child_sample_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                           const uint32_t* mask_bits, int64_t mask_ld, unsigned flags, uint64_t seed, uint64_t offset,
+                           int32_t* child_out, float* logp_out, float* logZ_out, void* workspace, size_t workspace_bytes,
+                           gt_stream stream) {
+    return child_sample_impl(t, ws, in_type, n_rows, ld_ws, nodes, true, mask_bits, mask_ld, flags, seed, offset, child_out,
+                             logp_out, logZ_out, workspace, workspace_bytes, stream, __func__);
+}
+
+static int symbol_masses_impl(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                              bool masked, const uint32_t* mask_bits, int64_t mask_ld, float* out_sum, float* out_max,
+                              int64_t ld_out, unsigned ops, unsigned flags, void* workspace, size_t workspace_bytes,
+                              gt_stream stream, const char* what) {
     gt::ChildArgs A{};
-    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kMassesFlags, __func__, A);
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, mask_bits, mask_ld, flags, kMassesFlags, what, A);
     if (rc != GT_OK) return rc;
     const int64_t S = t->layout.num_symbols;
     if (!ops_ok(ops) || ld_out < S + 1) {
-        gt::set_error("%s: bad ops, or output row stride %lld smaller than S + 1 = %lld", __func__, (long long)ld_out,
+        gt::set_error("%s: bad ops, or output row stride %lld smaller than S + 1 = %lld", what, (long long)ld_out,
                       (long long)(S + 1));
         return GT_ERR_ARG;
     }
     if (n_rows == 0) return GT_OK;
     if (((ops & GT_OP_SUM) && !out_sum) || ((ops & GT_OP_MAX) && !out_max)) {
-        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
+        gt::set_error("%s: null data pointer", what); return GT_ERR_ARG;
     }
-    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
+    if ((rc = child_check_pointers(t, ws, nodes, masked, mask_bits, workspace, what)) != GT_OK) return rc;
     A.need_max = (ops & GT_OP_MAX) ? 1 : 0;
     A.out_sum = (ops & GT_OP_SUM) ? out_sum : nullptr; A.out_max = (ops & GT_OP_MAX) ? out_max : nullptr; A.ld_out = ld_out;
-    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
+    return gt::launch_child(t, A, n_rows, ld_out, 0, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), what,
                             gt::symbol_masses_kernel);
+}
+
+int gt_symbol_masses(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                     float* out_sum, float* out_max, int64_t ld_out, unsigned ops, unsigned flags,
+                     void* workspace, size_t workspace_bytes, gt_stream stream) {
+    return symbol_masses_impl(t, ws, in_type, n_rows, ld_ws, nodes, false, nullptr, 0, out_sum, out_max, ld_out, ops, flags,
+                              workspace, workspace_bytes, stream, __func__);
+}
+
+int gt_symbol_masses_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                            const uint32_t* mask_bits, int64_t mask_ld, float* out_sum, float* out_max, int64_t ld_out,
+                            unsigned ops, unsigned flags, void* workspace, size_t workspace_bytes, gt_stream stream) {
+    return symbol_masses_impl(t, ws, in_type, n_rows, ld_ws, nodes, true, mask_bits, mask_ld, out_sum, out_max, ld_out, ops,
+                              flags, workspace, workspace_bytes, stream, __func__);
+}
+
+static int symbol_sample_impl(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                              bool masked, const uint32_t* mask_bits, int64_t mask_ld, const float* sym_logw, int64_t ld_w,
+                              unsigned flags, uint64_t seed, uint64_t offset, int32_t* child_out, int32_t* symbol_out,
+                              float* logp_out, float* logZ_out, float* logM_out, void* workspace, size_t workspace_bytes,
+                              gt_stream stream, const char* what) {
+    gt::ChildArgs A{};
+    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, mask_bits, mask_ld, flags, kSampleFlags, what, A);
+    if (rc != GT_OK) return rc;
+    const int64_t S = t->layout.num_symbols;
+    if (ld_w < 0 || (ld_w > 0 && ld_w < S + 1)) {
+        gt::set_error("%s: log-weight row stride %lld is neither 0 (shared) nor >= S + 1 = %lld", what, (long long)ld_w,
+                      (long long)(S + 1));
+        return GT_ERR_ARG;
+    }
+    if (n_rows == 0) return GT_OK;
+    if (!sym_logw || !child_out || !symbol_out || !logp_out || !logZ_out) {
+        gt::set_error("%s: null data pointer", what); return GT_ERR_ARG;
+    }
+    if ((rc = child_check_pointers(t, ws, nodes, masked, mask_bits, workspace, what)) != GT_OK) return rc;
+    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
+    A.sym_logw = sym_logw; A.ld_w = ld_w; A.symbol_out = symbol_out; A.logM_out = logM_out;
+    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), what,
+                            gt::child_draw_kernel);
 }
 
 int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
                      const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
                      int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
                      void* workspace, size_t workspace_bytes, gt_stream stream) {
-    gt::ChildArgs A{};
-    int rc = child_check_scalars(t, ws, in_type, n_rows, ld_ws, nodes, flags, kSampleFlags, __func__, A);
-    if (rc != GT_OK) return rc;
-    const int64_t S = t->layout.num_symbols;
-    if (ld_w < 0 || (ld_w > 0 && ld_w < S + 1)) {
-        gt::set_error("%s: log-weight row stride %lld is neither 0 (shared) nor >= S + 1 = %lld", __func__, (long long)ld_w,
-                      (long long)(S + 1));
-        return GT_ERR_ARG;
-    }
-    if (n_rows == 0) return GT_OK;
-    if (!sym_logw || !child_out || !symbol_out || !logp_out || !logZ_out) {
-        gt::set_error("%s: null data pointer", __func__); return GT_ERR_ARG;
-    }
-    if ((rc = child_check_pointers(t, ws, nodes, workspace, __func__)) != GT_OK) return rc;
-    A.seed = seed; A.child_out = child_out; A.logp_out = logp_out; A.logZ_out = logZ_out;
-    A.sym_logw = sym_logw; A.ld_w = ld_w; A.symbol_out = symbol_out; A.logM_out = logM_out;
-    return gt::launch_child(t, A, n_rows, 0, offset, workspace, workspace_bytes, static_cast<cudaStream_t>(stream), __func__,
-                            gt::child_draw_kernel);
+    return symbol_sample_impl(t, ws, in_type, n_rows, ld_ws, nodes, false, nullptr, 0, sym_logw, ld_w, flags, seed, offset,
+                              child_out, symbol_out, logp_out, logZ_out, logM_out, workspace, workspace_bytes, stream, __func__);
+}
+
+int gt_symbol_sample_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                            const uint32_t* mask_bits, int64_t mask_ld, const float* sym_logw, int64_t ld_w, unsigned flags,
+                            uint64_t seed, uint64_t offset, int32_t* child_out, int32_t* symbol_out, float* logp_out,
+                            float* logZ_out, float* logM_out, void* workspace, size_t workspace_bytes, gt_stream stream) {
+    return symbol_sample_impl(t, ws, in_type, n_rows, ld_ws, nodes, true, mask_bits, mask_ld, sym_logw, ld_w, flags, seed,
+                              offset, child_out, symbol_out, logp_out, logZ_out, logM_out, workspace, workspace_bytes, stream,
+                              __func__);
 }
 
 // Checks shared by the two DFA entry points (host only, before any CUDA call); fills the kernels' table / row arguments.

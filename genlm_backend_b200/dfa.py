@@ -6,7 +6,17 @@ both proposals of a constrained sampler:
 
 - token level: ``trie.dfa_token_mask(delta, states)`` -> ``smc.masked_logsumexp_sample`` -> ``trie.dfa_advance``;
 - byte level: ``symbol_logw(delta, states)`` -> ``trie.sample_next_symbol_weighted``; after a byte draw the next state is
-  ``delta[states, symbol]``, a plain gather (a drawn end of token, symbol ``S``, keeps the state).
+  ``delta[states, symbol]``, a plain gather (a drawn end of token, symbol ``S``, keeps the state).  This looks one symbol
+  ahead only: a byte can get weight 1 although most tokens below it are rejected later.
+- exact byte level: the token mask, computed once per token at the root, restricts the byte read-outs; drawing byte by
+  byte from the root under it draws exactly from the masked token distribution of ``smc.masked_logsumexp_sample``::
+
+      bits = trie.dfa_token_mask(delta, q)                    # once per token, at the root
+      child, label, logp, logZ = trie.sample_next_symbol(ws, n, mask=bits, seed=s, offset=k)   # per byte; logZ at the root = the token's weight increment
+      # a drawn leaf child ends token -1 - label; then q = trie.dfa_advance(delta, q, tok)
+
+  The mask stays valid for every byte of the token: the walk from the root equals the walk from ``n`` in the state
+  reached at ``n``.
 
 Several constraints in one call: stack their tables into one ``delta`` with disjoint state ranges (add each table's
 offset to its non-negative entries) and give each row its own start state.

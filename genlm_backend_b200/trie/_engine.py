@@ -369,61 +369,95 @@ class TrieEngine:
         self.ensure_device(ws.device.index)
         return ws, nodes, B, (ws.stride(0) if B > 1 else max(self.V, 1))
 
-    def child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
-        """``gt_child_masses`` on the current stream of the input's device.  Returns ``(child_ids int32[B, D],
-        sums float32[B, D] | None, maxes float32[B, D] | None)``; nothing is synchronised."""
+    def keep_bits(self, mask, B, device):
+        """A keep-mask for ``B`` rows as ``(bits, mask_ld)`` in ``GT_MASK_BITS_U32`` layout on ``device``: an int32
+        bitmask ``[ceil(V/32)]`` (shared, ``mask_ld = 0``) or ``[B, ceil(V/32)]`` (per row, any row stride of at least
+        ``ceil(V/32)``), or a bool keep-mask ``[V]`` / ``[B, V]``, packed.  Anything else raises ``ValueError``."""
+        from ..smc import _pack_keep_bits
+
+        V, W = self.V, (self.V + 31) // 32
+        mask = torch.as_tensor(mask)
+        if mask.dtype == torch.bool and mask.dim() in (1, 2) and mask.shape[-1] == V and (mask.dim() == 1 or mask.shape[0] == B):
+            keep = torch.nn.functional.pad(mask.to(device), (0, W * 32 - V))  # each row a whole number of words
+            mask = _pack_keep_bits(keep.reshape(-1)).view(keep.shape[:-1] + (W,))
+        elif mask.dtype != torch.int32 or mask.dim() not in (1, 2) or mask.shape[-1] != W or (mask.dim() == 2 and mask.shape[0] != B):
+            raise ValueError(f"mask must be an int32 keep-bitmask [{W}] or [{B}, {W}] (ceil(V/32) words per row), or a bool "
+                             f"keep-mask [{V}] or [{B}, {V}]; got {mask.dtype} of shape {tuple(mask.shape)}")
+        mask = mask.to(device)
+        if mask.dim() == 1:
+            return mask.contiguous(), 0
+        if mask.stride(1) != 1 or (B > 1 and mask.stride(0) < W):
+            mask = mask.contiguous()
+        return mask, (mask.stride(0) if B > 1 else W)
+
+    def _read_out(self, fn, mask, B, device):
+        """The entry point of a next-symbol read-out and the arguments that follow ``nodes``: ``fn`` without a mask,
+        ``fn + "_masked"`` with the mask's bits and row stride otherwise (``keep`` holds the bits until the launch)."""
+        if mask is None:
+            return fn, (), None
+        bits, ld = self.keep_bits(mask, B, device)
+        return fn + "_masked", (bits.data_ptr(), ld), bits
+
+    def child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False, mask=None):
+        """``gt_child_masses`` (``gt_child_masses_masked`` with a ``mask``, see ``keep_bits``) on the current stream of
+        the input's device.  Returns ``(child_ids int32[B, D], sums float32[B, D] | None, maxes float32[B, D] | None)``;
+        nothing is synchronised."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
         opmask = _opmask(ops)
         D, dev = self.max_children, ws.device
+        fn, margs, _keep = self._read_out("gt_child_masses", mask, B, dev)
         ids = torch.empty((B, D), dtype=torch.int32, device=dev)
         sums = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
         maxes = torch.empty((B, D), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
         if B and D:
             self._launch(
-                "gt_child_masses", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                fn, dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), *margs,
                 ids.data_ptr(), sums.data_ptr() if sums is not None else None,
                 maxes.data_ptr() if maxes is not None else None, D, opmask, _flags(log_input, dfs_order, normalize, log),
                 workspace=self._child_workspace, rows=B,
             )
         return ids, sums, maxes
 
-    def child_sample(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False):
-        """``gt_child_sample`` on the current stream of the input's device: ``(child int32[B], logp float32[B],
-        logZ float32[B])``; nothing is synchronised."""
+    def child_sample(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False, mask=None):
+        """``gt_child_sample`` (``gt_child_sample_masked`` with a ``mask``) on the current stream of the input's device:
+        ``(child int32[B], logp float32[B], logZ float32[B])``; nothing is synchronised."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
         dev = ws.device
+        fn, margs, _keep = self._read_out("gt_child_sample", mask, B, dev)
         child = torch.empty(B, dtype=torch.int32, device=dev)
         logp = torch.empty(B, dtype=torch.float32, device=dev)
         logZ = torch.empty(B, dtype=torch.float32, device=dev)
         if B:
             self._launch(
-                "gt_child_sample", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                fn, dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), *margs,
                 _flags(log_input, dfs_order), int(seed) & (2**64 - 1), int(offset) & (2**64 - 1), child.data_ptr(),
                 logp.data_ptr(), logZ.data_ptr(), workspace=self._child_workspace, rows=B,
             )
         return child, logp, logZ
 
     # ---- the same, indexed by symbol ---------------------------------------------------------------------------
-    def symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
-        """``gt_symbol_masses`` on the current stream of the input's device.  Returns ``(sums float32[B, S+1] | None,
-        maxes float32[B, S+1] | None)``; nothing is synchronised."""
+    def symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False, mask=None):
+        """``gt_symbol_masses`` (``gt_symbol_masses_masked`` with a ``mask``) on the current stream of the input's device.
+        Returns ``(sums float32[B, S+1] | None, maxes float32[B, S+1] | None)``; nothing is synchronised."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
         opmask = _opmask(ops)
         W, dev = self.num_symbols + 1, ws.device
+        fn, margs, _keep = self._read_out("gt_symbol_masses", mask, B, dev)
         sums = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_SUM else None
         maxes = torch.empty((B, W), dtype=torch.float32, device=dev) if opmask & _lib.GT_OP_MAX else None
         if B:
             self._launch(
-                "gt_symbol_masses", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                fn, dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), *margs,
                 sums.data_ptr() if sums is not None else None, maxes.data_ptr() if maxes is not None else None, W, opmask,
                 _flags(log_input, dfs_order, normalize, log), workspace=self._child_workspace, rows=B,
             )
         return sums, maxes
 
-    def symbol_sample(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False):
-        """``gt_symbol_sample`` on the current stream of the input's device: ``(child int32[B], symbol int32[B],
-        logp float32[B], logZ float32[B], logM float32[B])``; nothing is synchronised.  ``symbol_logw``: ``[S+1]``
-        (shared by all rows) or ``[B, S+1]``, converted to contiguous float32 on the input's device."""
+    def symbol_sample(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False, mask=None):
+        """``gt_symbol_sample`` (``gt_symbol_sample_masked`` with a ``mask``) on the current stream of the input's device:
+        ``(child int32[B], symbol int32[B], logp float32[B], logZ float32[B], logM float32[B])``; nothing is
+        synchronised.  ``symbol_logw``: ``[S+1]`` (shared by all rows) or ``[B, S+1]``, converted to contiguous float32
+        on the input's device."""
         ws, nodes, B, ld_ws = self._child_inputs(ws, nodes)
         W, dev = self.num_symbols + 1, ws.device
         logw = torch.as_tensor(symbol_logw)
@@ -433,6 +467,7 @@ class TrieEngine:
             raise ValueError(f"symbol_logw must hold floating-point log-weights, got {logw.dtype}")
         logw = logw.to(device=dev, dtype=torch.float32).contiguous()
         ld_w = 0 if logw.dim() == 1 else W
+        fn, margs, _keep = self._read_out("gt_symbol_sample", mask, B, dev)
         child = torch.empty(B, dtype=torch.int32, device=dev)
         symbol = torch.empty(B, dtype=torch.int32, device=dev)
         logp = torch.empty(B, dtype=torch.float32, device=dev)
@@ -440,7 +475,7 @@ class TrieEngine:
         logM = torch.empty(B, dtype=torch.float32, device=dev)
         if B:
             self._launch(
-                "gt_symbol_sample", dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(),
+                fn, dev.index, self._handle, ws.data_ptr(), _IN_TYPES[ws.dtype], B, ld_ws, nodes.data_ptr(), *margs,
                 logw.data_ptr(), ld_w, _flags(log_input, dfs_order), int(seed) & (2**64 - 1), int(offset) & (2**64 - 1),
                 child.data_ptr(), symbol.data_ptr(), logp.data_ptr(), logZ.data_ptr(), logM.data_ptr(),
                 workspace=self._child_workspace, rows=B,

@@ -247,7 +247,8 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
             ws = ws.to(torch.device("cuda", self._device_list()[0]), non_blocking=True)
         return ws
 
-    def batch_child_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+    def batch_child_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False,
+                                  mask=None):
         """Masses of the children of one node per row, computed from the rows alone (the ``[B, N]`` slab is never
         formed; only the leaves under ``nodes[b]`` are read).
 
@@ -256,14 +257,21 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         degree are padding (id ``-1``, mass 0 -- ``-inf`` with ``log``); an invalid id or a leaf gives a padding row.
         Sums are accumulated in fp64 and rounded once; ``normalize`` divides them by the node's mass (the conditional
         next-symbol distribution); ``log`` returns logs of both.  Maxes equal ``batch_weight_max_tensor(ws)`` at the ids.
-        ``dfs_order`` as for ``batch_weight_tensor``."""
-        return self._engine.child_masses(self._child_rows(ws), nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
-                                         normalize=normalize, log=log)
+        ``dfs_order`` as for ``batch_weight_tensor``.
 
-    def batch_child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+        ``mask``: restrict the rows to the tokens a keep-mask allows -- an int32 keep-bitmask ``[ceil(V/32)]`` (shared) or
+        ``[B, ceil(V/32)]`` (what ``dfa_token_mask`` and ``subtree_token_mask`` return; any row stride of at least
+        ``ceil(V/32)``), or a bool keep-mask ``[V]`` / ``[B, V]``, always in token order.  The results are bit for bit those
+        for rows whose masked-out weights are 0 (``-inf`` with ``log_input``), computed without that ``[B, V]`` pass: a
+        masked-out weight (NaN and inf included) never contributes, and a child without an allowed token has mass 0."""
+        return self._engine.child_masses(self._child_rows(ws), nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
+                                         normalize=normalize, log=log, mask=mask)
+
+    def batch_child_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False,
+                           mask=None):
         """``batch_child_masses_tensor`` as numpy arrays."""
         out = self.batch_child_masses_tensor(ws, nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
-                                             normalize=normalize, log=log)
+                                             normalize=normalize, log=log, mask=mask)
         return tuple(None if t is None else t.cpu().numpy() for t in out)
 
     def _edge_labels_on(self, device):
@@ -273,7 +281,7 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
             lab = cache[device.index] = torch.from_numpy(self.edge_labels).to(device)
         return lab
 
-    def sample_next_symbol(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False, check_valid=False):
+    def sample_next_symbol(self, ws, nodes, seed=0, offset=0, log_input=False, dfs_order=False, check_valid=False, mask=None):
         """One draw of the next symbol per row from the children of ``nodes[b]``, in proportion to their masses.
 
         Returns ``(child, label, logp, logZ)`` device tensors: the chosen child (int32), its ``edge_labels`` entry (a
@@ -281,10 +289,14 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         Row ``b`` uses the Philox counter ``offset + b`` under key ``seed`` (as ``smc.masked_logsumexp_sample``).  A row
         without mass (also a leaf or an invalid id) gives ``child = -1``, ``label = INT32_MIN`` and ``logZ = -inf``; a NaN
         weight under the node gives ``logZ = NaN``.  ``check_valid``: synchronise and raise ``RuntimeError`` like
-        ``torch.multinomial`` when a row has no mass or a NaN."""
+        ``torch.multinomial`` when a row has no mass or a NaN.
+
+        ``mask`` (as for ``batch_child_masses_tensor``): draw among the allowed tokens only.  With one token mask per
+        particle, drawing symbol by symbol from the root until a leaf child draws exactly from the masked token
+        distribution of ``smc.masked_logsumexp_sample``, and ``logZ`` at the root is that call's ``logZ``."""
         ws = self._child_rows(ws)
         child, logp, logZ = self._engine.child_sample(ws, nodes, seed=seed, offset=offset, log_input=log_input,
-                                                      dfs_order=dfs_order)
+                                                      dfs_order=dfs_order, mask=mask)
         lab = self._edge_labels_on(child.device)
         label = torch.where(child >= 0, lab[child.clamp(min=0).long()], torch.full_like(child, np.iinfo(np.int32).min))
         if check_valid and child.numel():
@@ -313,25 +325,27 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         in order of first appearance."""
         return list(self._edge_labels)
 
-    def batch_symbol_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+    def batch_symbol_masses_tensor(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False,
+                                   mask=None):
         """``batch_child_masses_tensor`` laid out by symbol: ``(sums float32[B, S+1] | None, maxes float32[B, S+1] |
         None)`` on the input's device, on its current stream, without a sync.
 
         Column ``s < S`` is the child of ``nodes[b]`` whose edge symbol is ``s`` (0 -- ``-inf`` with ``log`` -- when
         there is none); column ``S`` adds up (sum) or maxes over all leaf children of the node, i.e. the items whose
         spelling ends there.  The values of the non-end columns are bit-equal to those of ``batch_child_masses_tensor``
-        under the same flags; an invalid id or a leaf gives a padding row."""
+        under the same flags; an invalid id or a leaf gives a padding row.  ``mask`` as for ``batch_child_masses_tensor``."""
         return self._engine.symbol_masses(self._child_rows(ws), nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
-                                          normalize=normalize, log=log)
+                                          normalize=normalize, log=log, mask=mask)
 
-    def batch_symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False):
+    def batch_symbol_masses(self, ws, nodes, ops=("sum",), log_input=False, dfs_order=False, normalize=False, log=False,
+                            mask=None):
         """``batch_symbol_masses_tensor`` as numpy arrays."""
         out = self.batch_symbol_masses_tensor(ws, nodes, ops=ops, log_input=log_input, dfs_order=dfs_order,
-                                              normalize=normalize, log=log)
+                                              normalize=normalize, log=log, mask=mask)
         return tuple(None if t is None else t.cpu().numpy() for t in out)
 
     def sample_next_symbol_weighted(self, ws, nodes, symbol_logw, seed=0, offset=0, log_input=False, dfs_order=False,
-                                    check_valid=False):
+                                    check_valid=False, mask=None):
         """One draw of the next symbol per row in proportion to ``mass(child) * exp(symbol_logw[b, symbol(child)])``.
 
         ``symbol_logw`` holds log-weights by symbol, ``[S+1]`` (shared by every row) or ``[B, S+1]``; its last column
@@ -341,10 +355,11 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         log-mass.  Counters and key as in ``sample_next_symbol``; with all log-weights 0 the child, ``logp`` and
         ``logZ`` are those of ``sample_next_symbol``.  A row without a draw gives child and symbol ``-1`` and
         ``logZ = -inf`` (no weighted mass), NaN (a NaN weight or log-weight) or ``+inf``.  ``check_valid``:
-        synchronise and raise ``RuntimeError`` like ``torch.multinomial`` for such rows."""
+        synchronise and raise ``RuntimeError`` like ``torch.multinomial`` for such rows.  ``mask`` as for
+        ``sample_next_symbol``: the masses, and so ``log_mass``, count the allowed tokens only."""
         ws = self._child_rows(ws)
         child, symbol, logp, logZ, logM = self._engine.symbol_sample(ws, nodes, symbol_logw, seed=seed, offset=offset,
-                                                                     log_input=log_input, dfs_order=dfs_order)
+                                                                     log_input=log_input, dfs_order=dfs_order, mask=mask)
         if check_valid and child.numel():
             bad = child < 0
             if bool(bad.any()):

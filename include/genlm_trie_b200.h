@@ -27,6 +27,10 @@
  *                               per-symbol weight vector of a byte-level potential
  *   gt_symbol_sample            the draw of the next symbol in proportion to mass(child) * weight(symbol), with the
  *                               weighted normaliser (the particle's weight increment)
+ *   gt_child_masses_masked, gt_child_sample_masked, gt_symbol_masses_masked, gt_symbol_sample_masked
+ *                               the same four over the tokens a keep-bitmask allows: what a caller gets today by
+ *                               torch.where(keep, ws, 0) over the whole [B, V] rows before the unmasked call; drawn
+ *                               symbol by symbol from the root, the masked token draw of README.md:82-91
  *   gt_dfa_token_mask           the host-side walk of every token's bytes through a constraint's automaton that a
  *                               constrained token sampler does to build the mask of README.md:82-91's masked draw
  *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
@@ -293,6 +297,39 @@ int gt_symbol_sample(const gt_trie* t, const void* ws, int in_type, int64_t n_ro
                      const float* sym_logw, int64_t ld_w, unsigned flags, uint64_t seed, uint64_t offset,
                      int32_t* child_out, int32_t* symbol_out, float* logp_out, float* logZ_out, float* logM_out,
                      void* workspace, size_t workspace_bytes, gt_stream stream);
+
+/* ---- the next-symbol read-outs restricted to the items a per-row keep-bitmask allows -------------------------------- */
+
+/* gt_child_masses / gt_child_sample / gt_symbol_masses / gt_symbol_sample over the allowed items only.  mask_bits: device
+ * keep-bitmask in GT_MASK_BITS_U32 layout and item order (bit i % 32 of word i / 32 = 1: item i is kept) -- what
+ * gt_dfa_token_mask and gt_subtree_token_mask write; row b's mask starts at mask_bits + b * mask_ld words, mask_ld = 0
+ * shares one mask between all rows, else mask_ld >= ceil(V/32).  Bits at or above V are ignored.
+ * Every result -- ids, sums, maxes, normalised and log outputs, and the child, symbol, logp, logZ and logM of the draws
+ * under the same seed and offset -- is bit for bit that of the unmasked call on rows whose masked-out weights are 0
+ * (-inf with GT_FLAG_LOG_INPUT): a masked-out weight never contributes, NaN and inf included; a child without an
+ * allowed item has sum and max 0 (-inf with GT_CHILD_LOG) and is never drawn; a row without allowed mass under its node
+ * gives child -1 and logZ = -inf; an all-ones mask gives the unmasked results.  For a byte-level DFA, the mask of
+ * gt_dfa_token_mask at the root in the particle's state stays valid for every symbol of the token: drawing symbol by
+ * symbol from the root under it draws exactly from the masked token distribution of gt_lse_sample, and the root's
+ * logZ is that call's logZ.  Only the leaves under nodes[b] and their mask words are read; a weight whose bit is 0 is
+ * not read where its load can be skipped.  Argument checks, in order: the unmasked call's scalars and mask_ld (< 0, or
+ * between 0 and ceil(V/32): GT_ERR_ARG); no rows returns GT_OK, null pointers accepted; the data pointers (a null
+ * mask_bits: GT_ERR_ARG); the workspace.  No allocation, no synchronisation, graph-capturable. */
+int gt_child_masses_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                           const uint32_t* mask_bits, int64_t mask_ld, int32_t* child_ids, float* out_sum, float* out_max,
+                           int64_t ld_out, unsigned ops, unsigned flags, void* workspace, size_t workspace_bytes,
+                           gt_stream stream);
+int gt_child_sample_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                           const uint32_t* mask_bits, int64_t mask_ld, unsigned flags, uint64_t seed, uint64_t offset,
+                           int32_t* child_out, float* logp_out, float* logZ_out, void* workspace, size_t workspace_bytes,
+                           gt_stream stream);
+int gt_symbol_masses_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                            const uint32_t* mask_bits, int64_t mask_ld, float* out_sum, float* out_max, int64_t ld_out,
+                            unsigned ops, unsigned flags, void* workspace, size_t workspace_bytes, gt_stream stream);
+int gt_symbol_sample_masked(const gt_trie* t, const void* ws, int in_type, int64_t n_rows, int64_t ld_ws, const int32_t* nodes,
+                            const uint32_t* mask_bits, int64_t mask_ld, const float* sym_logw, int64_t ld_w, unsigned flags,
+                            uint64_t seed, uint64_t offset, int32_t* child_out, int32_t* symbol_out, float* logp_out,
+                            float* logZ_out, float* logM_out, void* workspace, size_t workspace_bytes, gt_stream stream);
 
 /* ---- token masks under a byte-level DFA, and the DFA advance over drawn tokens ------------------------------------ */
 
