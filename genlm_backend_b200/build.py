@@ -18,8 +18,10 @@ LIB_PATH = os.path.join(PKG_DIR, LIB_NAME)
 EXTRA_DEFINES = os.environ.get("GT_NVCC_DEFINES", "").split()
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 
-SOURCES = ["trie_builder.cpp", "trie_plan.cpp", "trie_kernels.cu", "sampler_kernels.cu"]
-HEADERS = [os.path.join(CSRC, "trie_internal.h"), os.path.join(CSRC, "philox.cuh"), os.path.join(INCLUDE, "genlm_trie_b200.h")]
+SOURCES = ["trie_builder.cpp", "trie_plan.cpp", "device_plan.cu", "mass_kernels.cu", "token_mask_kernels.cu",
+           "child_kernels.cu", "sampler_kernels.cu"]
+HEADERS = [os.path.join(CSRC, h) for h in ("trie_internal.h", "trie_device.cuh", "philox.cuh")] + [
+    os.path.join(INCLUDE, "genlm_trie_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -10,14 +10,10 @@
 // elements, which are re-read from L2 (a few KB).
 // The draw is an exact inverse CDF over a fixed permutation of the vocabulary, so it is distributed as
 // the reference's multinomial but is not stream-identical to torch's generator.
-#include <cuda_runtime.h>
-#include <cuda_fp16.h>
-#include <cuda_bf16.h>
-
 #include <cstdint>
 #include <type_traits>
 
-#include "trie_internal.h"
+#include "trie_device.cuh"
 #include "philox.cuh"
 
 namespace gt {
@@ -45,12 +41,6 @@ struct SampleArgs {
     float inv_temp; uint64_t seed, offset;
     float* logZ; int32_t* tok;
 };
-
-template <typename T> __device__ __forceinline__ float elem_to_float(T x);
-template <> __device__ __forceinline__ float elem_to_float<float>(float x) { return x; }
-template <> __device__ __forceinline__ float elem_to_float<double>(double x) { return (float)x; }
-template <> __device__ __forceinline__ float elem_to_float<__half>(__half x) { return __half2float(x); }
-template <> __device__ __forceinline__ float elem_to_float<__nv_bfloat16>(__nv_bfloat16 x) { return __bfloat162float(x); }
 
 // Per-row view: groups of EPV elements aligned to 16 bytes in global memory.
 //
@@ -149,7 +139,7 @@ template <typename IN_T, int MK> struct RowView {
     template <bool VEC> __device__ __forceinline__ void finish(const Cursor& c, int dg, const Raw& raw, float y[EPV]) const {
         const IN_T* e = reinterpret_cast<const IN_T*>(&raw.v);
 #pragma unroll
-        for (int k = 0; k < EPV; ++k) y[k] = elem_to_float<IN_T>(e[k]);
+        for (int k = 0; k < EPV; ++k) y[k] = in_to_float<IN_T>(e[k]);
         if (MK == GT_MASK_ADD_F32 && VEC) {
             const float* ma = reinterpret_cast<const float*>(&raw.ma);
             const float* mb = reinterpret_cast<const float*>(&raw.mb);
@@ -174,7 +164,7 @@ template <typename IN_T, int MK> struct RowView {
 #pragma unroll
         for (int k = 0; k < EPV; ++k) {
             const int i = i0 + k;
-            y[k] = (i >= 0 && i < V) ? mask_apply(elem_to_float<IN_T>(row[i]), i) : -INFINITY;
+            y[k] = (i >= 0 && i < V) ? mask_apply(in_to_float<IN_T>(row[i]), i) : -INFINITY;
         }
     }
     __device__ __forceinline__ void fetch(int g, float y[EPV]) const {
@@ -460,9 +450,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) lse_sample_kernel(SampleArgs A)
 }
 
 template <typename IN_T, int MK> static int launch_sampler_mk(const SampleArgs& A, cudaStream_t st) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
     const int grid = A.n_rows < sms * 8 ? A.n_rows : sms * 8;
     // 2-byte rows under an additive fp32 mask move twice as many mask bytes as row bytes per group and measured faster
     // with two wide CTAs per SM (40 vs 51 us); every other combination prefers four CTAs of kSThreads

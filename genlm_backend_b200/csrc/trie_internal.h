@@ -64,11 +64,7 @@ inline int32_t swizzle_slot(int32_t s, int32_t slot_bytes) {
 // 8: 256 leaves per warp.  7 (128 leaves per warp, all eight compute warps of a 1024-leaf tile busy) was measured
 // slower on B200 (tile kernel 50.2 vs 48.6 us at 64 rows): the phase is bound by shared-memory bandwidth, not by the
 // number of warps that work, and the 256-leaf blocks come back as extra two-term ranges.
-#ifndef GT_PYR_TOP
-#define GT_PYR_TOP 8
-#endif
-constexpr int kPyramidTop = GT_PYR_TOP;
-static_assert(kPyramidTop == 7 || kPyramidTop == 8, "pyramid top level must be 7 or 8");
+constexpr int kPyramidTop = 8;
 
 // Term rows of an ELL chunk are padded (with the identity slot) to a multiple of this.  The kernel adds terms four at a
 // time and finishes with a pair and / or a single term.  Measured on B200 (tile kernel, 64 rows, both reductions):
@@ -119,7 +115,7 @@ struct Plan {
     int32_t n_pieces = 0;
 };
 
-struct DevicePlan;  // defined in the CUDA translation unit
+struct DevicePlan;  // defined in trie_device.cuh
 void free_device_plan(DevicePlan*);
 
 }  // namespace gt

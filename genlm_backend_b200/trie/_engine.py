@@ -2,7 +2,7 @@
 per GPU, caches scratch buffers, and launches ``gt_weight_reduce`` on torch's current stream.
 
 PyTorch is used for device memory, streams and host<->device copies only; every reduction runs in the
-hand-written kernels behind the C ABI (``csrc/trie_kernels.cu``).  There is no CPU path.
+hand-written kernels behind the C ABI (``csrc/mass_kernels.cu``).  There is no CPU path.
 """
 import ctypes
 import os

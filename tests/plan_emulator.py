@@ -1,4 +1,4 @@
-"""CPU emulation of the data flow of csrc/trie_kernels.cu, driven by the plan arrays the C++ planner produced
+"""CPU emulation of the data flow of csrc/mass_kernels.cu, driven by the plan arrays the C++ planner produced
 (gt_export_plan_array).  Test infrastructure: it lets the ``-m "not gpu"`` suite check the planner's metadata
 (staging layout, value slots, aligned-block decomposition, spanning fix-up) against the oracle without a GPU.
 Float32 arithmetic in the same association order as the kernels (pairwise pyramid, sequential term sums).
