@@ -78,6 +78,8 @@ SIGNATURES = {
                                         c_void_p, c_size_t, c_void_p]),
     "gt_dfa_token_mask": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_int64,
                                   c_void_p]),
+    "gt_dfa_token_logw": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                  c_int64, c_void_p]),
     "gt_dfa_advance": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
                                c_void_p]),
     "gt_lse_sample": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_float,

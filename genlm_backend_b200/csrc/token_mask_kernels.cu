@@ -1,7 +1,9 @@
 // sm_100a kernels for per-row token masks over the trie: the items under a node (gt_subtree_token_mask), the items a
-// byte DFA accepts from there (gt_dfa_token_mask), and the DFA state after a drawn token (gt_dfa_advance).
+// byte DFA accepts from there (gt_dfa_token_mask), their log-weights under a weighted byte DFA (gt_dfa_token_logw), and
+// the DFA state after a drawn token (gt_dfa_advance).
 #include <climits>
 #include <algorithm>
+#include <type_traits>
 
 #include "trie_device.cuh"
 
@@ -36,7 +38,7 @@ __global__ void __launch_bounds__(kMaskThreads) subtree_mask_kernel(PlanView P, 
     }
 }
 
-// ---- token masks under a byte DFA (gt_dfa_token_mask / gt_dfa_advance) ------------------------------------------------
+// ---- token masks under a byte DFA (gt_dfa_token_mask / gt_dfa_token_logw / gt_dfa_advance) ----------------------------
 //
 // Row b stands at node n = nodes[b] (the root without nodes) in DFA state q = states[b].  Item i is allowed iff its leaf
 // lies under n, q is live (in [0, Q)) and delta walked from q over the item's symbols depth(n) .. len(i)-1 never leaves
@@ -75,8 +77,14 @@ __device__ __forceinline__ int dfa_step(const DfaArgs& A, int q, int s) {
     return (unsigned)nq < (unsigned)A.Q ? nq : -1;
 }
 
-__global__ void __launch_bounds__(kDfaThreads) dfa_mask_kernel(PlanView P, DfaArgs A, uint32_t* __restrict__ bits, int64_t ld_bits,
-                                                               int64_t words) {
+// kLogw = false (gt_dfa_token_mask): out holds keep-bitmask words, ld_out words per row, words of them written.
+// kLogw = true (gt_dfa_token_logw): out[b, i] is the fp64 sum of logw[q_k, s_k] over the walked transitions, in
+// increasing k and rounded once to fp32, where the bit would be set, else -inf; ld_out floats per row, the first V
+// written, words unused.  logw has delta's shape and is loaded at delta's index, as an independent load, so the chain
+// of dependent table loads does not grow.  A -inf accumulator does not stop the walk: only the states decide it.
+template <bool kLogw>
+__global__ void __launch_bounds__(kDfaThreads) dfa_mask_kernel(PlanView P, DfaArgs A, std::conditional_t<kLogw, float, uint32_t>* __restrict__ out,
+                                                               int64_t ld_out, int64_t words, const float* __restrict__ logw) {
     __shared__ int s_q[kDfaRows], s_lo[kDfaRows], s_d[kDfaRows];
     __shared__ unsigned s_len[kDfaRows];
     const int b0 = blockIdx.y * kDfaRows;
@@ -96,6 +104,7 @@ __global__ void __launch_bounds__(kDfaThreads) dfa_mask_kernel(PlanView P, DfaAr
     }
     __syncthreads();
     int st[kDfaRows], dk[kDfaRows];
+    double acc[kDfaRows] = {};
     int k0 = INT_MAX;
 #pragma unroll
     for (int g = 0; g < kDfaRows; ++g) {
@@ -110,18 +119,30 @@ __global__ void __launch_bounds__(kDfaThreads) dfa_mask_kernel(PlanView P, DfaAr
         bool any = false;
 #pragma unroll
         for (int g = 0; g < kDfaRows; ++g) {
-            if (st[g] >= 0 && k >= dk[g]) st[g] = dfa_step(A, st[g], s);
+            if (st[g] >= 0 && k >= dk[g]) {
+                if constexpr (kLogw) acc[g] += (double)__ldg(logw + st[g] * A.ld + s);
+                st[g] = dfa_step(A, st[g], s);
+            }
             any |= st[g] >= 0;
         }
         if (!any) break;
     }
-    const int64_t w = i >> 5;
     const int rows = min(kDfaRows, A.n_rows - b0);
+    if constexpr (kLogw) {
+        if (i >= P.V) return;
 #pragma unroll
-    for (int g = 0; g < kDfaRows; ++g) {
-        if (g >= rows) break;
-        const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
-        if ((threadIdx.x & 31) == 0 && w < words) bits[(size_t)(b0 + g) * ld_bits + w] = word;
+        for (int g = 0; g < kDfaRows; ++g) {  // consecutive threads store consecutive items: one coalesced store per warp
+            if (g >= rows) break;
+            out[(size_t)(b0 + g) * ld_out + i] = st[g] >= 0 ? (float)acc[g] : -INFINITY;
+        }
+    } else {
+        const int64_t w = i >> 5;
+#pragma unroll
+        for (int g = 0; g < kDfaRows; ++g) {
+            if (g >= rows) break;
+            const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
+            if ((threadIdx.x & 31) == 0 && w < words) out[(size_t)(b0 + g) * ld_out + w] = word;
+        }
     }
 }
 
@@ -197,7 +218,28 @@ int gt_dfa_token_mask(const gt_trie* t, const int32_t* delta, int64_t n_states, 
     // the grid covers whole mask words: ceil(V/32) of them, kDfaThreads/32 per CTA
     dim3 grid((unsigned)((words * 32 + gt::kDfaThreads - 1) / gt::kDfaThreads), (unsigned)((n_rows + gt::kDfaRows - 1) / gt::kDfaRows));
     gt::NvtxRange nv("gt:dfa_mask");
-    gt::dfa_mask_kernel<<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, mask_bits, mask_ld, words);
+    gt::dfa_mask_kernel<false><<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, mask_bits, mask_ld, words, nullptr);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
+}
+
+int gt_dfa_token_logw(const gt_trie* t, const int32_t* delta, const float* logw, int64_t n_states, int64_t ld_delta,
+                      const int32_t* states, const int32_t* nodes, int64_t n_rows, float* out, int64_t ld_out, gt_stream stream) {
+    if (!t) { gt::set_error("gt_dfa_token_logw: null trie"); return GT_ERR_ARG; }
+    if (!delta || !logw || !states || !out) { gt::set_error("gt_dfa_token_logw: null data pointer"); return GT_ERR_ARG; }
+    const int64_t V = t->layout.V;
+    if (ld_out < V) { gt::set_error("gt_dfa_token_logw: ld_out %lld < V = %lld", (long long)ld_out, (long long)V); return GT_ERR_ARG; }
+    gt::DfaArgs A{};
+    const int rc = dfa_args(t, delta, n_states, ld_delta, states, nodes, n_rows, "gt_dfa_token_logw", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0 || V == 0) return GT_OK;
+    if (n_rows > (int64_t)65535 * gt::kDfaRows) { gt::set_error("gt_dfa_token_logw: too many rows"); return GT_ERR_LIMIT; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
+    // the same grid as gt_dfa_token_mask's: ceil(ceil(V/32) * 32 / kDfaThreads) = ceil(V / kDfaThreads)
+    dim3 grid((unsigned)((V + gt::kDfaThreads - 1) / gt::kDfaThreads), (unsigned)((n_rows + gt::kDfaRows - 1) / gt::kDfaRows));
+    gt::NvtxRange nv("gt:dfa_logw");
+    gt::dfa_mask_kernel<true><<<grid, gt::kDfaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, out, ld_out, 0, logw);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }

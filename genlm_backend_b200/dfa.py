@@ -18,8 +18,25 @@ both proposals of a constrained sampler:
   The mask stays valid for every byte of the token: the walk from the root equals the walk from ``n`` in the state
   reached at ``n``.
 
+Soft constraints: a deterministic weighted byte automaton adds a float32 table ``logw[Q, S]`` of the same shape,
+``logw[q, s]`` the log-weight of the transition from ``q`` on ``s`` (the EOS column holds the final weights).  A weighted
+regex, a byte n-gram prior or a length or format penalty are all such tables.  A token's log-weight is the sum of the
+transition log-weights along its remaining bytes, ``-inf`` where the Boolean mask rejects it:
+
+- token level: ``tokw = trie.dfa_token_logw(delta, logw, q)`` -> ``logZ, tok = smc.masked_logsumexp_sample(logps, tokw)``
+  -> ``q = trie.dfa_advance(delta, q, tok)``; ``logZ = log sum_i p_i w_i`` is the particle's weight increment and
+  ``tok`` is drawn from ``p w / Z``;
+- exact byte level: ``trie.sample_next_symbol(logps + tokw, n, log_input=True, seed=s, offset=k)`` per byte, with one
+  ``tokw`` per token, computed at the root; the root's ``logZ`` is the token-level weight increment;
+- one symbol ahead: ``symbol_logw(delta, q, logw=logw)`` -> ``trie.sample_next_symbol_weighted``.
+
+Prefix weights: when the potential is a prefix weight ``phi`` given by a deterministic weighted automaton, the table
+after standard weight pushing makes the log-weights along token ``t`` sum to ``log phi(x t) - log phi(x)``, the exact
+token-level factor.  Computing the pushed table (a linear solve for cyclic automata) is left to the caller.
+
 Several constraints in one call: stack their tables into one ``delta`` with disjoint state ranges (add each table's
-offset to its non-negative entries) and give each row its own start state.
+offset to its non-negative entries; their ``logw`` tables stack the same way, unchanged) and give each row its own start
+state.
 """
 import numpy as np
 import torch
@@ -55,18 +72,27 @@ def trim(delta, accepting):
     return np.where(keep, delta, -1).astype(np.int32)
 
 
-def symbol_logw(delta, states, num_symbols=None):
-    """``float32[B, S+1]`` log-weights for ``sample_next_symbol_weighted``: column ``s < S`` is 0 where ``delta[q, s]``
-    is a live state and ``-inf`` elsewhere; column ``S`` ("the token ends here") is 0 iff ``q`` itself is live.  A
-    state outside ``[0, Q)`` gives an all ``-inf`` row.  ``S`` is ``num_symbols`` (default: the table's width).  The
-    result is on the device of ``delta`` when it is a tensor."""
+def symbol_logw(delta, states, num_symbols=None, logw=None):
+    """``float32[B, S+1]`` log-weights for ``sample_next_symbol_weighted``: column ``s < S`` is 0 (``logw[q, s]`` when
+    a weighted table ``logw`` of ``delta``'s shape is given) where ``delta[q, s]`` is a live state and ``-inf``
+    elsewhere; column ``S`` ("the token ends here") is 0 iff ``q`` itself is live.  A state outside ``[0, Q)`` gives an
+    all ``-inf`` row.  ``S`` is ``num_symbols`` (default: the table's width).  The result is on the device of ``delta``
+    when it is a tensor."""
     delta = torch.as_tensor(delta)
     states = torch.as_tensor(states, device=delta.device).reshape(-1).long()
     Q = delta.shape[0]
     S = delta.shape[1] if num_symbols is None else int(num_symbols)
     live = (states >= 0) & (states < Q)
-    nxt = delta[states.clamp(0, Q - 1), :S]
+    rows = states.clamp(0, Q - 1)
+    nxt = delta[rows, :S]
     ok = live[:, None] & (nxt >= 0) & (nxt < Q)
     zero = torch.zeros((), dtype=torch.float32, device=delta.device)
     ninf = torch.full((), float("-inf"), dtype=torch.float32, device=delta.device)
-    return torch.cat([torch.where(ok, zero, ninf), torch.where(live, zero, ninf)[:, None]], dim=1)
+    w = zero
+    if logw is not None:
+        logw = torch.as_tensor(logw)
+        if not logw.is_floating_point() or logw.shape != delta.shape:
+            raise ValueError(f"logw must be a float table of delta's shape {tuple(delta.shape)}, got {logw.dtype} "
+                             f"{tuple(logw.shape)}")
+        w = logw.to(device=delta.device, dtype=torch.float32)[rows, :S]
+    return torch.cat([torch.where(ok, w, ninf), torch.where(live, zero, ninf)[:, None]], dim=1)

@@ -337,6 +337,23 @@ class TrieEngine:
                          states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W)
         return bits
 
+    def dfa_token_logw(self, delta, logw, states, nodes=None):
+        """``gt_dfa_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
+        summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
+        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
+        logw = torch.as_tensor(logw)
+        if not logw.is_floating_point() or logw.shape != delta.shape:
+            raise ValueError(f"logw must be a float table of delta's shape {tuple(delta.shape)}, got {logw.dtype} "
+                             f"{tuple(logw.shape)}")
+        logw = logw.to(device=device, dtype=torch.float32).contiguous()
+        B, V = states.shape[0], self.V
+        out = torch.empty((B, V), dtype=torch.float32, device=device)
+        if B and V:
+            self._launch("gt_dfa_token_logw", device.index, self._handle, delta.data_ptr(), logw.data_ptr(), delta.shape[0],
+                         delta.shape[1], states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B,
+                         out.data_ptr(), V)
+        return out
+
     def dfa_advance(self, delta, states, tokens, nodes=None):
         """``gt_dfa_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after the remaining
         symbols of item ``tokens[b]``, or -1."""

@@ -220,6 +220,18 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         node or state gives an all-zero row.  Runs on the current stream of the inputs' device; no sync."""
         return self._engine.dfa_token_mask(delta, states, nodes)
 
+    def dfa_token_logw(self, delta, logw, states, nodes=None):
+        """``float32[B, V]``: the log-weight of each token under a weighted byte automaton, the additive mask of
+        ``smc.masked_logsumexp_sample``.
+
+        ``delta`` as in ``dfa_token_mask``; ``logw`` is a float table of ``delta``'s shape, ``logw[q, s]`` the
+        log-weight of the transition from ``q`` on symbol ``s`` (converted to float32 on the device).  A token that
+        ``dfa_token_mask`` allows gets the fp64 sum, rounded once to float32, of the log-weights along its remaining
+        symbols (0 when none remain); every other token gets ``-inf``.  IEEE arithmetic decides special values (a
+        ``-inf`` weight on the walk gives ``-inf``, a NaN gives NaN).  With ``logw`` all zero the result is the
+        ``{0, -inf}`` form of ``dfa_token_mask``.  Runs on the current stream of the inputs' device; no sync."""
+        return self._engine.dfa_token_logw(delta, logw, states, nodes)
+
     def dfa_advance(self, delta, states, tokens, nodes=None):
         """``int32[B]``: row ``b``'s DFA state after the remaining symbols of token ``tokens[b]`` (those past
         ``nodes[b]``'s depth), or -1 for a token that ``dfa_token_mask`` does not allow -- also the sampler's "no draw"

@@ -33,6 +33,8 @@
  *                               symbol by symbol from the root, the masked token draw of README.md:82-91
  *   gt_dfa_token_mask           the host-side walk of every token's bytes through a constraint's automaton that a
  *                               constrained token sampler does to build the mask of README.md:82-91's masked draw
+ *   gt_dfa_token_logw           the same walk through a weighted automaton, summing each token's transition
+ *                               log-weights: the additive mask of a soft byte-level potential
  *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
  *
  * Conventions
@@ -353,6 +355,27 @@ int gt_symbol_sample_masked(const gt_trie* t, const void* ws, int in_type, int64
 int gt_dfa_token_mask(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta,
                       const int32_t* states, const int32_t* nodes /* NULL = root */, int64_t n_rows,
                       uint32_t* mask_bits, int64_t mask_ld, gt_stream stream);
+
+/* Per-row token log-weights under a deterministic weighted byte automaton: delta as above, and logw: device fp32, the
+ * same shape and row stride, logw[q * ld_delta + s] the log-weight of the transition from q on symbol s.  For row b, with
+ * n and q as above, out[b * ld_out + i] is
+ *   - for an item gt_dfa_token_mask allows: the sum of (double) logw[q_k, s_k] over k = depth(n) .. len(i)-1, with q_k
+ *     the state before symbol s_k, added in increasing k in fp64 from 0.0 and rounded once to fp32 (0.0f for an item
+ *     with no remaining symbols);
+ *   - -inf for every other item (outside the subtree, an invalid node, a dead or invalid state, a reject on the way).
+ * IEEE arithmetic decides special values: a -inf transition weight makes the token -inf, a NaN weight on the walk or
+ * -inf + +inf gives NaN; the walk does not stop on a -inf sum, only on a reject.  With logw = 0 everywhere, out is the
+ * additive {0, -inf} form of gt_dfa_token_mask's bits, and isfinite(out) is that mask for any finite table whose sums
+ * stay inside the fp32 range.  End of sequence: the EOS column of logw holds the final weight.  The result is
+ * gt_lse_sample's GT_MASK_ADD_F32 mask (mask_ld = ld_out): its logZ is log sum_i p_i w_i, the particle's weight
+ * increment, and its draw is from p w / Z; gt_dfa_advance takes the same delta.  For a prefix weight phi given by a
+ * deterministic weighted automaton, the weight-pushed table makes the row log phi(x t) - log phi(x), the exact
+ * token-level factor.  Writes the first V floats of each row, nothing beyond them; ld_out >= V.  Argument checks, in
+ * order: null t; null delta / logw / states / out; ld_out < V (GT_ERR_ARG); n_states, ld_delta and n_rows as above (a
+ * table of 2^31 entries or more: GT_ERR_LIMIT); no rows returns GT_OK; more rows than the grid takes: GT_ERR_LIMIT. */
+int gt_dfa_token_logw(const gt_trie* t, const int32_t* delta, const float* logw, int64_t n_states, int64_t ld_delta,
+                      const int32_t* states, const int32_t* nodes /* NULL = root */, int64_t n_rows,
+                      float* out, int64_t ld_out, gt_stream stream);
 
 /* states_out[b] = state after item tokens[b]'s symbols depth(nodes[b]) .. end, walked from states[b]; -1 for a token < 0 or
  * >= V (the sampler's "no draw"), a token not under nodes[b], an invalid node, a dead or invalid start state, or any reject

@@ -16,8 +16,20 @@ it times with CUDA events over a CUDA graph of K steps:
   (c) ``dfa_token_mask`` -> ``masked_logsumexp_sample`` -> ``dfa_advance``     the whole step on the trie
   (d) (b) -> ``masked_logsumexp_sample`` -> a torch advance of ``Lmax`` gathers
 
+``--weighted`` times the step under a weighted automaton instead: each table gets seeded log-weights (normal, scale 0.5)
+on its live transitions, and the routes are
+
+  (a) ``dfa_token_logw``                                                       gt_dfa_token_logw
+  (b) the walk of (b) gathering ``delta`` and ``logw`` at each step, an fp64 sum, -inf where rejected
+  (c) ``dfa_token_logw`` -> ``masked_logsumexp_sample(logps, tokw)`` (per-row fp32 additive mask) -> ``dfa_advance``
+  (d) (b) -> ``masked_logsumexp_sample`` -> the torch advance
+  (m) ``dfa_token_mask`` and (s) the Boolean step of (c) above, on the same rows: what the weights and the additive mask
+      cost over the bits (``vs_boolean`` = (a) / (m) and (c) / (s)).
+
+``--routes`` and ``--dfas`` time a subset (comma-separated route and table names).
+
 Step k reads buffer set k % sets of log-softmax rows, states and nodes, with the rows of all sets covering more than three
-times the 126 MB L2.  Before timing, (b) and (d) are checked to compute exactly what (a) and (c) compute.  ``speedup`` is
+times the 126 MB L2.  Before timing, (b) and (d) are checked to compute exactly what (a) and (c) compute (when both are timed).  ``speedup`` is
 (b) / (a) for the mask and (d) / (c) for the step.  Prints one JSON line per (B, dfa, mix, route); ``--out`` also writes
 them to a file.
 """
@@ -85,22 +97,35 @@ class TorchDfa:
         self.depth, self.lo, self.hi = t(depth), t(lay["lo"]), t(lay["hi"])
         self.V = V
 
-    def _walk(self, delta, st, d, sym_of, lens):
+    def _walk(self, delta, st, d, sym_of, lens, logw=None):
         Q, ld = delta.shape
         flat = delta.reshape(-1).long()
+        wflat = None if logw is None else logw.reshape(-1)
+        acc = None if logw is None else torch.zeros(st.shape, dtype=torch.float64, device=st.device)
         for k in range(self.Lmax):
             act = (st >= 0) & (k >= d) & (k < lens)
-            nxt = flat[st.clamp(min=0) * ld + sym_of(k)]
+            idx = st.clamp(min=0) * ld + sym_of(k)
+            nxt = flat[idx]
+            if logw is not None:
+                acc = torch.where(act, acc + wflat[idx].double(), acc)
             st = torch.where(act, torch.where((nxt >= 0) & (nxt < Q), nxt, -1), st)
-        return st
+        return st if logw is None else (st, acc)
 
-    def mask(self, delta, states, nodes):
+    def _start(self, delta, states, nodes):
         Q = delta.shape[0]
         n, q = nodes.long(), states.long()
         inside = ((self.rank[None, :] - self.lo[n][:, None]) >= 0) & (self.rank[None, :] < self.hi[n][:, None])
-        st = torch.where(inside & ((q >= 0) & (q < Q))[:, None], q[:, None], -1)
-        st = self._walk(delta, st, self.depth[n][:, None], lambda k: self.sym[:, k][None, :], self.lens[None, :])
+        return torch.where(inside & ((q >= 0) & (q < Q))[:, None], q[:, None], -1), self.depth[n][:, None]
+
+    def mask(self, delta, states, nodes):
+        st, d = self._start(delta, states, nodes)
+        st = self._walk(delta, st, d, lambda k: self.sym[:, k][None, :], self.lens[None, :])
         return smc._pack_keep_bits((st >= 0).reshape(-1)).view(states.shape[0], -1)  # V is a multiple of 32
+
+    def logw(self, delta, logw, states, nodes):
+        st, d = self._start(delta, states, nodes)
+        st, acc = self._walk(delta, st, d, lambda k: self.sym[:, k][None, :], self.lens[None, :], logw)
+        return torch.where(st >= 0, acc.float(), float("-inf"))
 
     def advance(self, delta, states, nodes, tok):
         Q = delta.shape[0]
@@ -111,11 +136,24 @@ class TorchDfa:
         return st.int()
 
 
+def random_logw(table, seed):
+    """Seeded log-weights on the live transitions of ``table`` (normal, scale 0.5), 0 on the rejecting ones."""
+    rng = np.random.default_rng(seed)
+    return np.where(table >= 0, rng.normal(scale=0.5, size=table.shape), 0).astype(np.float32)
+
+
+def as_tuple(x):
+    return x if isinstance(x, tuple) else (x,)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--batches", default="64,1024")
     ap.add_argument("--steps", type=int, default=20, help="K: steps per CUDA graph")
     ap.add_argument("--reps", type=int, default=10, help="graph replays timed (median reported)")
+    ap.add_argument("--weighted", action="store_true", help="the step under a weighted automaton (legs a-d, m, s)")
+    ap.add_argument("--routes", default=None, help="comma-separated subset of the routes to time")
+    ap.add_argument("--dfas", default="utf8,rand256,rand4096", help="comma-separated subset of the tables")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     assert torch.cuda.is_available(), "dfa_step_bench.py measures on a GPU"
@@ -124,6 +162,8 @@ def main():
     N, S = len(trie), trie.num_symbols
     ref = TorchDfa(trie, "cuda")
     tables = {"utf8": utf8_dfa(S), "rand256": random_dfa(256, S, seed=1), "rand4096": random_dfa(4096, S, seed=2)}
+    seeds = {name: 10 + ti for ti, name in enumerate(tables)}  # the log-weights of a table do not depend on --dfas
+    tables = {name: t for name, t in tables.items() if name in args.dfas.split(",")}
     gpu, power = gpu_info()
     stream = torch.cuda.Stream()
     lines = []
@@ -132,6 +172,7 @@ def main():
         logps = [torch.tensor(logsoftmax_rows(B, V, seed=s)).cuda() for s in range(sets)]
         for name, table in tables.items():
             delta = torch.tensor(table).cuda()
+            logw = torch.tensor(random_logw(table, seed=seeds[name])).cuda()
             Q = table.shape[0]
             for mix in ("root", "depth1"):
                 rng = np.random.default_rng(7)
@@ -149,28 +190,56 @@ def main():
                     _, tok = smc.masked_logsumexp_sample(lp, bits, seed=1)
                     return bits, tok, ref.advance(delta, st, nd, tok)
 
-                for s in range(min(sets, 2)):
-                    for have, want in zip(torch_step(*bufs[s]), kernel_step(*bufs[s])):
-                        assert torch.equal(have, want), (B, name, mix)
+                def kernel_logw_step(lp, st, nd):
+                    tokw = trie.dfa_token_logw(delta, logw, st, nd)
+                    logZ, tok = smc.masked_logsumexp_sample(lp, tokw, seed=1)
+                    return tokw, logZ, tok, trie.dfa_advance(delta, st, tok, nd)
+
+                def torch_logw_step(lp, st, nd):
+                    tokw = ref.logw(delta, logw, st, nd)
+                    logZ, tok = smc.masked_logsumexp_sample(lp, tokw, seed=1)
+                    return tokw, logZ, tok, ref.advance(delta, st, nd, tok)
+
+                if args.weighted:
+                    routes = {
+                        "a_dfa_token_logw": lambda lp, st, nd: trie.dfa_token_logw(delta, logw, st, nd),
+                        "b_torch_logw": lambda lp, st, nd: ref.logw(delta, logw, st, nd),
+                        "c_logw_sample_advance": kernel_logw_step,
+                        "d_torch_logw_sample_advance": torch_logw_step,
+                        "m_dfa_token_mask": lambda lp, st, nd: trie.dfa_token_mask(delta, st, nd),
+                        "s_mask_sample_advance": kernel_step,
+                    }
+                    vs = {"a_dfa_token_logw": "b_torch_logw", "c_logw_sample_advance": "d_torch_logw_sample_advance"}
+                    vs_bool = {"a_dfa_token_logw": "m_dfa_token_mask", "c_logw_sample_advance": "s_mask_sample_advance"}
+                else:
+                    routes = {
+                        "a_dfa_token_mask": lambda lp, st, nd: trie.dfa_token_mask(delta, st, nd),
+                        "b_torch_mask": lambda lp, st, nd: ref.mask(delta, st, nd),
+                        "c_mask_sample_advance": kernel_step,
+                        "d_torch_mask_sample_advance": torch_step,
+                    }
+                    vs, vs_bool = {"a_dfa_token_mask": "b_torch_mask", "c_mask_sample_advance": "d_torch_mask_sample_advance"}, {}
+                if args.routes:
+                    routes = {r: fn for r, fn in routes.items() if r in args.routes.split(",")}
+                for r, other in vs.items():  # the torch composition computes exactly what the kernels compute
+                    if r in routes and other in routes:
+                        for s in range(min(sets, 2)):
+                            for have, want in zip(as_tuple(routes[other](*bufs[s])), as_tuple(routes[r](*bufs[s]))):
+                                assert torch.equal(have, want), (B, name, mix, r)
                 allowed = float(np.mean([smc.masked_logsumexp_sample(lp, trie.dfa_token_mask(delta, st, nd))[1].ge(0)
                                          .float().mean().item() for lp, st, nd in bufs]))
-                routes = {
-                    "a_dfa_token_mask": lambda lp, st, nd: trie.dfa_token_mask(delta, st, nd),
-                    "b_torch_mask": lambda lp, st, nd: ref.mask(delta, st, nd),
-                    "c_mask_sample_advance": kernel_step,
-                    "d_torch_mask_sample_advance": torch_step,
-                }
                 res = {r: time_graph(fn, bufs, args.steps, args.reps, stream) for r, fn in routes.items()}
-                vs = {"a_dfa_token_mask": "b_torch_mask", "c_mask_sample_advance": "d_torch_mask_sample_advance"}
                 for r, (med, best) in res.items():
                     line = {
                         "B": B, "dfa": name, "states": Q, "mix": mix, "route": r, "us_per_step": round(med, 2),
                         "us_per_step_min": round(best, 2),
-                        "speedup": round(res[vs[r]][0] / med, 2) if r in vs else None,
+                        "speedup": round(res[vs[r]][0] / med, 2) if vs.get(r) in res else None,
                         "rows_with_a_draw": round(allowed, 3),
                         "V": V, "N": N, "S": S, "Lmax": ref.Lmax, "buffer_sets": sets, "steps_per_graph": args.steps,
                         "meta_bytes": trie._engine.plan_info()["meta_bytes"], "gpu": gpu, "power_limit": power,
                     }
+                    if args.weighted:
+                        line["vs_boolean"] = round(med / res[vs_bool[r]][0], 3) if vs_bool.get(r) in res else None
                     lines.append(line)
                     print(json.dumps(line), flush=True)
         del logps
