@@ -1,6 +1,6 @@
 // Definitions shared by the CUDA translation units of the library (mass_kernels.cu, token_mask_kernels.cu,
-// child_kernels.cu, sampler_kernels.cu, device_plan.cu): the resident plan, the launch helpers and the element
-// conversions as inline functions and templates, and the host helpers device_plan.cu defines once per process.
+// child_kernels.cu, sampler_kernels.cu, resample_kernels.cu, device_plan.cu): the resident plan, the launch helpers and
+// the element conversions as inline functions and templates, and the host helpers device_plan.cu defines once per process.
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>

@@ -9,7 +9,8 @@ Replaces the per-particle torch sequence of the reference idiom (``README.md:82-
 
 ``masked_logsumexp_sample`` does this for a whole ``[B, V]`` batch of particles without a host sync per row.
 Draws use one Philox uniform per row through an exact inverse CDF: distribution-equal to
-``torch.multinomial``, not stream-equal.
+``torch.multinomial``, not stream-equal.  ``resample`` takes the step an SMC driver takes next: each particle group's
+effective sample size and, below a threshold, its ancestors, again without a host sync.
 """
 import weakref
 
@@ -158,3 +159,73 @@ def masked_logsumexp_sample(logps, mask=None, temperature=1.0, seed=0, offset=0,
     if squeeze:
         return logZ[0], tok[0]
     return logZ, tok
+
+
+_RESAMPLE_METHODS = {"multinomial": _lib.GT_RESAMPLE_MULTINOMIAL, "stratified": _lib.GT_RESAMPLE_STRATIFIED,
+                     "systematic": _lib.GT_RESAMPLE_SYSTEMATIC}
+
+
+def resample(log_weights, method="systematic", ess_threshold=0.5, seed=0, offset=0):
+    """Per-group effective sample size and, where it falls below ``ess_threshold * P``, ancestors drawn on the device.
+
+    The constrained SMC step, weight bookkeeping and reindexing included, runs as one CUDA graph::
+
+        tokw = trie.dfa_token_logw(delta, logw, q)                  # [B, V] token log-weights at the root
+        logZ, tok = smc.masked_logsumexp_sample(logps, tokw, seed=seed, offset=step * B)
+        q = trie.dfa_advance(delta, q, tok)
+        log_weights += logZ
+        anc, log_weights, ess, log_mean_w, resampled = smc.resample(
+            log_weights.view(G, P), "systematic", 0.5, seed=seed, offset=step * B)
+        log_weights = log_weights.view(-1)
+        q = q.index_select(0, anc.view(-1))                        # and every per-particle state of the caller
+        tokens = tokens.index_select(0, anc.view(-1))
+
+    Args:
+        log_weights (torch.Tensor): CUDA log-weights, ``[P]`` for one group or ``[G, P]`` for ``G`` groups of ``P``
+            particles (``P <= 16384``); other float dtypes are converted to float32.
+        method (str): ``"multinomial"``, ``"stratified"`` or ``"systematic"``.
+        ess_threshold (float): a group resamples iff its ESS ``S^2 / Q`` is below ``ess_threshold * P`` (0: never,
+            ``inf``: every group with a positive, finite total).
+        seed, offset (int): Philox key and counter base; particle ``b = g * P + j`` uses counter ``offset + b`` (with
+            the third counter word 1, so the sampler's ``seed`` and ``offset`` give independent uniforms).
+
+    Returns:
+        ``(ancestors, new_log_weights, ess, log_mean_w, resampled)``: ancestors int32 and new log-weights (the group's
+        log mean weight where it resampled, else unchanged) shaped like the input, ancestors as flat indices into the
+        ``G * P`` particles; ``ess`` and ``log_mean_w`` float32 ``[G]``; ``resampled`` bool ``[G]``.  A group with a NaN
+        weight gives ess and log mean weight NaN; one with a ``+inf`` weight ess NaN and ``+inf``; an all ``-inf`` group
+        ess 0 and ``-inf``; none of them resamples.  The full semantics are those of ``gt_resample``
+        (``include/genlm_trie_b200.h``).
+    """
+    if method not in _RESAMPLE_METHODS:
+        raise ValueError(f"unknown resampling method {method!r}: one of {sorted(_RESAMPLE_METHODS)}")
+    if not isinstance(log_weights, torch.Tensor):
+        raise ValueError("log_weights must be a tensor")
+    if log_weights.dim() not in (1, 2):
+        raise ValueError("log_weights must be [P] or [G, P]")
+    if not 1 <= log_weights.shape[-1] <= _lib.GT_RESAMPLE_MAX_GROUP:
+        raise ValueError(f"group size {log_weights.shape[-1]} is not in [1, {_lib.GT_RESAMPLE_MAX_GROUP}]")
+    if not log_weights.is_floating_point():
+        raise ValueError(f"log_weights must be a float tensor, not {log_weights.dtype}")
+    if not log_weights.is_cuda:
+        raise ValueError("log_weights must be a CUDA tensor")
+    shape = log_weights.shape
+    lw = log_weights.to(torch.float32).reshape(-1, shape[-1]).contiguous()
+    G, P = lw.shape
+    dev = lw.device
+    anc = torch.empty((G, P), dtype=torch.int32, device=dev)
+    out = torch.empty((G, P), dtype=torch.float32, device=dev)
+    ess = torch.empty(G, dtype=torch.float32, device=dev)
+    lmw = torch.empty(G, dtype=torch.float32, device=dev)
+    res = torch.empty(G, dtype=torch.bool, device=dev)
+    if G:
+        with torch.cuda.device(dev.index):
+            check(
+                lib.gt_resample(
+                    lw.data_ptr(), G, P, _RESAMPLE_METHODS[method], float(ess_threshold), int(seed) & (2**64 - 1),
+                    int(offset) & (2**64 - 1), anc.data_ptr(), out.data_ptr(), ess.data_ptr(), lmw.data_ptr(),
+                    res.data_ptr(), torch.cuda.current_stream(dev.index).cuda_stream,
+                ),
+                "gt_resample",
+            )
+    return anc.view(shape), out.view(shape), ess, lmw, res

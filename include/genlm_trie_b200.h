@@ -36,6 +36,8 @@
  *   gt_dfa_token_logw           the same walk through a weighted automaton, summing each token's transition
  *                               log-weights: the additive mask of a soft byte-level potential
  *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
+ *   gt_resample                 the effective sample size of each particle group and, below a threshold, the
+ *                               multinomial, stratified or systematic ancestors an SMC driver draws on the host
  *
  * Conventions
  *   - every function returns 0 on success, non-zero on failure; gt_last_error() returns a
@@ -383,6 +385,37 @@ int gt_dfa_token_logw(const gt_trie* t, const int32_t* delta, const float* logw,
 int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta,
                    const int32_t* states, const int32_t* nodes /* NULL = root */, const int32_t* tokens,
                    int64_t n_rows, int32_t* states_out, gt_stream stream);
+
+/* ---- particle resampling: per-group effective sample size and ancestors ----------------------------------------- */
+
+#define GT_RESAMPLE_MULTINOMIAL 0
+#define GT_RESAMPLE_STRATIFIED 1
+#define GT_RESAMPLE_SYSTEMATIC 2
+#define GT_RESAMPLE_MAX_GROUP 16384
+
+/* Particles lie contiguously in n_groups groups of P = group_size: particle b = g * P + j is particle j of group g.  For
+ * group g, with lw_j = logw[g * P + j] and m = max_j lw_j:
+ *   - any NaN: ess = NaN, log_mean_w = NaN; else any +inf: ess = NaN, log_mean_w = +inf; else all -inf: ess = 0,
+ *     log_mean_w = -inf.  None of these resamples.
+ *   - otherwise, in fp64: w_j = exp((double) lw_j - m), S = sum_j w_j, Q = sum_j w_j^2; ess = (float)(S^2 / Q),
+ *     log_mean_w = (float)(m + log S - log P).  The group resamples iff S^2 / Q < ess_threshold * P (fp64): a threshold of
+ *     0 never resamples, +inf always does, and uniform weights (ess exactly P) do not at a threshold of 1.
+ *   - a group that does not resample: ancestors[b] = b, logw_out[b] = logw[b].
+ *   - a group that resamples: with c_i = w_0 + ... + w_i (an fp64 inclusive scan in a fixed order), particle j gets
+ *     ancestors[b] = g * P + i for the first i with c_i > t_j, else the last i with w_i > 0 (a particle with w_i = 0 is
+ *     never an ancestor); logw_out[b] = log_mean_w, which keeps the running marginal-likelihood estimate.  The points are
+ *       multinomial  t_j = u_b * S;  stratified  t_j = (j + u_b) / P * S;  systematic  t_j = (j + u_{g*P}) / P * S,
+ *     so stratified and systematic ancestors are non-decreasing in j and multinomial ones come in draw order.
+ *   - u_b: the 53-bit Philox4x32-10 uniform of the samplers under key seed, with counter offset + b in the first two words
+ *     and 1 (the samplers: 0) in the third, so one (seed, offset) can drive a sampler and the resampler.
+ * ess_out, log_mean_w_out and resampled_out (0 or 1) hold one entry per group.  logw_out may equal logw (in place); any
+ * other overlap is undefined.  A group's results depend only on its weights, P, method, threshold, seed and
+ * offset + g * P.  Argument checks, in order: n_groups < 0, group_size < 1, an unknown method or a NaN threshold:
+ * GT_ERR_ARG; group_size > GT_RESAMPLE_MAX_GROUP or n_groups * P > INT32_MAX: GT_ERR_LIMIT; no groups returns GT_OK, null
+ * pointers accepted; a null pointer: GT_ERR_ARG.  No allocation, no synchronisation, graph-capturable. */
+int gt_resample(const float* logw, int64_t n_groups, int64_t group_size, int method, float ess_threshold,
+                uint64_t seed, uint64_t offset, int32_t* ancestors, float* logw_out, float* ess_out,
+                float* log_mean_w_out, uint8_t* resampled_out, gt_stream stream);
 
 #ifdef __cplusplus
 }
