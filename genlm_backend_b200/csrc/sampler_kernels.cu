@@ -439,6 +439,18 @@ __global__ void __launch_bounds__(NT, 1024 / NT) lse_sample_kernel(SampleArgs A)
         const double resid = s_resid;
         __syncthreads();  // s_pick / s_resid / s_mass are reused below
         if (pick < 0) {
+            if (M == INFINITY) {
+                // A +inf at an allowed position made its thread's sum NaN (inf - inf in the exponent), so logZ was
+                // written NaN above.  As torch.logsumexp: +inf unless an allowed value is NaN; a re-scan decides.
+                bool nan = false;
+                for (int g = tid; g < ng; g += NT) {
+                    float y[EPV];
+                    rv.fetch(g, y);
+#pragma unroll
+                    for (int k = 0; k < EPV; ++k) nan |= y[k] != y[k];
+                }
+                if (__syncthreads_or(nan) == 0 && tid == 0) A.logZ[b] = INFINITY;
+            }
             if (tid == 0) A.tok[b] = -1;
             continue;
         }

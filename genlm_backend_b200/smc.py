@@ -120,7 +120,11 @@ def masked_logsumexp_sample(logps, mask=None, temperature=1.0, seed=0, offset=0,
             mass or a NaN.
 
     Returns:
-        ``(logZ float32[B], tokens int32[B])`` on the device; rows without mass give ``(-inf, -1)``.
+        ``(logZ float32[B], tokens int32[B])`` on the device; rows without mass give ``(-inf, -1)``.  As
+        ``torch.logsumexp``, a row with an allowed NaN gives ``(NaN, -1)``, else one with an allowed ``+inf``
+        ``(+inf, -1)``.  A bool or bit mask drops a masked-out value whatever it is; an additive mask adds ``-inf`` to
+        it, so a masked-out ``+inf`` gives NaN, as in torch.  A shared ``{0, -inf}`` float mask is packed into bits and
+        so drops it too.
     """
     require_cuda()
     if not isinstance(logps, torch.Tensor) or not logps.is_cuda:

@@ -194,7 +194,10 @@ int gt_weight_reduce(const gt_trie* t, const void* ws, int in_type, int64_t n_ro
 
 /* For each row b: masked = logp[b]/temperature + mask;  logZ[b] = logsumexp(masked);
  * tok[b] ~ Categorical(exp(masked - logZ[b])) by inverse CDF with one Philox uniform per row,
- * counter = (seed, offset + b).  Rows with no mass get logZ = -inf, tok = -1.
+ * counter = (seed, offset + b).  Rows with no mass get logZ = -inf, tok = -1.  As torch.logsumexp, an allowed NaN
+ * gives logZ = NaN, else an allowed +inf gives logZ = +inf; both give tok = -1.  A masked-out value is dropped by a
+ * GT_MASK_BOOL_U8 or GT_MASK_BITS_U32 mask whatever it is (NaN and +inf included), while an additive mask adds -inf to
+ * it: a masked-out +inf (or NaN) then makes logZ NaN, as in torch.
  *   mask_ld   elements (floats / bytes / words) between consecutive rows' masks; 0 = shared mask */
 int gt_lse_sample(const void* logp, int in_type, int64_t n_rows, int64_t n_vocab, int64_t ld_logp,
                   const void* mask, int mask_kind, int64_t mask_ld, float temperature,

@@ -3,6 +3,7 @@
 logZ is pinned against torch.logsumexp in float64 (golden, and the numpy float64 oracle); the draw has no
 result-pinning test in the reference ("parity unpinned"), so it is checked by chi-square goodness of fit
 against the exact probabilities and by a two-sample chi-square against a stored torch.multinomial histogram.
+tests/test_draw_replay.py replays every draw exactly against its Philox uniform and an fp64 inverse CDF.
 """
 import numpy as np
 import pytest
