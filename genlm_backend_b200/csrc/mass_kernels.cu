@@ -628,6 +628,7 @@ __global__ void __launch_bounds__(256) span_kernel(PlanView P, MassArgs<VT> A) {
 // ---- host side ---------------------------------------------------------------------------------------
 
 template <typename VT, int R> static size_t mass_smem(const PlanView& v) { return MassSmem(v, (int)sizeof(VT) * R).total; }
+constexpr size_t kMaxMassSmem = 227 * 1024;  // dynamic shared memory one CTA may use on sm_100a
 
 // Scratch layout: a batch is reduced in *chunks* of at most kMaxChunkRows rows (what the staging buffer holds), and the
 // pieces of spanning nodes are collected over a *span group* of up to kMaxSpanRows rows, so that span_kernel runs once
@@ -689,11 +690,7 @@ static int launch_mass(const PlanView& v, const void* ws, int in_type, int64_t l
         GT_CUDA(launch_pdl(permute_kernel<VT, R>, dim3((unsigned)pgrid), dim3(kPermThreads), 0, st, v, A, (unsigned)units));
     }
     if (phases & GT_FLAG_PHASE_TILE) {
-        const size_t smem = mass_smem<VT, R>(v);
-        if (smem > 227 * 1024) {
-            set_error("tile plan needs %zu bytes of shared memory per CTA (limit 232448): use a smaller tile", smem);
-            return GT_ERR_LIMIT;
-        }
+        const size_t smem = mass_smem<VT, R>(v);  // checked against kMaxMassSmem by reduce_typed
         GT_CUDA(allow_smem(mass_kernel<VT, R>, smem));
         // persistent grid: one CTA per resident slot; CTA b takes the (row group, tile) pairs b, b + grid, ...
         const int64_t pairs = (int64_t)v.NT * RG;
@@ -736,6 +733,17 @@ static int reduce_typed(const PlanView& v, const void* ws, int in_type, int64_t 
             if (out) GT_CUDA(cudaMemset2DAsync(out, (size_t)ld_out * sizeof(VT), 0, (size_t)v.N * sizeof(VT), (size_t)n_rows, st));
         return GT_OK;
     }
+    const unsigned phases = (flags & GT_FLAG_PHASE_MASK) ? (flags & GT_FLAG_PHASE_MASK) : GT_FLAG_PHASE_MASK;
+    // a plan whose tile node table does not fit is refused before anything is enqueued (the permute of the first chunk
+    // would already write the caller's workspace)
+    if (phases & GT_FLAG_PHASE_TILE) {
+        const size_t smem = mass_smem<VT, R>(v);
+        if (smem > kMaxMassSmem) {
+            set_error("tile plan needs %zu bytes of shared memory per CTA (limit %zu): %s", smem, kMaxMassSmem,
+                      v.T > 1024 ? "plan with 1024-leaf tiles" : "1024 leaves is already the smallest tile");
+            return GT_ERR_LIMIT;
+        }
+    }
     // rows per launch: what the caller's scratch can stage (a partial row group is legal: the kernels alias the missing
     // rows to the last valid one)
     const Scratch<VT, R> sc(v, workspace, workspace_bytes);
@@ -743,7 +751,6 @@ static int reduce_typed(const PlanView& v, const void* ws, int in_type, int64_t 
         set_error("workspace too small: %zu bytes given, one row needs %zu", workspace_bytes, Scratch<VT, R>::total(v, 1, 1));
         return GT_ERR_STATE;
     }
-    const unsigned phases = (flags & GT_FLAG_PHASE_MASK) ? (flags & GT_FLAG_PHASE_MASK) : GT_FLAG_PHASE_MASK;
     const int64_t chunk_rows = sc.chunk_rows;
     for (int64_t s0 = 0; s0 < n_rows; s0 += sc.span_rows) {  // span groups
         const int64_t s1 = std::min<int64_t>(n_rows, s0 + sc.span_rows);
