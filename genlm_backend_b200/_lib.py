@@ -21,6 +21,7 @@ GT_CHILD_NORMALIZE, GT_CHILD_LOG = 0x10, 0x20
 GT_MASK_NONE, GT_MASK_ADD_F32, GT_MASK_BOOL_U8, GT_MASK_BITS_U32 = 0, 1, 2, 3
 GT_RESAMPLE_MULTINOMIAL, GT_RESAMPLE_STRATIFIED, GT_RESAMPLE_SYSTEMATIC = 0, 1, 2
 GT_RESAMPLE_MAX_GROUP = 16384
+GT_PDA_POP, GT_PDA_MAX_DEPTH = -2, 64
 
 
 class PlanInfo(ctypes.Structure):
@@ -84,6 +85,10 @@ SIGNATURES = {
                                   c_int64, c_void_p]),
     "gt_dfa_advance": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,
                                c_void_p]),
+    "gt_pda_token_mask": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                  c_int64, c_void_p, c_int64, c_void_p]),
+    "gt_pda_advance": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                               c_void_p, c_int64, c_void_p, c_void_p]),
     "gt_lse_sample": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_float,
                               c_uint64, c_uint64, c_void_p, c_void_p, c_void_p]),
     "gt_resample": (c_int, [c_void_p, c_int64, c_int64, c_int, c_float, c_uint64, c_uint64, c_void_p, c_void_p, c_void_p,

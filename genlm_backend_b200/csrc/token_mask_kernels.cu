@@ -1,6 +1,7 @@
 // sm_100a kernels for per-row token masks over the trie: the items under a node (gt_subtree_token_mask), the items a
 // byte DFA accepts from there (gt_dfa_token_mask), their log-weights under a weighted byte DFA (gt_dfa_token_logw), and
-// the DFA state after a drawn token (gt_dfa_advance).
+// the DFA state after a drawn token (gt_dfa_advance); the items a byte pushdown automaton accepts from a row's
+// configuration at the root (gt_pda_token_mask), and the configuration after a drawn token (gt_pda_advance).
 #include <climits>
 #include <algorithm>
 #include <type_traits>
@@ -163,6 +164,133 @@ __global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanVie
     out[b] = res;
 }
 
+// ---- token masks under a byte-level pushdown automaton, and the PDA advance (gt_pda_token_mask / gt_pda_advance) -------
+//
+// Row b stands at the root in configuration (states[b], stack[b, 0 .. depth[b]-1]).  A walk over an item's symbols pushes
+// onto a private overlay and pops from it first; only once the overlay is empty does a pop read the row's stack, below a
+// read cursor that starts at depth[b].  The walk therefore never writes the row's stack, and the configuration after
+// the item is row stack[0 .. cursor) followed by the overlay.  A push past stack_ld rejects, so the overlay never holds
+// more than stack_ld - depth[b] <= GT_PDA_MAX_DEPTH entries, whatever the item's length.
+constexpr int kPdaMaxDepth = GT_PDA_MAX_DEPTH;
+
+struct PdaArgs {
+    DfaArgs A;  // delta, Q, ld, states, n_rows (nodes is null: every row at the root)
+    const int32_t* push;  // push[q * ld + s], read where delta[q, s] is a move
+    int cap;  // stack_ld: the row stride of the stacks and every row's capacity
+};
+
+// A row is valid iff its state lies in [0, Q) and its depth in [0, cap].
+__device__ __forceinline__ bool pda_row_valid(const PdaArgs& A, int q, int d) {
+    return q >= 0 && q < A.A.Q && d >= 0 && d <= A.cap;
+}
+
+// One symbol of a walk from q: a move (with an optional push onto the overlay ov[0 .. n)) or a pop (from the overlay,
+// else from row_stack below the cursor rd).  Returns the next state, or -1 on any reject.
+__device__ __forceinline__ int pda_step(const PdaArgs& A, int q, int s, int* ov, int& n, const int32_t* row_stack, int& rd) {
+    const int nq = dfa_step(A.A, q, s);
+    if (nq >= 0) {
+        const int pu = __ldg(A.push + q * A.A.ld + s);
+        if (pu < 0) return nq;
+        if (pu >= A.A.Q || rd + n >= A.cap) return -1;
+        ov[n++] = pu;
+        return nq;
+    }
+    if (__ldg(A.A.delta + q * A.A.ld + s) != GT_PDA_POP) return -1;
+    const int v = n > 0 ? ov[--n] : rd > 0 ? row_stack[--rd] : -1;
+    return (unsigned)v < (unsigned)A.A.Q ? v : -1;
+}
+
+// One thread per item, kPdaRows rows per CTA, so that a warp's ballot is one mask word as in dfa_mask_kernel.  As there,
+// the loop runs over the item's symbols outside and the rows inside, which gives each thread kPdaRows independent chains
+// of dependent table loads; each row has its own overlay of GT_PDA_MAX_DEPTH words in local memory (L1-resident, touched
+// only by pushes and pops).  The rows' stacks are staged in shared memory, where every item of the CTA reads them.
+// Rows per CTA, measured on B200 (DESIGN section 5.14): at 128k tokens 4 interleaved rows take 1-18 % less time than 8
+// and 3-17 % less than 2; walking 8 rows one after another with a single overlay took 10-19 % more.
+#ifndef GT_PDA_ROWS
+#define GT_PDA_ROWS 4
+#endif
+constexpr int kPdaThreads = 256, kPdaRows = GT_PDA_ROWS;
+
+__global__ void __launch_bounds__(kPdaThreads) pda_mask_kernel(PlanView P, PdaArgs A, const int32_t* __restrict__ stack,
+                                                               const int32_t* __restrict__ depth, uint32_t* __restrict__ out,
+                                                               int64_t ld_out, int64_t words) {
+    __shared__ int s_q[kPdaRows], s_d[kPdaRows];
+    __shared__ int32_t s_stack[kPdaRows][kPdaMaxDepth];
+    const int b0 = blockIdx.y * kPdaRows;
+    const int rows = min(kPdaRows, A.A.n_rows - b0);
+    if (threadIdx.x < kPdaRows) {
+        int q = -1, d = 0;
+        if (threadIdx.x < rows) { q = __ldg(A.A.states + b0 + threadIdx.x); d = __ldg(depth + b0 + threadIdx.x); }
+        if (!pda_row_valid(A, q, d)) { q = -1; d = 0; }
+        s_q[threadIdx.x] = q; s_d[threadIdx.x] = d;
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < kPdaRows * kPdaMaxDepth; e += kPdaThreads) {
+        const int g = e / kPdaMaxDepth, k = e % kPdaMaxDepth;
+        if (k < s_d[g]) s_stack[g][k] = __ldg(stack + (size_t)(b0 + g) * A.cap + k);
+    }
+    const int64_t i = (int64_t)blockIdx.x * kPdaThreads + threadIdx.x;
+    int p0 = 0, L = 0;
+    if (i < P.V) {
+        p0 = __ldg(P.item_sym_ptr + i);
+        L = __ldg(P.item_sym_ptr + i + 1) - p0;
+    }
+    __syncthreads();
+    int st[kPdaRows], n[kPdaRows], rd[kPdaRows];
+    int ov[kPdaRows][kPdaMaxDepth];
+#pragma unroll
+    for (int g = 0; g < kPdaRows; ++g) {
+        st[g] = i < P.V ? s_q[g] : -1;
+        n[g] = 0;
+        rd[g] = s_d[g];
+    }
+    const int32_t* sy = P.item_sym + p0;
+    for (int k = 0; k < L; ++k) {
+        const int s = __ldg(sy + k);
+        bool any = false;
+#pragma unroll
+        for (int g = 0; g < kPdaRows; ++g) {
+            if (st[g] >= 0) st[g] = pda_step(A, st[g], s, ov[g], n[g], s_stack[g], rd[g]);
+            any |= st[g] >= 0;
+        }
+        if (!any) break;
+    }
+    const int64_t w = i >> 5;
+#pragma unroll
+    for (int g = 0; g < kPdaRows; ++g) {
+        if (g >= rows) break;
+        const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
+        if ((threadIdx.x & 31) == 0 && w < words) out[(size_t)(b0 + g) * ld_out + w] = word;
+    }
+}
+
+// One thread per row walks the drawn item from the row's configuration, then writes the overlay over the row's stack
+// above the read cursor.  Nothing is written on a reject, so a rejected row keeps its stack and depth.  states and depth
+// are read with plain loads: out may alias states, and depth is written in place.
+constexpr int kPdaAdvanceThreads = 128;
+__global__ void __launch_bounds__(kPdaAdvanceThreads) pda_advance_kernel(PlanView P, PdaArgs A, int32_t* __restrict__ stack,
+                                                                         int32_t* __restrict__ depth,
+                                                                         const int32_t* __restrict__ tokens,
+                                                                         int32_t* out) {
+    const int b = blockIdx.x * kPdaAdvanceThreads + threadIdx.x;
+    if (b >= A.A.n_rows) return;
+    const int t = __ldg(tokens + b);
+    int q = A.A.states[b], res = -1;
+    const int d = depth[b];
+    if (t >= 0 && t < P.V && pda_row_valid(A, q, d)) {
+        int32_t* row_stack = stack + (size_t)b * A.cap;
+        int ov[kPdaMaxDepth], n = 0, rd = d;
+        const int p1 = __ldg(P.item_sym_ptr + t + 1);
+        for (int p = __ldg(P.item_sym_ptr + t); p < p1 && q >= 0; ++p) q = pda_step(A, q, __ldg(P.item_sym + p), ov, n, row_stack, rd);
+        if (q >= 0) {
+            for (int k = 0; k < n; ++k) row_stack[rd + k] = ov[k];
+            depth[b] = rd + n;
+        }
+        res = q;
+    }
+    out[b] = res;
+}
+
 }  // namespace gt
 
 extern "C" {
@@ -257,6 +385,59 @@ int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int
     if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     const unsigned grid = (unsigned)((n_rows + gt::kDfaAdvanceThreads - 1) / gt::kDfaAdvanceThreads);
     gt::dfa_advance_kernel<<<grid, gt::kDfaAdvanceThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, tokens, states_out);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
+}
+
+// Checks shared by the two PDA entry points after their null-pointer checks: dfa_args, then the stack capacity.
+static int pda_args(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
+                    const int32_t* states, int64_t stack_ld, int64_t n_rows, const char* what, gt::PdaArgs& A) {
+    if (const int rc = dfa_args(t, delta, n_states, ld_delta, states, nullptr, n_rows, what, A.A); rc != GT_OK) return rc;
+    if (stack_ld < 1) { gt::set_error("%s: stack_ld %lld < 1", what, (long long)stack_ld); return GT_ERR_ARG; }
+    if (stack_ld > GT_PDA_MAX_DEPTH) {
+        gt::set_error("%s: stack_ld %lld > GT_PDA_MAX_DEPTH = %d", what, (long long)stack_ld, GT_PDA_MAX_DEPTH);
+        return GT_ERR_LIMIT;
+    }
+    A.push = push; A.cap = (int)stack_ld;
+    return GT_OK;
+}
+
+int gt_pda_token_mask(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
+                      const int32_t* states, const int32_t* stack, int64_t stack_ld, const int32_t* depth, int64_t n_rows,
+                      uint32_t* mask_bits, int64_t mask_ld, gt_stream stream) {
+    if (!t) { gt::set_error("gt_pda_token_mask: null trie"); return GT_ERR_ARG; }
+    if (!delta || !push || !states || !stack || !depth || !mask_bits) { gt::set_error("gt_pda_token_mask: null data pointer"); return GT_ERR_ARG; }
+    const int64_t words = (t->layout.V + 31) / 32;
+    if (mask_ld < words) { gt::set_error("gt_pda_token_mask: mask_ld %lld < %lld words", (long long)mask_ld, (long long)words); return GT_ERR_ARG; }
+    gt::PdaArgs A{};
+    const int rc = pda_args(t, delta, push, n_states, ld_delta, states, stack_ld, n_rows, "gt_pda_token_mask", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0 || words == 0) return GT_OK;
+    if (n_rows > (int64_t)65535 * gt::kPdaRows) { gt::set_error("gt_pda_token_mask: too many rows"); return GT_ERR_LIMIT; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
+    dim3 grid((unsigned)((words * 32 + gt::kPdaThreads - 1) / gt::kPdaThreads), (unsigned)((n_rows + gt::kPdaRows - 1) / gt::kPdaRows));
+    gt::NvtxRange nv("gt:pda_mask");
+    gt::pda_mask_kernel<<<grid, gt::kPdaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, stack, depth, mask_bits, mask_ld, words);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
+}
+
+int gt_pda_advance(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
+                   const int32_t* states, int32_t* stack, int64_t stack_ld, int32_t* depth, const int32_t* tokens,
+                   int64_t n_rows, int32_t* states_out, gt_stream stream) {
+    if (!t) { gt::set_error("gt_pda_advance: null trie"); return GT_ERR_ARG; }
+    if (!delta || !push || !states || !stack || !depth || !tokens || !states_out) { gt::set_error("gt_pda_advance: null data pointer"); return GT_ERR_ARG; }
+    gt::PdaArgs A{};
+    const int rc = pda_args(t, delta, push, n_states, ld_delta, states, stack_ld, n_rows, "gt_pda_advance", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0) return GT_OK;
+    if (n_rows > INT32_MAX) { gt::set_error("gt_pda_advance: too many rows"); return GT_ERR_LIMIT; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
+    const unsigned grid = (unsigned)((n_rows + gt::kPdaAdvanceThreads - 1) / gt::kPdaAdvanceThreads);
+    gt::NvtxRange nv("gt:pda_advance");
+    gt::pda_advance_kernel<<<grid, gt::kPdaAdvanceThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, stack, depth, tokens, states_out);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }

@@ -366,6 +366,54 @@ class TrieEngine:
                          out.data_ptr())
         return out
 
+    # ---- token masks under a byte pushdown automaton, and the PDA advance ------------------------------------------
+    def _pda_inputs(self, delta, push, states, stack, depth, tokens=None):
+        """``_dfa_inputs`` plus ``push`` (an int32 table of ``delta``'s shape) and the rows' stacks, which must already be
+        int32 CUDA tensors on the rows' device: ``stack`` ``[B, stack_ld]`` with contiguous rows and ``depth`` ``[B]``,
+        since the advance updates them in place and a converted copy would lose the update."""
+        delta, states, _, tokens, device = self._dfa_inputs(delta, states, None, tokens)
+        push = torch.as_tensor(push)
+        if push.shape != delta.shape or push.is_floating_point() or push.is_complex():
+            raise ValueError(f"push must be an integer table of delta's shape {tuple(delta.shape)}, got {push.dtype} "
+                             f"{tuple(push.shape)}")
+        push = push.to(device=device, dtype=torch.int32).contiguous()
+        B = states.shape[0]
+        for x, what, dim in ((stack, "stack", 2), (depth, "depth", 1)):
+            if not (isinstance(x, torch.Tensor) and x.dtype == torch.int32 and x.device == device and x.dim() == dim
+                    and x.shape[0] == B):
+                raise ValueError(f"{what} must be an int32 tensor on {device} of {dim} dimensions with one row per state "
+                                 f"({B})")
+        if not (1 <= stack.shape[1] <= _lib.GT_PDA_MAX_DEPTH):
+            raise ValueError(f"stack must be [B, stack_ld] with 1 <= stack_ld <= {_lib.GT_PDA_MAX_DEPTH}, got "
+                             f"{tuple(stack.shape)}")
+        if not stack.is_contiguous() or not depth.is_contiguous():
+            raise ValueError("stack and depth must be contiguous: [B, stack_ld] rows of stack_ld entries and [B]")
+        return delta, push, states, tokens, device
+
+    def pda_token_mask(self, delta, push, states, stack, depth):
+        """``gt_pda_token_mask`` on the current stream of the inputs' device: keep-bitmask ``int32[B, ceil(V/32)]`` of the
+        items the PDA (``delta``, ``push``) accepts from each row's configuration at the root."""
+        delta, push, states, _, device = self._pda_inputs(delta, push, states, stack, depth)
+        B, W = states.shape[0], (self.V + 31) // 32
+        bits = torch.empty((B, W), dtype=torch.int32, device=device)
+        if B and W:
+            self._launch("gt_pda_token_mask", device.index, self._handle, delta.data_ptr(), push.data_ptr(), delta.shape[0],
+                         delta.shape[1], states.data_ptr(), stack.data_ptr(), stack.shape[1], depth.data_ptr(), B,
+                         bits.data_ptr(), W)
+        return bits
+
+    def pda_advance(self, delta, push, states, stack, depth, tokens):
+        """``gt_pda_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after item
+        ``tokens[b]``, or -1; ``stack`` and ``depth`` are updated in place where the result is not -1."""
+        delta, push, states, tokens, device = self._pda_inputs(delta, push, states, stack, depth, tokens)
+        B = states.shape[0]
+        out = torch.empty(B, dtype=torch.int32, device=device)
+        if B:
+            self._launch("gt_pda_advance", device.index, self._handle, delta.data_ptr(), push.data_ptr(), delta.shape[0],
+                         delta.shape[1], states.data_ptr(), stack.data_ptr(), stack.shape[1], depth.data_ptr(),
+                         tokens.data_ptr(), B, out.data_ptr())
+        return out
+
     # ---- child masses of one node per row, straight from the rows -----------------------------------------------
     def _child_inputs(self, ws, nodes):
         """Checks shared by the child read-outs (those of ``reduce``, plus one node id per row)."""

@@ -238,6 +238,28 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         (-1).  Keeps ``mask -> masked_logsumexp_sample -> advance`` on the device."""
         return self._engine.dfa_advance(delta, states, tokens, nodes)
 
+    # ---- token masks under a byte-level pushdown automaton (nested constraints such as JSON) ------------------------
+    def pda_token_mask(self, delta, push, states, stack, depth):
+        """Keep-bitmask ``int32[B, ceil(V/32)]`` of the tokens each particle may emit next under a deterministic
+        byte-level pushdown automaton, in the bit-mask layout of ``smc.masked_logsumexp_sample``.
+
+        ``delta`` and ``push`` are int32 ``[Q, ld >= S]`` tables in the format of ``genlm_backend_b200.pda`` (a move,
+        optionally pushing a return state; ``GT_PDA_POP`` = -2 to return to the popped state; anything else rejects).
+        Row ``b`` stands at the root in state ``states[b]`` with the stack ``stack[b, :depth[b]]`` (bottom first);
+        ``stack`` is an int32 CUDA ``[B, stack_ld]`` tensor with contiguous rows (``stack_ld <= 64`` is every row's
+        capacity) and ``depth`` an int32 CUDA ``[B]`` tensor.  A token is allowed iff the walk over its symbols never
+        rejects; an invalid state or depth gives an all-zero row.  Runs on the current stream of the inputs' device; no
+        sync."""
+        return self._engine.pda_token_mask(delta, push, states, stack, depth)
+
+    def pda_advance(self, delta, push, states, stack, depth, tokens):
+        """``int32[B]``: row ``b``'s state after token ``tokens[b]``, or -1 for a token that ``pda_token_mask`` does not
+        allow -- also the sampler's "no draw" (-1).  Where the result is not -1, ``stack`` and ``depth`` are advanced in
+        place (entries at or above the new depth are unspecified); elsewhere the row's stack and depth are unchanged.
+        ``stack`` and ``depth`` must be int32 CUDA tensors as in ``pda_token_mask``: anything else raises ``ValueError``,
+        since a converted copy would lose the update.  The result may be written back into ``states``."""
+        return self._engine.pda_advance(delta, push, states, stack, depth, tokens)
+
     # ---- child masses of one node per row (the next-symbol distribution of a character-level sampler) ------------
     @property
     def max_children(self):

@@ -36,6 +36,9 @@
  *   gt_dfa_token_logw           the same walk through a weighted automaton, summing each token's transition
  *                               log-weights: the additive mask of a soft byte-level potential
  *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
+ *   gt_pda_token_mask           the host-side walk of every token's bytes through a parser (a pushdown automaton
+ *                               with a stack per particle) for a nested constraint such as JSON
+ *   gt_pda_advance              the host-side tracking of each particle's parser state and stack over the drawn token
  *   gt_resample                 the effective sample size of each particle group and, below a threshold, the
  *                               multinomial, stratified or systematic ancestors an SMC driver draws on the host
  *
@@ -388,6 +391,47 @@ int gt_dfa_token_logw(const gt_trie* t, const int32_t* delta, const float* logw,
 int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int64_t ld_delta,
                    const int32_t* states, const int32_t* nodes /* NULL = root */, const int32_t* tokens,
                    int64_t n_rows, int32_t* states_out, gt_stream stream);
+
+/* ---- token masks under a byte-level pushdown automaton, and the PDA advance over drawn tokens ---------------------- */
+
+#define GT_PDA_POP (-2)
+#define GT_PDA_MAX_DEPTH 64
+
+/* A deterministic byte-level pushdown automaton in return-state form (a push saves the state to return to, a pop goes
+ * there), as a grammar compiles into a recursive transition network.  delta and push: device int32 [n_states][ld_delta],
+ * ld_delta >= S (gt_num_symbols), the same shape and row stride.  From state q on symbol s:
+ *   - delta[q, s] in [0, n_states): if push[q, s] >= 0, push it (push[q, s] >= n_states, or a stack already holding
+ *     stack_ld entries, rejects), then go to delta[q, s];
+ *   - delta[q, s] == GT_PDA_POP: pop the top of the stack and go to the popped state (an empty stack, or a popped value
+ *     outside [0, n_states), rejects);
+ *   - any other value rejects.  push[q, s] is read only for a move.
+ * Row b's configuration is its state states[b], its depth depth[b] and its stack stack[b * stack_ld + 0 .. depth[b]-1],
+ * bottom first; stack_ld is both the row stride and every row's capacity, 1 <= stack_ld <= GT_PDA_MAX_DEPTH.  A state
+ * outside [0, n_states) or a depth outside [0, stack_ld] makes the row invalid.  Rows stand at the root: item i is
+ * allowed iff the row is valid and the walk over all of item i's symbols never rejects (an item with no symbols: iff the
+ * row is valid).  End of sequence needs no special case: the EOS item's symbol column decides it.  A table with push
+ * -1 everywhere and no GT_PDA_POP entry is a DFA: both calls then give what gt_dfa_token_mask and gt_dfa_advance give at
+ * the root, and leave stack and depth untouched.
+ * Argument checks, in order: null t or data pointers, mask_ld < ceil(V/32) (GT_ERR_ARG); n_states, ld_delta and n_rows as
+ * for the DFA calls (a table of 2^31 entries or more: GT_ERR_LIMIT); stack_ld < 1 (GT_ERR_ARG) or > GT_PDA_MAX_DEPTH
+ * (GT_ERR_LIMIT); no rows returns GT_OK; more rows than the grid takes: GT_ERR_LIMIT.  No allocation, no
+ * synchronisation, launches on `stream`, graph-capturable. */
+
+/* keep-bitmask of the items allowed under the PDA from each row's configuration, in gt_dfa_token_mask's layout: every word
+ * of the first ceil(V/32) words of each row is written (bits >= V of the last word are 0), words beyond them are not
+ * touched.  An invalid row gives an all-zero row.  stack and depth are only read. */
+int gt_pda_token_mask(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
+                      const int32_t* states, const int32_t* stack, int64_t stack_ld, const int32_t* depth,
+                      int64_t n_rows, uint32_t* mask_bits, int64_t mask_ld, gt_stream stream);
+
+/* states_out[b] = the state after all of item tokens[b]'s symbols from row b's configuration, or -1 for a token < 0 or
+ * >= V (the sampler's "no draw"), an invalid row or any reject on the way; states_out[b] >= 0 exactly where
+ * gt_pda_token_mask sets the token's bit.  Where states_out[b] >= 0, stack and depth[b] hold the new configuration, in
+ * place (entries at or above the new depth are unspecified); elsewhere the row's stack and depth[b] are unchanged.
+ * states_out may equal states. */
+int gt_pda_advance(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
+                   const int32_t* states, int32_t* stack, int64_t stack_ld, int32_t* depth,
+                   const int32_t* tokens, int64_t n_rows, int32_t* states_out, gt_stream stream);
 
 /* ---- particle resampling: per-group effective sample size and ancestors ----------------------------------------- */
 
