@@ -87,6 +87,8 @@ SIGNATURES = {
                                c_void_p]),
     "gt_pda_token_mask": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
                                   c_int64, c_void_p, c_int64, c_void_p]),
+    "gt_pda_token_logw": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64,
+                                  c_void_p, c_int64, c_void_p, c_int64, c_void_p]),
     "gt_pda_advance": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
                                c_void_p, c_int64, c_void_p, c_void_p]),
     "gt_lse_sample": (c_int, [c_void_p, c_int, c_int64, c_int64, c_int64, c_void_p, c_int, c_int64, c_float,

@@ -1,7 +1,8 @@
 // sm_100a kernels for per-row token masks over the trie: the items under a node (gt_subtree_token_mask), the items a
 // byte DFA accepts from there (gt_dfa_token_mask), their log-weights under a weighted byte DFA (gt_dfa_token_logw), and
 // the DFA state after a drawn token (gt_dfa_advance); the items a byte pushdown automaton accepts from a row's
-// configuration at the root (gt_pda_token_mask), and the configuration after a drawn token (gt_pda_advance).
+// configuration at the root (gt_pda_token_mask), their log-weights under a weighted one (gt_pda_token_logw), and the
+// configuration after a drawn token (gt_pda_advance).
 #include <climits>
 #include <algorithm>
 #include <type_traits>
@@ -164,7 +165,7 @@ __global__ void __launch_bounds__(kDfaAdvanceThreads) dfa_advance_kernel(PlanVie
     out[b] = res;
 }
 
-// ---- token masks under a byte-level pushdown automaton, and the PDA advance (gt_pda_token_mask / gt_pda_advance) -------
+// ---- token masks under a byte-level pushdown automaton (gt_pda_token_mask / gt_pda_token_logw / gt_pda_advance) --------
 //
 // Row b stands at the root in configuration (states[b], stack[b, 0 .. depth[b]-1]).  A walk over an item's symbols pushes
 // onto a private overlay and pops from it first; only once the overlay is empty does a pop read the row's stack, below a
@@ -211,9 +212,17 @@ __device__ __forceinline__ int pda_step(const PdaArgs& A, int q, int s, int* ov,
 #endif
 constexpr int kPdaThreads = 256, kPdaRows = GT_PDA_ROWS;
 
+// kLogw = false (gt_pda_token_mask): out holds keep-bitmask words, ld_out words per row, words of them written.
+// kLogw = true (gt_pda_token_logw): out[b, i] is the fp64 sum of logw[q_k, s_k] over the walked transitions (moves,
+// pushes and pops alike), in increasing k and rounded once to fp32, where the bit would be set, else -inf; ld_out floats
+// per row, the first V written, words unused.  As in dfa_mask_kernel, logw is loaded at delta's index as an independent
+// load, and a -inf accumulator does not stop the walk.  logw is a trailing parameter, so the bits instantiation keeps
+// its parameter offsets.
+template <bool kLogw>
 __global__ void __launch_bounds__(kPdaThreads) pda_mask_kernel(PlanView P, PdaArgs A, const int32_t* __restrict__ stack,
-                                                               const int32_t* __restrict__ depth, uint32_t* __restrict__ out,
-                                                               int64_t ld_out, int64_t words) {
+                                                               const int32_t* __restrict__ depth,
+                                                               std::conditional_t<kLogw, float, uint32_t>* __restrict__ out,
+                                                               int64_t ld_out, int64_t words, const float* __restrict__ logw) {
     __shared__ int s_q[kPdaRows], s_d[kPdaRows];
     __shared__ int32_t s_stack[kPdaRows][kPdaMaxDepth];
     const int b0 = blockIdx.y * kPdaRows;
@@ -238,6 +247,7 @@ __global__ void __launch_bounds__(kPdaThreads) pda_mask_kernel(PlanView P, PdaAr
     __syncthreads();
     int st[kPdaRows], n[kPdaRows], rd[kPdaRows];
     int ov[kPdaRows][kPdaMaxDepth];
+    double acc[kPdaRows] = {};
 #pragma unroll
     for (int g = 0; g < kPdaRows; ++g) {
         st[g] = i < P.V ? s_q[g] : -1;
@@ -250,17 +260,29 @@ __global__ void __launch_bounds__(kPdaThreads) pda_mask_kernel(PlanView P, PdaAr
         bool any = false;
 #pragma unroll
         for (int g = 0; g < kPdaRows; ++g) {
-            if (st[g] >= 0) st[g] = pda_step(A, st[g], s, ov[g], n[g], s_stack[g], rd[g]);
+            if (st[g] >= 0) {
+                if constexpr (kLogw) acc[g] += (double)__ldg(logw + st[g] * A.A.ld + s);
+                st[g] = pda_step(A, st[g], s, ov[g], n[g], s_stack[g], rd[g]);
+            }
             any |= st[g] >= 0;
         }
         if (!any) break;
     }
-    const int64_t w = i >> 5;
+    if constexpr (kLogw) {
+        if (i >= P.V) return;
 #pragma unroll
-    for (int g = 0; g < kPdaRows; ++g) {
-        if (g >= rows) break;
-        const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
-        if ((threadIdx.x & 31) == 0 && w < words) out[(size_t)(b0 + g) * ld_out + w] = word;
+        for (int g = 0; g < kPdaRows; ++g) {  // consecutive threads store consecutive items: one coalesced store per warp
+            if (g >= rows) break;
+            out[(size_t)(b0 + g) * ld_out + i] = st[g] >= 0 ? (float)acc[g] : -INFINITY;
+        }
+    } else {
+        const int64_t w = i >> 5;
+#pragma unroll
+        for (int g = 0; g < kPdaRows; ++g) {
+            if (g >= rows) break;
+            const unsigned word = __ballot_sync(0xffffffffu, st[g] >= 0);
+            if ((threadIdx.x & 31) == 0 && w < words) out[(size_t)(b0 + g) * ld_out + w] = word;
+        }
     }
 }
 
@@ -389,7 +411,7 @@ int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int
     return GT_OK;
 }
 
-// Checks shared by the two PDA entry points after their null-pointer checks: dfa_args, then the stack capacity.
+// Checks shared by the three PDA entry points after their null-pointer checks: dfa_args, then the stack capacity.
 static int pda_args(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
                     const int32_t* states, int64_t stack_ld, int64_t n_rows, const char* what, gt::PdaArgs& A) {
     if (const int rc = dfa_args(t, delta, n_states, ld_delta, states, nullptr, n_rows, what, A.A); rc != GT_OK) return rc;
@@ -418,7 +440,30 @@ int gt_pda_token_mask(const gt_trie* t, const int32_t* delta, const int32_t* pus
     if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
     dim3 grid((unsigned)((words * 32 + gt::kPdaThreads - 1) / gt::kPdaThreads), (unsigned)((n_rows + gt::kPdaRows - 1) / gt::kPdaRows));
     gt::NvtxRange nv("gt:pda_mask");
-    gt::pda_mask_kernel<<<grid, gt::kPdaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, stack, depth, mask_bits, mask_ld, words);
+    gt::pda_mask_kernel<false><<<grid, gt::kPdaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, stack, depth, mask_bits, mask_ld,
+                                                                                               words, nullptr);
+    GT_CUDA(cudaGetLastError());
+    return GT_OK;
+}
+
+int gt_pda_token_logw(const gt_trie* t, const int32_t* delta, const int32_t* push, const float* logw, int64_t n_states,
+                      int64_t ld_delta, const int32_t* states, const int32_t* stack, int64_t stack_ld, const int32_t* depth,
+                      int64_t n_rows, float* out, int64_t ld_out, gt_stream stream) {
+    if (!t) { gt::set_error("gt_pda_token_logw: null trie"); return GT_ERR_ARG; }
+    if (!delta || !push || !logw || !states || !stack || !depth || !out) { gt::set_error("gt_pda_token_logw: null data pointer"); return GT_ERR_ARG; }
+    const int64_t V = t->layout.V;
+    if (ld_out < V) { gt::set_error("gt_pda_token_logw: ld_out %lld < V = %lld", (long long)ld_out, (long long)V); return GT_ERR_ARG; }
+    gt::PdaArgs A{};
+    const int rc = pda_args(t, delta, push, n_states, ld_delta, states, stack_ld, n_rows, "gt_pda_token_logw", A);
+    if (rc != GT_OK) return rc;
+    if (n_rows == 0 || V == 0) return GT_OK;
+    if (n_rows > (int64_t)65535 * gt::kPdaRows) { gt::set_error("gt_pda_token_logw: too many rows"); return GT_ERR_LIMIT; }
+    const gt::PlanView* v = nullptr;
+    if (const int rc = gt::resident_plan(t, v); rc != GT_OK) return rc;
+    // the same grid as gt_pda_token_mask's: ceil(ceil(V/32) * 32 / kPdaThreads) = ceil(V / kPdaThreads)
+    dim3 grid((unsigned)((V + gt::kPdaThreads - 1) / gt::kPdaThreads), (unsigned)((n_rows + gt::kPdaRows - 1) / gt::kPdaRows));
+    gt::NvtxRange nv("gt:pda_logw");
+    gt::pda_mask_kernel<true><<<grid, gt::kPdaThreads, 0, static_cast<cudaStream_t>(stream)>>>(*v, A, stack, depth, out, ld_out, 0, logw);
     GT_CUDA(cudaGetLastError());
     return GT_OK;
 }

@@ -39,6 +39,32 @@ Resampling reindexes every per-particle tensor, the stacks included::
     idx = anc.view(-1)
     q, stack, depth = q.index_select(0, idx), stack.index_select(0, idx), depth.index_select(0, idx)
 
+Weighted automata: a float table ``logw`` of ``delta``'s shape, ``logw[q, s]`` the log-weight of the transition from
+``q`` on ``s`` -- a plain move, a move with a push or a pop alike; the EOS column holds the final weights.  This carries a
+probabilistic grammar compiled into return-state form (rule probabilities on the transitions that choose a rule), a
+prior on the nesting depth (a weight on every push), or a preference per container kind (``json_pda`` copies scalar
+states per context, so a weight can depend on where a value sits).  A pop's weight is read at ``(q, s)`` and does not
+depend on the popped state: a weight that should depend on the state returned to belongs on the push that saved it.
+``pda_token_logw`` gives each token the fp64 sum, rounded once to float32, of the log-weights along its symbols where
+``pda_token_mask`` allows it, and ``-inf`` elsewhere; with ``logw`` all zero that is the ``{0, -inf}`` form of the
+mask.  It is the sampler's additive mask, whose ``logZ = log sum_i p_i w_i`` is the particle's weight increment.  For a
+prefix weight ``phi`` (a weighted grammar), the tables after weight pushing make the row ``log phi(x t) - log phi(x)``,
+the exact token-level factor; computing the pushed tables is the caller's job.
+
+Weighted token-level step (``pda_advance`` takes the same ``delta`` and ``push``)::
+
+    tokw = trie.pda_token_logw(delta, push, logw, q, stack, depth)
+    logZ, tok = smc.masked_logsumexp_sample(logps, tokw, seed=seed, offset=step * B)   # tok from p * w / Z
+    q = trie.pda_advance(delta, push, q, stack, depth, tok)
+    log_weights += logZ
+
+Exact weighted byte-level step: one ``tokw`` per token, at the root, and the next-symbol draws from ``logps + tokw``
+with ``log_input=True`` (a ``-inf`` is a zero weight, as under ``mask=``)::
+
+    tokw = trie.pda_token_logw(delta, push, logw, q, stack, depth)  # once per token, at the root
+    child, label, logp, logZ = trie.sample_next_symbol(logps + tokw, n, log_input=True, seed=s, offset=k)  # per byte
+    # the root's logZ is masked_logsumexp_sample(logps, tokw)'s; a drawn leaf ends token -1 - label, then pda_advance
+
 ``json_pda`` builds the automaton of RFC 8259 JSON text.
 """
 import numpy as np

@@ -337,15 +337,21 @@ class TrieEngine:
                          states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W)
         return bits
 
-    def dfa_token_logw(self, delta, logw, states, nodes=None):
-        """``gt_dfa_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
-        summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
-        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
+    @staticmethod
+    def _logw_input(logw, delta, device):
+        """A float table of ``delta``'s shape as a contiguous float32 tensor on ``device``: the transition log-weights
+        of the weighted DFA and PDA calls."""
         logw = torch.as_tensor(logw)
         if not logw.is_floating_point() or logw.shape != delta.shape:
             raise ValueError(f"logw must be a float table of delta's shape {tuple(delta.shape)}, got {logw.dtype} "
                              f"{tuple(logw.shape)}")
-        logw = logw.to(device=device, dtype=torch.float32).contiguous()
+        return logw.to(device=device, dtype=torch.float32).contiguous()
+
+    def dfa_token_logw(self, delta, logw, states, nodes=None):
+        """``gt_dfa_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
+        summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
+        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
+        logw = self._logw_input(logw, delta, device)
         B, V = states.shape[0], self.V
         out = torch.empty((B, V), dtype=torch.float32, device=device)
         if B and V:
@@ -401,6 +407,19 @@ class TrieEngine:
                          delta.shape[1], states.data_ptr(), stack.data_ptr(), stack.shape[1], depth.data_ptr(), B,
                          bits.data_ptr(), W)
         return bits
+
+    def pda_token_logw(self, delta, push, logw, states, stack, depth):
+        """``gt_pda_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
+        summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
+        delta, push, states, _, device = self._pda_inputs(delta, push, states, stack, depth)
+        logw = self._logw_input(logw, delta, device)
+        B, V = states.shape[0], self.V
+        out = torch.empty((B, V), dtype=torch.float32, device=device)
+        if B and V:
+            self._launch("gt_pda_token_logw", device.index, self._handle, delta.data_ptr(), push.data_ptr(),
+                         logw.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(), stack.data_ptr(),
+                         stack.shape[1], depth.data_ptr(), B, out.data_ptr(), V)
+        return out
 
     def pda_advance(self, delta, push, states, stack, depth, tokens):
         """``gt_pda_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after item

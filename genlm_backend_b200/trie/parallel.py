@@ -252,6 +252,20 @@ class ParallelTokenCharacterTrie(TokenCharacterTrie):
         sync."""
         return self._engine.pda_token_mask(delta, push, states, stack, depth)
 
+    def pda_token_logw(self, delta, push, logw, states, stack, depth):
+        """``float32[B, V]``: the log-weight of each token under a weighted byte-level pushdown automaton, the additive
+        mask of ``smc.masked_logsumexp_sample``.
+
+        ``delta``, ``push``, ``states``, ``stack`` and ``depth`` as in ``pda_token_mask``; ``logw`` is a float table of
+        ``delta``'s shape, ``logw[q, s]`` the log-weight of the transition from ``q`` on symbol ``s`` -- a move, a move
+        with a push or a pop alike (converted to float32 on the device).  A pop's weight does not depend on the popped
+        state: a weight that should belongs on the push that saved it.  A token that ``pda_token_mask`` allows gets the
+        fp64 sum, rounded once to float32, of the log-weights along its symbols (0 for an empty token); every other
+        token gets ``-inf``.  IEEE arithmetic decides special values (a ``-inf`` weight on the walk gives ``-inf``, a
+        NaN gives NaN).  With ``logw`` all zero the result is the ``{0, -inf}`` form of ``pda_token_mask``.  Runs on the
+        current stream of the inputs' device; no sync."""
+        return self._engine.pda_token_logw(delta, push, logw, states, stack, depth)
+
     def pda_advance(self, delta, push, states, stack, depth, tokens):
         """``int32[B]``: row ``b``'s state after token ``tokens[b]``, or -1 for a token that ``pda_token_mask`` does not
         allow -- also the sampler's "no draw" (-1).  Where the result is not -1, ``stack`` and ``depth`` are advanced in

@@ -38,7 +38,9 @@
  *   gt_dfa_advance              the host-side tracking of each particle's automaton state over the drawn token
  *   gt_pda_token_mask           the host-side walk of every token's bytes through a parser (a pushdown automaton
  *                               with a stack per particle) for a nested constraint such as JSON
- *   gt_pda_advance              the host-side tracking of each particle's parser state and stack over the drawn token
+ *   gt_pda_token_logw           the same walk through a weighted pushdown automaton (a probabilistic grammar, a
+ *                               nesting penalty), summing each token's transition log-weights: an additive mask
+ *   gt_pda_advance             the host-side tracking of each particle's parser state and stack over the drawn token
  *   gt_resample                 the effective sample size of each particle group and, below a threshold, the
  *                               multinomial, stratified or systematic ancestors an SMC driver draws on the host
  *
@@ -423,6 +425,29 @@ int gt_dfa_advance(const gt_trie* t, const int32_t* delta, int64_t n_states, int
 int gt_pda_token_mask(const gt_trie* t, const int32_t* delta, const int32_t* push, int64_t n_states, int64_t ld_delta,
                       const int32_t* states, const int32_t* stack, int64_t stack_ld, const int32_t* depth,
                       int64_t n_rows, uint32_t* mask_bits, int64_t mask_ld, gt_stream stream);
+
+/* Per-row token log-weights under a deterministic weighted pushdown automaton: delta, push and the rows as above, and
+ * logw: device fp32, the same shape and row stride, logw[q * ld_delta + s] the log-weight of the transition from q on
+ * symbol s, be it a move, a move with a push or a pop.  A pop's weight is read at (q, s) and does not depend on the
+ * popped state: a weight that should depend on the state returned to belongs on the push that saved it.  For row b,
+ * out[b * ld_out + i] is
+ *   - for an item gt_pda_token_mask allows: the sum of (double) logw[q_k, s_k] over all of item i's symbols, with q_k
+ *     the state before symbol s_k, added in increasing k in fp64 from 0.0 and rounded once to fp32 (0.0f for an item
+ *     with no symbols);
+ *   - -inf for every other item (an invalid row, any reject on the way: a push past stack_ld, a pop from an empty stack,
+ *     a popped value outside [0, n_states)), whatever the weights.
+ * IEEE arithmetic decides special values: a -inf transition weight makes the token -inf, a NaN weight on the walk or
+ * -inf followed by +inf gives NaN; the walk does not stop on a -inf sum, only on a reject.  With logw = 0 everywhere,
+ * out is the additive {0, -inf} form of gt_pda_token_mask's bits; on a table with no push and no pop and empty stacks,
+ * out is gt_dfa_token_logw's at the root.  End of sequence: the EOS column of logw holds the final weights.  The
+ * result is gt_lse_sample's GT_MASK_ADD_F32 mask (mask_ld = ld_out): its logZ is log sum_i p_i w_i, the particle's
+ * weight increment; gt_pda_advance takes the same delta and push.  Writes the first V floats of each row, nothing
+ * beyond them; ld_out >= V.  Argument checks, in order: null t; null delta / push / logw / states / stack / depth / out;
+ * ld_out < V (GT_ERR_ARG); the table, row and capacity checks of gt_pda_token_mask; no rows returns GT_OK; more rows than
+ * the grid takes: GT_ERR_LIMIT.  No allocation, no synchronisation, launches on `stream`, graph-capturable. */
+int gt_pda_token_logw(const gt_trie* t, const int32_t* delta, const int32_t* push, const float* logw, int64_t n_states,
+                      int64_t ld_delta, const int32_t* states, const int32_t* stack, int64_t stack_ld,
+                      const int32_t* depth, int64_t n_rows, float* out, int64_t ld_out, gt_stream stream);
 
 /* states_out[b] = the state after all of item tokens[b]'s symbols from row b's configuration, or -1 for a token < 0 or
  * >= V (the sampler's "no draw"), an invalid row or any reject on the way; states_out[b] >= 0 exactly where

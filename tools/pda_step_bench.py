@@ -18,6 +18,17 @@ it times with CUDA events over a CUDA graph of K steps:
 
 (the DFA routes do not depend on the mix; they are timed again beside each mix).
 
+``--weighted`` adds the same step under weighted automata: ``json_pda`` and the DFA get seeded log-weights (normal,
+scale 0.5) on every transition, and four routes are timed on the same rows:
+
+  pda_logw        ``pda_token_logw`` under the weighted ``json_pda``                      gt_pda_token_logw
+  pda_wstep       pda_logw -> ``masked_logsumexp_sample(logps, tokw)`` -> ``pda_advance``
+  dfa_logw        ``dfa_token_logw`` under the weighted DFA                               gt_dfa_token_logw
+  pdadfa_logw     ``pda_token_logw`` on that DFA with ``push`` all -1 and empty stacks (the same log-weights)
+
+with ``vs_boolean``, a route's time over its Boolean counterpart's on the same rows (pda_mask, pda_step, dfa_mask,
+pdadfa_mask).  pdadfa_logw is checked bit-equal to dfa_logw before timing.  Without the flag the lines are unchanged.
+
 The advance updates stacks and depths in place, so each PDA step first copies the rows' stacks and depths to scratch
 tensors (two copies) and advances those: every replay starts from the same configurations.  The DFA step has no such
 copies.  ``vs_dfa`` is a route's time over the matching DFA route's.  Step k reads buffer set k % sets of log-softmax
@@ -68,6 +79,7 @@ def main():
     ap.add_argument("--vocabs", default="synth128256,json")
     ap.add_argument("--steps", type=int, default=20, help="K: steps per CUDA graph")
     ap.add_argument("--reps", type=int, default=10, help="graph replays timed (median reported)")
+    ap.add_argument("--weighted", action="store_true", help="also the routes under weighted automata")
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     assert torch.cuda.is_available(), "pda_step_bench.py measures on a GPU"
@@ -85,6 +97,8 @@ def main():
         dd = random_dfa(Q, S, seed=3)
         jd_c, jp_c, dd_c = (torch.tensor(x).cuda() for x in (jd, jp, dd))
         nopush = torch.full_like(dd_c, -1)
+        wrng = np.random.default_rng(5)
+        jw_c, dw_c = (torch.tensor((wrng.normal(size=x.shape) * 0.5).astype(np.float32)).cuda() for x in (jd, dd))
         for B in [int(x) for x in args.batches.split(",")]:
             sets = min(64, max(2, -(-3 * L2_BYTES // (4 * B * V))))
             logps = [torch.tensor(logsoftmax_rows(B, V, seed=s)).cuda() for s in range(sets)]
@@ -103,6 +117,13 @@ def main():
                     scratch_depth.copy_(n)
                     return bits, tok, trie.pda_advance(d, p, q, scratch_stack, scratch_depth, tok)
 
+                def pda_wstep(lp, q, s, n):
+                    tokw = trie.pda_token_logw(jd_c, jp_c, jw_c, q, s, n)
+                    _, tok = smc.masked_logsumexp_sample(lp, tokw, seed=1)
+                    scratch_stack.copy_(s)
+                    scratch_depth.copy_(n)
+                    return tokw, tok, trie.pda_advance(jd_c, jp_c, q, scratch_stack, scratch_depth, tok)
+
                 def dfa_step(lp, q):
                     bits = trie.dfa_token_mask(dd_c, q)
                     _, tok = smc.masked_logsumexp_sample(lp, bits, seed=1)
@@ -116,6 +137,20 @@ def main():
                     "pdadfa_mask": (lambda lp, q: trie.pda_token_mask(dd_c, nopush, q, zero_stack, zero_depth), "dfa_mask"),
                     "pdadfa_step": (lambda lp, q: pda_step(dd_c, nopush, lp, q, zero_stack, zero_depth), "dfa_step"),
                 }
+                boolean = {}
+                if args.weighted:
+                    routes.update({
+                        "pda_logw": (lambda lp, q: trie.pda_token_logw(jd_c, jp_c, jw_c, st, stk, dep), "dfa_logw"),
+                        "pda_wstep": (lambda lp, q: pda_wstep(lp, st, stk, dep), None),
+                        "dfa_logw": (lambda lp, q: trie.dfa_token_logw(dd_c, dw_c, q), None),
+                        "pdadfa_logw": (lambda lp, q: trie.pda_token_logw(dd_c, nopush, dw_c, q, zero_stack, zero_depth),
+                                        "dfa_logw"),
+                    })
+                    boolean = {"pda_logw": "pda_mask", "pda_wstep": "pda_step", "dfa_logw": "dfa_mask",
+                               "pdadfa_logw": "pdadfa_mask"}
+                    for s in range(2):  # the PDA log-weights on the push-free table are the DFA's
+                        assert torch.equal(routes["pdadfa_logw"][0](logps[s], dfa_states[s]).view(torch.int32),
+                                           routes["dfa_logw"][0](logps[s], dfa_states[s]).view(torch.int32)), (vname, B)
                 for s in range(2):  # the PDA calls on the push-free table give the DFA calls' results
                     for have, want in zip(routes["pdadfa_step"][0](logps[s], dfa_states[s]), dfa_step(logps[s], dfa_states[s])):
                         assert torch.equal(have, want), (vname, B)
@@ -134,6 +169,8 @@ def main():
                         "Lmax": int(max(len(getattr(t, "byte_string", b"")) for t in dec)),
                         "buffer_sets": sets, "steps_per_graph": args.steps, "gpu": gpu, "power_limit": power,
                     }
+                    if args.weighted:
+                        line["vs_boolean"] = round(med / res[boolean[r]][0], 3) if r in boolean else None
                     lines.append(line)
                     print(json.dumps(line), flush=True)
             del logps
