@@ -302,10 +302,17 @@ class TrieEngine:
             self._launch("gt_subtree_token_mask", device.index, self._handle, nodes.data_ptr(), B, bits.data_ptr(), W)
         return bits
 
-    # ---- token masks under a byte DFA, and the DFA advance -------------------------------------------------------
-    def _dfa_inputs(self, delta, states, nodes, tokens=None):
-        """``(delta, states, nodes | None, tokens | None, device)`` as contiguous int32 tensors on one CUDA device: that of
-        ``states`` when it is a CUDA tensor, else that of ``delta``, else the current device."""
+    # ---- token masks under a byte DFA or pushdown automaton, and the advance ------------------------------------
+    def _automaton_args(self, delta, states, nodes=None, tokens=None, logw=None, pda=None):
+        """The leading arguments of an automaton entry point, the trie handle to ``n_rows``, as ``(args, B, device,
+        keep)``; ``keep`` holds the converted tensors until the launch.  The device is that of ``states`` when it is a
+        CUDA tensor, else that of ``delta``, else the current device.  ``delta`` and ``states``, and ``nodes`` and
+        ``tokens`` where given (one entry per row), become contiguous int32 tensors on it.  ``pda = (push, stack,
+        depth)`` makes it a PDA call: ``push`` is an integer table of ``delta``'s shape, converted the same way, and the
+        rows' stacks must already be int32 tensors on the device, ``stack`` ``[B, stack_ld]`` with contiguous rows and
+        ``depth`` ``[B]``, since the advance updates them in place and a converted copy would lose the update.
+        ``logw``, the transition log-weights of the weighted calls, is a float table of ``delta``'s shape, converted to
+        contiguous float32."""
         require_cuda()
         delta, states = torch.as_tensor(delta), torch.as_tensor(states)
         device = states.device if states.is_cuda else delta.device if delta.is_cuda else torch.device("cuda", torch.cuda.current_device())
@@ -324,113 +331,96 @@ class TrieEngine:
         nodes = None if nodes is None else per_row(nodes, "nodes")
         tokens = None if tokens is None else per_row(tokens, "tokens")
         self.ensure_device(device.index)
-        return delta, states, nodes, tokens, device
+        keep = [delta, states, nodes, tokens]
+        args = [self._handle, delta.data_ptr()]
+        if pda is not None:
+            push, stack, depth = pda
+            push = torch.as_tensor(push)
+            if push.shape != delta.shape or push.is_floating_point() or push.is_complex():
+                raise ValueError(f"push must be an integer table of delta's shape {tuple(delta.shape)}, got {push.dtype} "
+                                 f"{tuple(push.shape)}")
+            push = push.to(device=device, dtype=torch.int32).contiguous()
+            for x, what, dim in ((stack, "stack", 2), (depth, "depth", 1)):
+                if not (isinstance(x, torch.Tensor) and x.dtype == torch.int32 and x.device == device and x.dim() == dim
+                        and x.shape[0] == B):
+                    raise ValueError(f"{what} must be an int32 tensor on {device} of {dim} dimensions with one row per "
+                                     f"state ({B})")
+            if not (1 <= stack.shape[1] <= _lib.GT_PDA_MAX_DEPTH):
+                raise ValueError(f"stack must be [B, stack_ld] with 1 <= stack_ld <= {_lib.GT_PDA_MAX_DEPTH}, got "
+                                 f"{tuple(stack.shape)}")
+            if not stack.is_contiguous() or not depth.is_contiguous():
+                raise ValueError("stack and depth must be contiguous: [B, stack_ld] rows of stack_ld entries and [B]")
+            keep.append(push)
+            args.append(push.data_ptr())
+        if logw is not None:
+            logw = torch.as_tensor(logw)
+            if not logw.is_floating_point() or logw.shape != delta.shape:
+                raise ValueError(f"logw must be a float table of delta's shape {tuple(delta.shape)}, got {logw.dtype} "
+                                 f"{tuple(logw.shape)}")
+            logw = logw.to(device=device, dtype=torch.float32).contiguous()
+            keep.append(logw)
+            args.append(logw.data_ptr())
+        args += [delta.shape[0], delta.shape[1], states.data_ptr()]
+        if pda is None:
+            args.append(nodes.data_ptr() if nodes is not None else None)
+        else:
+            args += [stack.data_ptr(), stack.shape[1], depth.data_ptr()]
+        if tokens is not None:
+            args.append(tokens.data_ptr())
+        return args + [B], B, device, keep
 
     def dfa_token_mask(self, delta, states, nodes=None):
         """``gt_dfa_token_mask`` on the current stream of the inputs' device: keep-bitmask ``int32[B, ceil(V/32)]`` of the
         items allowed under the DFA ``delta`` (``[Q, ld >= S]``) from ``states[b]`` at ``nodes[b]`` (the root when None)."""
-        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
-        B, W = states.shape[0], (self.V + 31) // 32
-        bits = torch.empty((B, W), dtype=torch.int32, device=device)
-        if B and W:
-            self._launch("gt_dfa_token_mask", device.index, self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1],
-                         states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B, bits.data_ptr(), W)
+        args, B, device, _keep = self._automaton_args(delta, states, nodes=nodes)
+        bits = torch.empty((B, (self.V + 31) // 32), dtype=torch.int32, device=device)
+        if bits.numel():
+            self._launch("gt_dfa_token_mask", device.index, *args, bits.data_ptr(), bits.shape[1])
         return bits
-
-    @staticmethod
-    def _logw_input(logw, delta, device):
-        """A float table of ``delta``'s shape as a contiguous float32 tensor on ``device``: the transition log-weights
-        of the weighted DFA and PDA calls."""
-        logw = torch.as_tensor(logw)
-        if not logw.is_floating_point() or logw.shape != delta.shape:
-            raise ValueError(f"logw must be a float table of delta's shape {tuple(delta.shape)}, got {logw.dtype} "
-                             f"{tuple(logw.shape)}")
-        return logw.to(device=device, dtype=torch.float32).contiguous()
 
     def dfa_token_logw(self, delta, logw, states, nodes=None):
         """``gt_dfa_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
         summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
-        delta, states, nodes, _, device = self._dfa_inputs(delta, states, nodes)
-        logw = self._logw_input(logw, delta, device)
-        B, V = states.shape[0], self.V
-        out = torch.empty((B, V), dtype=torch.float32, device=device)
-        if B and V:
-            self._launch("gt_dfa_token_logw", device.index, self._handle, delta.data_ptr(), logw.data_ptr(), delta.shape[0],
-                         delta.shape[1], states.data_ptr(), nodes.data_ptr() if nodes is not None else None, B,
-                         out.data_ptr(), V)
+        args, B, device, _keep = self._automaton_args(delta, states, nodes=nodes, logw=logw)
+        out = torch.empty((B, self.V), dtype=torch.float32, device=device)
+        if out.numel():
+            self._launch("gt_dfa_token_logw", device.index, *args, out.data_ptr(), self.V)
         return out
 
     def dfa_advance(self, delta, states, tokens, nodes=None):
         """``gt_dfa_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after the remaining
         symbols of item ``tokens[b]``, or -1."""
-        delta, states, nodes, tokens, device = self._dfa_inputs(delta, states, nodes, tokens)
-        B = states.shape[0]
+        args, B, device, _keep = self._automaton_args(delta, states, nodes=nodes, tokens=tokens)
         out = torch.empty(B, dtype=torch.int32, device=device)
         if B:
-            self._launch("gt_dfa_advance", device.index, self._handle, delta.data_ptr(), delta.shape[0], delta.shape[1],
-                         states.data_ptr(), nodes.data_ptr() if nodes is not None else None, tokens.data_ptr(), B,
-                         out.data_ptr())
+            self._launch("gt_dfa_advance", device.index, *args, out.data_ptr())
         return out
-
-    # ---- token masks under a byte pushdown automaton, and the PDA advance ------------------------------------------
-    def _pda_inputs(self, delta, push, states, stack, depth, tokens=None):
-        """``_dfa_inputs`` plus ``push`` (an int32 table of ``delta``'s shape) and the rows' stacks, which must already be
-        int32 CUDA tensors on the rows' device: ``stack`` ``[B, stack_ld]`` with contiguous rows and ``depth`` ``[B]``,
-        since the advance updates them in place and a converted copy would lose the update."""
-        delta, states, _, tokens, device = self._dfa_inputs(delta, states, None, tokens)
-        push = torch.as_tensor(push)
-        if push.shape != delta.shape or push.is_floating_point() or push.is_complex():
-            raise ValueError(f"push must be an integer table of delta's shape {tuple(delta.shape)}, got {push.dtype} "
-                             f"{tuple(push.shape)}")
-        push = push.to(device=device, dtype=torch.int32).contiguous()
-        B = states.shape[0]
-        for x, what, dim in ((stack, "stack", 2), (depth, "depth", 1)):
-            if not (isinstance(x, torch.Tensor) and x.dtype == torch.int32 and x.device == device and x.dim() == dim
-                    and x.shape[0] == B):
-                raise ValueError(f"{what} must be an int32 tensor on {device} of {dim} dimensions with one row per state "
-                                 f"({B})")
-        if not (1 <= stack.shape[1] <= _lib.GT_PDA_MAX_DEPTH):
-            raise ValueError(f"stack must be [B, stack_ld] with 1 <= stack_ld <= {_lib.GT_PDA_MAX_DEPTH}, got "
-                             f"{tuple(stack.shape)}")
-        if not stack.is_contiguous() or not depth.is_contiguous():
-            raise ValueError("stack and depth must be contiguous: [B, stack_ld] rows of stack_ld entries and [B]")
-        return delta, push, states, tokens, device
 
     def pda_token_mask(self, delta, push, states, stack, depth):
         """``gt_pda_token_mask`` on the current stream of the inputs' device: keep-bitmask ``int32[B, ceil(V/32)]`` of the
         items the PDA (``delta``, ``push``) accepts from each row's configuration at the root."""
-        delta, push, states, _, device = self._pda_inputs(delta, push, states, stack, depth)
-        B, W = states.shape[0], (self.V + 31) // 32
-        bits = torch.empty((B, W), dtype=torch.int32, device=device)
-        if B and W:
-            self._launch("gt_pda_token_mask", device.index, self._handle, delta.data_ptr(), push.data_ptr(), delta.shape[0],
-                         delta.shape[1], states.data_ptr(), stack.data_ptr(), stack.shape[1], depth.data_ptr(), B,
-                         bits.data_ptr(), W)
+        args, B, device, _keep = self._automaton_args(delta, states, pda=(push, stack, depth))
+        bits = torch.empty((B, (self.V + 31) // 32), dtype=torch.int32, device=device)
+        if bits.numel():
+            self._launch("gt_pda_token_mask", device.index, *args, bits.data_ptr(), bits.shape[1])
         return bits
 
     def pda_token_logw(self, delta, push, logw, states, stack, depth):
         """``gt_pda_token_logw`` on the current stream of the inputs' device: ``float32[B, V]``, each allowed item's
         summed transition log-weights under ``logw`` (a float table of ``delta``'s shape), ``-inf`` elsewhere."""
-        delta, push, states, _, device = self._pda_inputs(delta, push, states, stack, depth)
-        logw = self._logw_input(logw, delta, device)
-        B, V = states.shape[0], self.V
-        out = torch.empty((B, V), dtype=torch.float32, device=device)
-        if B and V:
-            self._launch("gt_pda_token_logw", device.index, self._handle, delta.data_ptr(), push.data_ptr(),
-                         logw.data_ptr(), delta.shape[0], delta.shape[1], states.data_ptr(), stack.data_ptr(),
-                         stack.shape[1], depth.data_ptr(), B, out.data_ptr(), V)
+        args, B, device, _keep = self._automaton_args(delta, states, logw=logw, pda=(push, stack, depth))
+        out = torch.empty((B, self.V), dtype=torch.float32, device=device)
+        if out.numel():
+            self._launch("gt_pda_token_logw", device.index, *args, out.data_ptr(), self.V)
         return out
 
     def pda_advance(self, delta, push, states, stack, depth, tokens):
         """``gt_pda_advance`` on the current stream of the inputs' device: ``int32[B]``, the state after item
         ``tokens[b]``, or -1; ``stack`` and ``depth`` are updated in place where the result is not -1."""
-        delta, push, states, tokens, device = self._pda_inputs(delta, push, states, stack, depth, tokens)
-        B = states.shape[0]
+        args, B, device, _keep = self._automaton_args(delta, states, tokens=tokens, pda=(push, stack, depth))
         out = torch.empty(B, dtype=torch.int32, device=device)
         if B:
-            self._launch("gt_pda_advance", device.index, self._handle, delta.data_ptr(), push.data_ptr(), delta.shape[0],
-                         delta.shape[1], states.data_ptr(), stack.data_ptr(), stack.shape[1], depth.data_ptr(),
-                         tokens.data_ptr(), B, out.data_ptr())
+            self._launch("gt_pda_advance", device.index, *args, out.data_ptr())
         return out
 
     # ---- child masses of one node per row, straight from the rows -----------------------------------------------
